@@ -2,6 +2,7 @@
 """bench.py -- rectified block-sparse attention call on B200: ms per attention call and dense-equivalent TFLOP/s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3a] [--regime walk] [--impl ours|reference]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one call of the reference's inner surface (rectified_block_sparse_attention) on one batch of synthetic
@@ -208,6 +209,24 @@ def synth_heads_device(heads, head0, s, regime, dev, seed=0, d=128):
                 x = x + mu.repeat_interleave(128, dim=0)
             outs[ti][0, hi] = x[:s].to(torch.bfloat16)
     return outs
+
+
+DUMP_BYTES = 32 << 20     # --dump-outputs: float32 bytes written at most (larger outputs are sampled by token row)
+
+
+def dump_outputs(out_dir, out):
+    """--dump-outputs: the attention output [B, S, heads, D] of the timed call as out_dir/output.npy, float32
+    [rows, heads, D] of batch 0.  An output above DUMP_BYTES is sampled: a fixed, seeded set of token rows (ascending, all
+    heads and columns), the same for every run of a workload, so two builds can be compared element for element."""
+    import numpy as np
+    import torch
+    o = out[0]
+    row_bytes = o[0].numel() * 4
+    if o.shape[0] * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(o.shape[0], DUMP_BYTES // row_bytes, replace=False))
+        o = o[torch.from_numpy(rows).to(o.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), o.float().cpu().numpy())
 
 
 def product_geometry(wp):
@@ -557,7 +576,14 @@ def main():
     ap.add_argument("--no-ulysses", action="store_true", help="world > 1: skip the sequence-parallel (Ulysses) leg")
     ap.add_argument("--host-chunk", type=int, default=0,
                     help="heads per chunk of the pipelined host-buffer call (0 = library default: 2, or 1 below 8 heads)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed call to DIR/output.npy (float32; rank 0's heads; token "
+                         "rows sampled with a fixed seed when it exceeds 32 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
 
     # stdout carries exactly ONE JSON line.  Native libraries write to file descriptor 1 behind Python's back (NCCL
@@ -666,6 +692,8 @@ def main():
     if rank == 0:
         sampler.start()
     ms_step = timed(plan.run, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, plan.out)     # before the legs below run the plan again
 
     # per-stage device times (same launches, timed alone) and the roofline of the dominant kernel
     stages = {}

@@ -79,9 +79,15 @@ def _close(a, b):
     assert cos_sim(a, b) >= 0.999 and abs(a - b).max() <= 4e-2 * max(1.0, abs(b).max())
 
 
+@pytest.fixture(scope="module")
+def dev():
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    return torch.device("cuda:0")
+
+
 @pytest.mark.gpu
-def test_wan_processors_dense_limit():
-    dev = torch.device("cuda:0")
+def test_wan_processors_dense_limit(dev):
     dim, heads, s = 256, 2, 1000
     x = torch.randn(1, s, dim, device=dev).to(torch.bfloat16)
     cos, sin, ang = _rope_tables(s, 128, dev)
@@ -112,8 +118,7 @@ def test_wan_processors_dense_limit():
 
 
 @pytest.mark.gpu
-def test_joint_text_processors_dense_limit():
-    dev = torch.device("cuda:0")
+def test_joint_text_processors_dense_limit(dev):
     dim, heads, nv = 256, 2, 1024
     x = torch.randn(1, nv, dim, device=dev).to(torch.bfloat16)
     cos, sin, _ = _rope_tables(nv, 128, dev)
@@ -153,12 +158,11 @@ def test_joint_text_processors_dense_limit():
 
 
 @pytest.mark.gpu
-def test_fused_prep_processors_match_unfused():
+def test_fused_prep_processors_match_unfused(dev):
     """HunyuanVideo / Flux processors with kernel 0 (head split + QK RMSNorm + RoPE + pooling fused, the default) against
     the same processors running those steps op by op (`fuse_prep = False`): dual-stream, single-stream and a ragged
     visual segment.  (torch.nn.RMSNorm rounds once where diffusers' RMSNorm -- which kernel 0 follows -- rounds twice,
     so rows differ by at most a bf16 ulp before the attention; the dense limit keeps the block choice out of it.)"""
-    dev = torch.device("cuda:0")
     dim, heads = 256, 2
     for nv in (1024, 1000):
         x = torch.randn(1, nv, dim, device=dev).to(torch.bfloat16)
@@ -217,11 +221,10 @@ def test_fused_prep_processors_match_unfused():
 
 
 @pytest.mark.gpu
-def test_whole_layer_records_into_a_cuda_graph():
+def test_whole_layer_records_into_a_cuda_graph(dev):
     """SURVEY 8f rank 3, last clause: with the host synchronisations gone (the caller supplies `num_true`), a whole
     attention layer through the processor protocol -- projections, kernel 0, kernels 3a-4, output projections --
     records into one CUDA graph and replays on new inputs with the eager result, bit for bit."""
-    dev = torch.device("cuda:0")
     dim, heads, nv = 256, 2, 1024
     attn = _mk(dev, dim, heads, added=True)
     cos, sin, _ = _rope_tables(nv, 128, dev)
@@ -250,10 +253,9 @@ def test_whole_layer_records_into_a_cuda_graph():
 
 
 @pytest.mark.gpu
-def test_processor_mask_refresh_interval():
+def test_processor_mask_refresh_interval(dev):
     """`mask_refresh_interval = 2`: the second call of a layer keeps the first call's block selection (fused and
     op-by-op paths); on unchanged inputs that is bit-identical to rebuilding, and the third call rebuilds."""
-    dev = torch.device("cuda:0")
     dim, heads, nv = 256, 2, 2048
     attn = _mk(dev, dim, heads, added=True)
     cos, sin, _ = _rope_tables(nv, 128, dev)
@@ -276,13 +278,12 @@ def test_processor_mask_refresh_interval():
 
 
 @pytest.mark.gpu
-def test_cogvideox_processor_with_64_dim_heads():
+def test_cogvideox_processor_with_64_dim_heads(dev):
     """CogVideoX1.5's real geometry: 64-dimensional heads, LayerNorm(64) on q/k, 226 text tokens.  Kernel 0 does not
     apply (it is built for 128 columns), so the processor runs the reference's op sequence and the attention goes
     through kernels 2-4 with head_dim 64 (missing columns read as zeros); dense warm-up call (kernel 4, all blocks) and
     sparse call in the dense limit must agree with each other and with PyTorch SDPA through the same module."""
     from rectified_spaattn import _processors as P
-    dev = torch.device("cuda:0")
     dim, heads, nv = 256, 4, 1024
     attn = FakeAttention(dim, heads, head_dim=64, norm="layer").to(dev).to(torch.bfloat16)
     x = torch.randn(1, nv, dim, device=dev).to(torch.bfloat16)
