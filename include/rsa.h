@@ -8,8 +8,8 @@
  * (rectified-spaattn_b200/rectified_spaattn/*.py) binds these with ctypes; INTEGRATION.md shows the stub a
  * maintainer of the reference would add.
  *
- * Conventions: all tensors are bf16 unless stated (query/key/value/out may be fp16: rsa_attn_desc.dtype), head_dim ==
- * 128, block size == 128 tokens.
+ * Conventions: all tensors are bf16 unless stated (query/key/value/out may be fp16: rsa_attn_desc.dtype), head_dim
+ * 128 or 64 (CogVideoX; see rsa_attn_desc.head_dim and the entry points), block size == 128 tokens.
  * "BH" = batch * heads (heads are independent end to end).  Strides are in ELEMENTS of the tensor's dtype.
  */
 #ifndef RSA_H_
@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define RSA_VERSION 106
+#define RSA_VERSION 107 /* 107: kernel 0 and the fused Ulysses exchange take head_dim 64 (norm 3) */
 #define RSA_BLOCK 128
 #define RSA_HEAD_DIM 128
 #define RSA_MAX_ENTRIES 2048 /* max sortable entries per query block: NQ (+1 for the text aggregate) */
@@ -30,7 +30,7 @@ extern "C" {
 enum rsa_status {
   RSA_OK = 0,
   RSA_ERR_ARG = -1,         /* null pointer, negative size, inconsistent geometry */
-  RSA_ERR_UNSUPPORTED = -2, /* head_dim != 128, too many blocks, misaligned strides */
+  RSA_ERR_UNSUPPORTED = -2, /* head_dim / norm form not built, too many blocks, misaligned strides */
   RSA_ERR_CUDA = -3,        /* a CUDA runtime/driver call failed; see rsa_last_error_string() */
   RSA_ERR_WORKSPACE = -4    /* workspace pointer null or smaller than rsa_attn_workspace_bytes() */
 };
@@ -206,7 +206,7 @@ int rsa_rectified_attention_reuse(const rsa_attn_desc* d, const void* q, const v
 /* ------------------------------------------------------------------------------------------------------
  * Kernel 0 (SURVEY 8f rank 1): what the reference's processors do between the QKV projections and the attention call,
  * fused into one pass over the projection outputs: head split, per-head QK RMSNorm, rotary embedding, re-layout
- * [B, rows, H*128] -> [B, H, S, 128], and (pool != 0) kernel 2's block pooling of the rows just produced, so Q, K, V
+ * [B, rows, H*D] -> [B, H, S, D] (D = head_dim), and (pool != 0) kernel 2's block pooling of the rows just produced, so Q, K, V
  * are written once and never read back before kernel 4.  Replaces rectified_hunyuan_attn.py:448-479 and the same
  * sequence in rectified_flux_attn.py:
  *   query.unflatten(2, (heads, -1)).transpose(1, 2)                                   :448-450
@@ -224,28 +224,30 @@ int rsa_rectified_attention_reuse(const rsa_attn_desc* d, const void* q, const v
  * encoder stream (dst_row = visual token count; rope_rows = 0).  Destination tensors, their strides and the block
  * geometry come from the attention descriptor the rows are produced for.  With pool != 0 the workspace must be that
  * descriptor's workspace and every visual / text block must be produced by such calls before
- * rsa_rectified_attention_pooled runs. */
+ * rsa_rectified_attention_pooled runs.
+ * head_dim 128 takes every norm; head_dim 64 (CogVideoX1.5: 48 heads x 64) takes norm 3 only (RSA_ERR_UNSUPPORTED
+ * otherwise), with the pooled statistics' columns 64..127 written as zeros, as rsa_pool_stats computes them. */
 typedef struct rsa_prep_desc {
   int32_t rows;             /* tokens in the source tensors                                                   */
   int32_t dst_row;          /* memory row of the destination the first source token goes to: 0 or the visual  */
                             /* token count                                                                    */
-  int64_t src_stride[3][2]; /* q, k, v sources [batch, rows, heads*128]: (batch, token) element strides        */
+  int64_t src_stride[3][2]; /* q, k, v sources [batch, rows, heads*head_dim]: (batch, token) element strides   */
   int32_t norm;             /* 0 = none, 1 = RMSNorm over head_dim (HunyuanVideo, Flux), 2 = RMSNorm over all  */
                             /* heads*128 channels of a token (Wan2.1 / Wan2.2, rectified_wan21_attn.py:423-426)*/
                             /* 3 = LayerNorm over head_dim with weight and bias (CogVideoX, cogvideo :452-455) */
   float eps;
-  const void* q_weight;     /* DEVICE bf16 [128] (norm 1) or [heads*128] (norm 2): norm_q.weight               */
+  const void* q_weight;     /* DEVICE bf16 [head_dim] (norms 1, 3) or [heads*128] (norm 2): norm_q.weight      */
   const void* k_weight;     /* likewise norm_k.weight                                                          */
   int32_t rope_rows;        /* source tokens [0, rope_rows) are rotated; 0 = no rotary embedding               */
-  int32_t rope_compact;     /* 0: cos and sin are two tables.  1: `cos` is ONE table [rope_rows, 64] of          */
+  int32_t rope_compact;     /* 0: cos and sin are two tables.  1: `cos` is ONE table [rope_rows, head_dim/2] of */
                             /* (cos_i, sin_i) pairs and `sin` is ignored -- diffusers' tables repeat every value  */
                             /* for the two elements of a pair (repeat_interleave(2)), so this holds the same      */
                             /* numbers in half the bytes; the caller vouches for cos[2i] == cos[2i+1] and         */
                             /* sin[2i] == sin[2i+1] (rsa_b200/ops.py checks once per table).  Same arithmetic.    */
-  const float* cos;         /* DEVICE fp32 [rope_rows, 128] (diffusers' repeat-interleaved cos table)          */
+  const float* cos;         /* DEVICE fp32 [rope_rows, head_dim] (diffusers' repeat-interleaved cos table)     */
   const float* sin;
   float* row_scratch;       /* norm 2 only: DEVICE scratch of 2*batch*rows floats for the per-token statistics  */
-  const void* q_bias;       /* norm 3 only: DEVICE bf16 [128] (norm_q.bias)                                     */
+  const void* q_bias;       /* norm 3 only: DEVICE bf16 [head_dim] (norm_q.bias)                                */
   const void* k_bias;
 } rsa_prep_desc;
 
@@ -297,20 +299,20 @@ int rsa_peer_close(void* ptr);
  * when the tokens do not divide (every rank must own at least one; all buffers are laid out for rows_per_rank rows).
  * This rank computes heads [head0, head0 + desc->heads) of the heads_total heads; the shards need not be even (12 heads
  * on 8 ranks: 2,2,2,2,1,1,1,1), every rank states its own first head and its own count.  Prep norm 0, 1, or 2 (2 needs
- * rinv_table).  A ragged visual segment (HunyuanVideo 129
+ * rinv_table) at head_dim 128; norm 3 (LayerNorm, CogVideoX) over the whole sequence at head_dim 64.  A ragged visual segment (HunyuanVideo 129
  * frames) takes two gather calls like rsa_qkv_prep: the visual tokens (dst_row 0) and the text tokens (dst_row = visual
  * token count); the source token of row r is dst_row + r in both. */
 typedef struct rsa_peer_route {
   int32_t n_ranks, rank;
   int32_t rows_per_rank;
-  int32_t heads_total;          /* heads of the host model = channels / 128 of the source and result rows          */
+  int32_t heads_total;          /* heads of the host model = channels / head_dim of the source and result rows     */
   int32_t head0;                /* this rank's first head: it computes heads [head0, head0 + desc->heads)          */
   int32_t reserved;             /* 0                                                                               */
   const void* const* src_table; /* DEVICE array [3][n_ranks] (q, k, v): every rank's projection output,           */
-                                /* [batch, rows_per_rank, heads_total*128] bf16, as mapped in THIS process          */
+                                /* [batch, rows_per_rank, heads_total*head_dim] bf16, as mapped in THIS process     */
   int64_t src_stride[2];        /* (batch, token) element strides of those buffers                                 */
   void* const* out_table;       /* DEVICE array [n_ranks]: every rank's result buffer [batch, rows_per_rank,       */
-                                /* heads_total, 128] bf16, as mapped in this process                               */
+                                /* heads_total, head_dim] bf16, as mapped in this process                          */
   int64_t out_stride[2];        /* (batch, token) element strides of those buffers                                 */
   const float* const* rinv_table; /* prep norm 2 (Wan: RMSNorm over all heads_total*128 channels of a token) only:  */
                                 /* DEVICE array [2][n_ranks] (q, k): every rank's per-token statistics              */

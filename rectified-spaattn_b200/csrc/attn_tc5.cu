@@ -527,7 +527,7 @@ attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       } else {  // fused Ulysses scatter: the row belongs to rank mrow / peer_rows; store into its buffer over NVLink
         const int owner = store ? mrow / a.peer_rows : 0;  // rows that are not stored must not index past the table
         orow = a.o_table[owner] + b * a.peer_os[0] +
-               (int64_t)(mrow - owner * a.peer_rows) * a.peer_os[1] + (a.peer_head0 + h) * 128;
+               (int64_t)(mrow - owner * a.peer_rows) * a.peer_os[1] + (a.peer_head0 + h) * kD;
       }
       if (cnt > 0) {
         mbar_wait(bar(B_OFULL + s), 0);

@@ -15,7 +15,7 @@
 // zeros above, a text block reads memory rows shifted down by the gap.
 //
 // The same kernel has a second front end ("prep", kernel 0): instead of loading finished Q/K/V rows it builds them from
-// the projection outputs [B, S, H*128] -- per-head RMSNorm, rotary embedding, re-layout to [B, H, S, 128] -- stores
+// the projection outputs [B, S, H*D] -- per-head RMSNorm, rotary embedding, re-layout to [B, H, S, D] -- stores
 // them, and pools the values it has just rounded to bf16, so the pooled statistics are bit-identical to pooling the
 // stored rows and Q, K, V are never read back.  Replaces rectified_hunyuan_attn.py:448-479 (and the same sequence
 // in rectified_flux_attn.py): unflatten/transpose, attn.norm_q / attn.norm_k (diffusers RMSNorm(head_dim, eps):
@@ -33,18 +33,18 @@ namespace {
 constexpr int kThreads = 256;
 
 struct PrepArgs {
-  const __nv_bfloat16* src[3];  // q, k, v projection outputs [B, rows, H*128]
+  const __nv_bfloat16* src[3];  // q, k, v projection outputs [B, rows, H*D], D = head_dim (128, or 64 with layer_norm)
   int64_t src_stride[3][2];     // (batch, token) element strides
-  __nv_bfloat16* dst[3];        // [B, H, S, 128] views
+  __nv_bfloat16* dst[3];        // [B, H, S, D] views
   int64_t dst_stride[3][3];     // (batch, head, token)
-  const __nv_bfloat16* w[2];    // RMSNorm weights of q, k (bf16 [128], or [H*128] with w_head_stride = 128) or nullptr
-  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k (bf16 [128]) -- layer_norm only
+  const __nv_bfloat16* w[2];    // norm weights of q, k (bf16 [D], or [H*128] with w_head_stride = 128) or nullptr
+  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k (bf16 [D]) -- layer_norm only
   int layer_norm;               // 1: LayerNorm over head_dim (CogVideoX: mean removed, bias added, one rounding)
   int w_head_stride;            // 0: one weight vector per tensor (norm over head_dim); 128: norm across heads (Wan)
   const float* row_rinv[2];     // norm across heads: rsqrt(mean(x^2) + eps) per (batch, source row), from row_rms_kernel
   float eps;
-  const float *cos, *sin;       // fp32 [rope_rows, 128]
-  int rope_compact;             // cos = [rope_rows, 64] pairs (cos_i, sin_i), sin unused: half the table bytes per row
+  const float *cos, *sin;       // fp32 [rope_rows, D]
+  int rope_compact;             // cos = [rope_rows, D / 2] pairs (cos_i, sin_i), sin unused: half the table bytes per row
   int rope_rows;                // source rows below this are rotated
   int rows;                     // source rows
   int dst_row0;                 // memory row of source row 0 in the destination
@@ -97,19 +97,19 @@ __device__ __forceinline__ uint4 ld_global_v4(const void* p) {
 struct RopeRow {
   float4 c0, c1, s0, s1;
 };
-template <bool kCompact>
+template <bool kCompact, int kD = 128>
 __device__ __forceinline__ RopeRow load_rope(const PrepArgs& p, int r, int col, bool on) {
   RopeRow t;
   t.c0 = t.c1 = t.s0 = t.s1 = make_float4(0.f, 0.f, 0.f, 0.f);
   if (on) {
-    const float4* cp = reinterpret_cast<const float4*>(p.cos + (int64_t)r * 128 + col);
+    const float4* cp = reinterpret_cast<const float4*>(p.cos + (int64_t)r * kD + col);
     if constexpr (kCompact) {
-      // the thread's 8 columns are 4 pairs: (cos, sin) x 4 = 8 floats at the same offset of the 128-float row
+      // the thread's 8 columns are 4 pairs: (cos, sin) x 4 = 8 floats at the same offset of the kD-float row
       const float4 a = __ldg(cp), b = __ldg(cp + 1);
       t.c0 = make_float4(a.x, a.x, a.z, a.z), t.c1 = make_float4(b.x, b.x, b.z, b.z);
       t.s0 = make_float4(a.y, a.y, a.w, a.w), t.s1 = make_float4(b.y, b.y, b.w, b.w);
     } else {
-      const float4* sp = reinterpret_cast<const float4*>(p.sin + (int64_t)r * 128 + col);
+      const float4* sp = reinterpret_cast<const float4*>(p.sin + (int64_t)r * kD + col);
       t.c0 = __ldg(cp), t.c1 = __ldg(cp + 1), t.s0 = __ldg(sp), t.s1 = __ldg(sp + 1);
     }
   }
@@ -119,9 +119,11 @@ __device__ __forceinline__ RopeRow load_rope(const PrepArgs& p, int r, int col, 
 // kNorm: 0 none, 1 RMSNorm over head_dim, 2 RMSNorm across heads (row statistic precomputed), 3 LayerNorm over head_dim.
 // kGather: rows come from peer-mapped buffers.  kCompact: one (cos, sin)-pair table.  Compile-time so that each form
 // carries only its own code and registers (with all of them behind run-time flags the HunyuanVideo form lost 40 %).
-template <int kNorm, bool kCompact, bool kGather>
+// kD: head_dim.  At 64 (CogVideoX, LayerNorm only) a thread's 8 columns belong to one of two adjacent heads h, h + 1
+// (see qkv_prep_stream_kernel); `heads` tells whether head h + 1 exists.
+template <int kNorm, bool kCompact, bool kGather, int kD = 128>
 __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
-                                             uint4 (&raw)[8]);
+                                             uint4 (&raw)[8], int heads = 0);
 
 template <int kNorm, bool kGather, bool kCompact>
 __device__ __forceinline__ void prep_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
@@ -154,19 +156,23 @@ __device__ __forceinline__ void prep_rows(const PrepArgs& p, int which, int b, i
   process_rows<kNorm, kCompact, kGather>(p, which, b, h, jblk, warp, lane, raw);
 }
 
-// raw[it] = source row jblk * 128 + 16 warp + 2 it + (lane >> 4), columns 8 (lane & 15) .. +7 of head h (zeros beyond the
-// source): normalise / rotate / round, store to the destination, and leave the rounded values in raw.
-template <int kNorm, bool kCompact, bool kGather>
+// raw[it] = source row jblk * 128 + 16 warp + 2 it + (lane >> 4), columns 8 (lane & 15) .. +7 of head h (kD = 64:
+// columns 8 (lane & 7) .. +7 of head h + ((lane >> 3) & 1)), zeros beyond the source: normalise / rotate / round, store
+// to the destination, and leave the rounded values in raw (zeros for the lanes of a head that does not exist).
+template <int kNorm, bool kCompact, bool kGather, int kD>
 __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
-                                             uint4 (&raw)[8]) {
-  const int col = 8 * (lane & 15);
-  __nv_bfloat16* dst = p.dst[which] + b * p.dst_stride[which][0] + h * p.dst_stride[which][1] + col;
+                                             uint4 (&raw)[8], int heads) {
+  static_assert(kD == 128 || (kD == 64 && kNorm == 3), "the 64-column form is built for LayerNorm (CogVideoX) only");
+  const int col = kD == 128 ? 8 * (lane & 15) : 8 * (lane & 7);
+  const int hh = kD == 128 ? h : h + ((lane >> 3) & 1);
+  const bool head_live = kD == 128 || hh < heads;
+  __nv_bfloat16* dst = p.dst[which] + b * p.dst_stride[which][0] + hh * p.dst_stride[which][1] + col;
   const int r0 = jblk * 128 + 16 * warp + (lane >> 4);
   if (which == 2) {  // V: re-layout only
 #pragma unroll
     for (int it = 0; it < 8; ++it) {
       const int r = r0 + 2 * it;
-      if (r < p.rows) *reinterpret_cast<uint4*>(dst + (int64_t)(p.dst_row0 + r) * p.dst_stride[which][2]) = raw[it];
+      if (r < p.rows && head_live) *reinterpret_cast<uint4*>(dst + (int64_t)(p.dst_row0 + r) * p.dst_stride[which][2]) = raw[it];
     }
     return;
   }
@@ -177,25 +183,25 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
   const float* rinv_rows = (kNorm == 2 && !kGather) ? p.row_rinv[which] + (int64_t)b * p.rows : nullptr;
   float bia[8];
   if constexpr (kNorm == 3) unpack8(__ldg(reinterpret_cast<const uint4*>(p.bias[which] + col)), bia);
-  RopeRow next = load_rope<kCompact>(p, r0, col, r0 < p.rows && r0 < p.rope_rows);
+  RopeRow next = load_rope<kCompact, kD>(p, r0, col, r0 < p.rows && r0 < p.rope_rows);
 #pragma unroll
   for (int it = 0; it < 8; ++it) {
     const int r = r0 + 2 * it;
     const bool live = r < p.rows;
     const bool rot = live && r < p.rope_rows;
     const RopeRow t = next;
-    if (it < 7) next = load_rope<kCompact>(p, r + 2, col, r + 2 < p.rows && r + 2 < p.rope_rows);
+    if (it < 7) next = load_rope<kCompact, kD>(p, r + 2, col, r + 2 < p.rows && r + 2 < p.rope_rows);
     float f[8];
     unpack8(raw[it], f);
     if constexpr (kNorm == 3) {
       // torch.nn.LayerNorm(head_dim) on a bf16 tensor: statistics and affine in fp32, ONE rounding to bf16
-      // (cogvideo :452-455; two-pass variance, fixed butterfly order over the 16 lanes that share the row)
+      // (cogvideo :452-455; two-pass variance, fixed butterfly order over the kD / 8 lanes that share the (row, head))
       float sm = 0.f;
 #pragma unroll
       for (int c = 0; c < 8; ++c) sm = __fadd_rn(sm, f[c]);
 #pragma unroll
-      for (int o = 1; o < 16; o <<= 1) sm = __fadd_rn(sm, __shfl_xor_sync(0xffffffffu, sm, o));
-      const float mean = __fmul_rn(sm, 1.0f / 128.0f);
+      for (int o = 1; o < kD / 8; o <<= 1) sm = __fadd_rn(sm, __shfl_xor_sync(0xffffffffu, sm, o));
+      const float mean = __fmul_rn(sm, 1.0f / kD);
       float ss = 0.f;
 #pragma unroll
       for (int c = 0; c < 8; ++c) {
@@ -203,8 +209,8 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
         ss = __fmaf_rn(f[c], f[c], ss);
       }
 #pragma unroll
-      for (int o = 1; o < 16; o <<= 1) ss = __fadd_rn(ss, __shfl_xor_sync(0xffffffffu, ss, o));
-      const float rstd = rsqrtf(__fadd_rn(__fmul_rn(ss, 1.0f / 128.0f), p.eps));
+      for (int o = 1; o < kD / 8; o <<= 1) ss = __fadd_rn(ss, __shfl_xor_sync(0xffffffffu, ss, o));
+      const float rstd = rsqrtf(__fadd_rn(__fmul_rn(ss, 1.0f / kD), p.eps));
 #pragma unroll
       for (int c = 0; c < 8; c += 2) {
         const float2 y = __bfloat1622float2(__floats2bfloat162_rn(__fmaf_rn(wgt[c], __fmul_rn(rstd, f[c]), bia[c]),
@@ -254,8 +260,8 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
 #pragma unroll
     for (int c = 0; c < 4; ++c) o2[c] = __floats2bfloat162_rn(f[2 * c], f[2 * c + 1]);
     const uint4 u = *reinterpret_cast<const uint4*>(o2);
-    if (live) *reinterpret_cast<uint4*>(dst + (int64_t)(p.dst_row0 + r) * p.dst_stride[which][2]) = u;
-    raw[it] = live ? u : make_uint4(0, 0, 0, 0);
+    if (live && head_live) *reinterpret_cast<uint4*>(dst + (int64_t)(p.dst_row0 + r) * p.dst_stride[which][2]) = u;
+    raw[it] = live && head_live ? u : make_uint4(0, 0, 0, 0);
   }
 }
 
@@ -434,10 +440,13 @@ constexpr int kPoolSmem = kPoolStages * kPoolStageBytes + 64;
 // block (two without deviations); s_part has one buffer per sweep, which saves the barrier between blocks: the next
 // block writes s_part[0] (last read two barriers ago) and s_mean / s_part[1] only after its own first / second
 // barrier, which every reader reaches first.
-template <class F>
+// kD = 64 (kernel 0's head pairs): columns [0, 64) are head bh's, [64, 128) head bh + 1's, which exists only when
+// live_cols == 128; each head's statistics row gets exact zeros in its columns [64, 128), as kernel 2 computes them for
+// 64-column heads.
+template <int kD = 128, class F>
 __device__ __forceinline__ void pool_block(const PoolArgs& a, const float2 (&f)[8][4], int which, int bh, int blk,
                                            float (*s_part)[8][128], float* s_mean, int tid, int warp, int lane,
-                                           F&& after_first_barrier) {
+                                           F&& after_first_barrier, int live_cols = 128) {
   const int col = 8 * (lane & 15);
   float2 acc[4];
 #pragma unroll
@@ -463,7 +472,13 @@ __device__ __forceinline__ void pool_block(const PoolArgs& a, const float2 (&f)[
     for (int w = 1; w < 8; ++w) t = __fadd_rn(t, s_part[0][w][tid]);
     const float m = __fmul_rn(t, 1.0f / 128.0f);
     s_mean[tid] = m;
-    a.mean[which][((int64_t)bh * a.out_rows[which] + blk) * 128 + tid] = m;
+    if constexpr (kD == 128) {
+      a.mean[which][((int64_t)bh * a.out_rows[which] + blk) * 128 + tid] = m;
+    } else if (tid < live_cols) {
+      float* row = a.mean[which] + ((int64_t)(bh + (tid >> 6)) * a.out_rows[which] + blk) * 128 + (tid & 63);
+      row[0] = m;
+      row[64] = 0.f;
+    }
   }
   __syncthreads();
   if (a.mad[which] == nullptr) return;  // V: means only (uniform over the CTA)
@@ -492,7 +507,13 @@ __device__ __forceinline__ void pool_block(const PoolArgs& a, const float2 (&f)[
     float t = s_part[1][0][tid];
 #pragma unroll
     for (int w = 1; w < 8; ++w) t = __fadd_rn(t, s_part[1][w][tid]);
-    a.mad[which][((int64_t)bh * a.n_blk[which] + blk) * 128 + tid] = __fmul_rn(t, 1.0f / 128.0f);
+    if constexpr (kD == 128) {
+      a.mad[which][((int64_t)bh * a.n_blk[which] + blk) * 128 + tid] = __fmul_rn(t, 1.0f / 128.0f);
+    } else if (tid < live_cols) {
+      float* row = a.mad[which] + ((int64_t)(bh + (tid >> 6)) * a.n_blk[which] + blk) * 128 + (tid & 63);
+      row[0] = __fmul_rn(t, 1.0f / 128.0f);
+      row[64] = 0.f;
+    }
   }
 }
 
@@ -640,7 +661,12 @@ __global__ void __launch_bounds__(kThreads, 2) pool_stats_stream_kernel(const Po
 // Items are ordered block-major, then tensor, then head: the 3 * B * H items of one token block read the same source
 // rows (all heads of a token are contiguous) and the same rotary-table rows, which therefore stay in L1 / L2 instead
 // of being streamed from HBM once per head (the table alone is as large as L2 at the HunyuanVideo size).
-template <int kNorm, bool kGather, bool kCompact>
+// kD = 64 (CogVideoX): an item is a pair of adjacent heads (h, h + 1) of one batch element, whose two 64-column slices
+// are one 256-byte run of the source row -- the same copies into the same stage rows as at 128 columns.  Lanes 0-7 of
+// each half-warp take head h, lanes 8-15 head h + 1; an odd head count leaves the last pair half empty (128-byte
+// copies, nothing stored for the missing head).  Every lane stays busy: the kernel is bound by issue slots, and one
+// head per item would idle half of them.  n_bh counts pairs then (B * ceil(H / 2)).
+template <int kNorm, bool kGather, bool kCompact, int kD = 128>
 __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const PoolArgs a, const PrepArgs p, const int n_blocks,
                                                                       const int n_bh) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -683,10 +709,13 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
     advance(nxt);
     const int st = n % kPoolStages;
     const int rows = max(0, min(128, p.rows - it.jblk * 128));
-    const int b = it.bh / a.heads, h = it.bh - b * a.heads;
+    const int per_b = kD == 128 ? a.heads : (a.heads + 1) >> 1;  // items per (block, tensor, batch element)
+    const int b = it.bh / per_b, u = it.bh - b * per_b;
+    const int h = kD == 128 ? u : 2 * u;  // (first) head of the item
+    const uint32_t row_bytes = (kD == 128 || h + 1 < a.heads) ? 256u : 128u;
     const uint32_t dst = sbase + st * kPoolStageBytes, bar = bar0 + 8 * st;
     if (tid == 0) {
-      if (rows > 0) mbar_arrive_expect_tx(bar, (uint32_t)(rows * 256));
+      if (rows > 0) mbar_arrive_expect_tx(bar, (uint32_t)rows * row_bytes);
       else mbar_arrive(bar);
     }
     const int r = 16 * warp + lane;
@@ -694,13 +723,13 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
       const int64_t ts = p.src_stride[it.which][1];
       const int row = it.jblk * 128 + r;
       if constexpr (!kGather) {
-        bulk_load_1d(dst + r * 256, p.src[it.which] + b * p.src_stride[it.which][0] + (int64_t)h * 128 + (int64_t)row * ts, 256u, bar);
+        bulk_load_1d(dst + r * 256, p.src[it.which] + b * p.src_stride[it.which][0] + (int64_t)h * kD + (int64_t)row * ts, row_bytes, bar);
       } else {
         const int tok = p.dst_row0 + row;  // the peer buffers hold the tokens in memory order, like the destination
         const int owner = tok / p.src_rows;
         const __nv_bfloat16* base = p.src_table[it.which * p.n_src + owner];
-        bulk_load_1d(dst + r * 256, base + b * p.src_stride[it.which][0] + (int64_t)(p.src_head0 + h) * 128 +
-                                        (int64_t)(tok - owner * p.src_rows) * ts, 256u, bar);
+        bulk_load_1d(dst + r * 256, base + b * p.src_stride[it.which][0] + (int64_t)(p.src_head0 + h) * kD +
+                                        (int64_t)(tok - owner * p.src_rows) * ts, row_bytes, bar);
       }
     }
   };
@@ -713,7 +742,12 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
     const int which = cur.which, bh = cur.bh, jblk = cur.jblk;
     advance(cur);
     const int blk = p.blk0 + jblk;
-    const int b = bh / a.heads, h = bh - b * a.heads;
+    const int per_b = kD == 128 ? a.heads : (a.heads + 1) >> 1;
+    const int b = bh / per_b, u = bh - b * per_b;
+    const int h = kD == 128 ? u : 2 * u;
+    const int bh0 = kD == 128 ? bh : b * a.heads + h;          // (first) head's row of the statistics
+    const int live_cols = (kD == 128 || h + 1 < a.heads) ? 128 : 64;  // 64: head h + 1 does not exist
+    const bool lane_live = kD == 128 || col < live_cols;
     const int st = n % kPoolStages;
     mbar_wait(bar0 + 8 * st, (n / kPoolStages) & 1);
     const uint4* tp = reinterpret_cast<const uint4*>(smem + st * kPoolStageBytes + rloc * 256 + col * 2);
@@ -722,9 +756,9 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       raw[i] = make_uint4(0, 0, 0, 0);
-      if (rloc + 2 * i < rows) raw[i] = tp[i * 32];
+      if (rloc + 2 * i < rows && lane_live) raw[i] = tp[i * 32];
     }
-    process_rows<kNorm, kCompact, kGather>(p, which, b, h, jblk, warp, lane, raw);
+    process_rows<kNorm, kCompact, kGather, kD>(p, which, b, h, jblk, warp, lane, raw, a.heads);
     const bool visual = blk < a.nq_vis;
     bool pooled = false;
     if (p.pool) {
@@ -739,12 +773,18 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const int t = (blk - a.nq_vis) * 128 + rloc + 2 * i;  // text token index
-          if (t < a.text_keys) {
+          if (t < a.text_keys && lane_live) {
             float f[8];
             unpack8<false>(raw[i], f);
-            float* dstk = a.mean[1] + ((int64_t)bh * a.out_rows[1] + a.n_blk[1] + t) * 128 + col;
+            // kD = 64: head bh0 + (col >> 6), its columns (col & 63) .. +7, and zeros in the 64 columns it lacks
+            const int row_bh = kD == 128 ? bh : bh0 + (col >> 6), row_col = kD == 128 ? col : col & 63;
+            float* dstk = a.mean[1] + ((int64_t)row_bh * a.out_rows[1] + a.n_blk[1] + t) * 128 + row_col;
             reinterpret_cast<float4*>(dstk)[0] = make_float4(f[0], f[1], f[2], f[3]);
             reinterpret_cast<float4*>(dstk)[1] = make_float4(f[4], f[5], f[6], f[7]);
+            if constexpr (kD == 64) {
+              reinterpret_cast<float4*>(dstk + 64)[0] = make_float4(0.f, 0.f, 0.f, 0.f);
+              reinterpret_cast<float4*>(dstk + 64)[1] = make_float4(0.f, 0.f, 0.f, 0.f);
+            }
           }
         }
       }
@@ -754,9 +794,9 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
       float2 f[8][4];
 #pragma unroll
       for (int i = 0; i < 8; ++i) unpack_row<false>(raw[i], f[i]);
-      pool_block(a, f, which, bh, blk, s_part, s_mean, tid, warp, lane, [&]() {
+      pool_block<kD>(a, f, which, bh0, blk, s_part, s_mean, tid, warp, lane, [&]() {
         if (n + kPoolStages < n_mine) issue(n + kPoolStages);
-      });
+      }, live_cols);
     } else {
       __syncthreads();  // every thread has taken its rows out of the stage
       if (n + kPoolStages < n_mine) issue(n + kPoolStages);
@@ -934,33 +974,44 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
     RSA_CUDA_CHECK(cudaGetDevice(&dev));
     RSA_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   }
-  const int n_bh = d->batch * d->heads;
+  const bool hd64 = d->head_dim == 64;  // items are head pairs (qkv_prep_stream_kernel)
+  const int n_bh = d->batch * (hd64 ? (d->heads + 1) / 2 : d->heads);
   const int64_t items = (int64_t)blocks * 3 * n_bh;
   if (items > 0x7fffffffLL) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: too many blocks");
   const int sgrid = (int)(items < 2 * sms ? items : 2 * sms);
   dim3 grid(3 * d->batch * d->heads, blocks);
   // per-block form: 2 CTAs per SM (about 100 registers): capping at 3 or 4 CTAs spills and is no faster (1.24 / 1.25 / 2.17 ms at C3b)
-#define RSA_PREP_STREAM(NORM, GATHER, COMPACT)                                                                          \
+#define RSA_PREP_STREAM(NORM, GATHER, COMPACT, D)                                                                       \
   do {                                                                                                                  \
     static bool cfg = false;                                                                                            \
     if (!cfg) {                                                                                                         \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT>,                                 \
+      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D>,                              \
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));                     \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT>,                                 \
+      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D>,                              \
                                           cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
       cfg = true;                                                                                                       \
     }                                                                                                                   \
-    qkv_prep_stream_kernel<NORM, GATHER, COMPACT><<<sgrid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);               \
+    qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D><<<sgrid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);            \
   } while (0)
 #define RSA_PREP_LAUNCH(NORM, GATHER)                                                               \
   do {                                                                                              \
     if (form == 1) {                                                                                \
-      if (compact) RSA_PREP_STREAM(NORM, GATHER, true);                                             \
-      else RSA_PREP_STREAM(NORM, GATHER, false);                                                    \
+      if (compact) RSA_PREP_STREAM(NORM, GATHER, true, 128);                                        \
+      else RSA_PREP_STREAM(NORM, GATHER, false, 128);                                               \
     } else if (compact) pool_stats_kernel<true, 2, NORM, GATHER, true><<<grid, kThreads, 0, s>>>(a, pa);   \
     else pool_stats_kernel<true, 2, NORM, GATHER, false><<<grid, kThreads, 0, s>>>(a, pa);          \
   } while (0)
-  if (route) {
+  if (hd64) {
+    // 64-column heads: CogVideoX's LayerNorm only (rsa_api.cu refuses the other norms), always the streaming kernel
+    if (route) {
+      if (compact) RSA_PREP_STREAM(3, true, true, 64);
+      else RSA_PREP_STREAM(3, true, false, 64);
+    } else if (compact) {
+      RSA_PREP_STREAM(3, false, true, 64);
+    } else {
+      RSA_PREP_STREAM(3, false, false, 64);
+    }
+  } else if (route) {
     if (p->norm == 1) RSA_PREP_LAUNCH(1, true);
     else if (p->norm == 2) RSA_PREP_LAUNCH(2, true);
     else RSA_PREP_LAUNCH(0, true);

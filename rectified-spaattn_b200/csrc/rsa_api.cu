@@ -487,7 +487,9 @@ extern "C" int rsa_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, cons
   if (rc != RSA_OK) return rc;
   if (!p) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep: descriptor is null");
   if (d->dtype != RSA_DTYPE_BF16) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep follows diffusers' bf16 rounding points: bf16 only");
-  if (d->head_dim != RSA_HEAD_DIM) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: head_dim 128 only");
+  if (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: head_dim must be 128 or 64 (got %d)", d->head_dim);
+  if (d->head_dim == 64 && p->norm != 3)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: head_dim 64 is built for norm 3 (LayerNorm, CogVideoX) only, not norm %d", p->norm);
   if (!q_src || !k_src || !v_src || !q || !k || !v) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep: null tensor");
   const RowMap rm = row_map(d);
   if (p->rows < 1) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep: rows must be positive");
@@ -528,9 +530,10 @@ static int validate_route(const rsa_attn_desc* d, const rsa_peer_route* r, bool 
              r->rows_per_rank, d->seq);
   if (r->head0 < 0 || d->heads < 1 || r->head0 + d->heads > r->heads_total)
     RSA_FAIL(RSA_ERR_ARG, "peer route: heads [%d, %d) outside the %d heads of a row", r->head0, r->head0 + d->heads, r->heads_total);
-  if (need_src && (!r->src_table || r->src_stride[0] < 0 || r->src_stride[1] < r->heads_total * 128 || r->src_stride[0] % 8 || r->src_stride[1] % 8))
+  const int64_t row = (int64_t)r->heads_total * d->head_dim;  // channels of a source / result row
+  if (need_src && (!r->src_table || r->src_stride[0] < 0 || r->src_stride[1] < row || r->src_stride[0] % 8 || r->src_stride[1] % 8))
     RSA_FAIL(RSA_ERR_ARG, "peer route: source table / strides");
-  if (need_out && (!r->out_table || r->out_stride[0] < 0 || r->out_stride[1] < r->heads_total * 128 || r->out_stride[0] % 8 || r->out_stride[1] % 8))
+  if (need_out && (!r->out_table || r->out_stride[0] < 0 || r->out_stride[1] < row || r->out_stride[0] % 8 || r->out_stride[1] % 8))
     RSA_FAIL(RSA_ERR_ARG, "peer route: result table / strides");
   return RSA_OK;
 }
@@ -541,7 +544,8 @@ extern "C" int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* 
   if (rc != RSA_OK) return rc;
   if ((rc = validate_route(d, route, true, false)) != RSA_OK) return rc;
   if (!p || !q || !k || !v) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: null pointer");
-  if (d->dtype != RSA_DTYPE_BF16 || d->head_dim != RSA_HEAD_DIM) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: bf16 and head_dim 128 only");
+  if (d->dtype != RSA_DTYPE_BF16 || (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64))
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: bf16 and head_dim 128 or 64 only");
   // like rsa_qkv_prep: the whole sequence in one call, or -- ragged visual segment -- the visual tokens (dst_row 0) and
   // the text tokens (dst_row = visual token count) in two; source token = dst_row + row either way
   const RowMap rm = row_map(d);
@@ -550,7 +554,16 @@ extern "C" int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* 
   const bool txt = p->dst_row == rm.vis_len && p->rows == d->seq - rm.vis_len && d->family == RSA_FAMILY_JOINT;
   if (!whole && !vis && !txt)
     RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: rows / dst_row must name the whole sequence, the visual tokens or the text tokens");
-  if (p->norm < 0 || p->norm > 2) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: norm must be 0, 1 or 2");
+  // head_dim 128: norms 0-2; head_dim 64 (CogVideoX): LayerNorm (norm 3) over the whole sequence (no gap in its geometry)
+  if (d->head_dim == 64) {
+    if (p->norm != 3)
+      RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: head_dim 64 is built for norm 3 (LayerNorm, CogVideoX) only, not norm %d", p->norm);
+    if (!whole) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: head_dim 64 takes the whole sequence in one call");
+    if (!p->q_bias || !p->k_bias || (uintptr_t)p->q_bias % 16 || (uintptr_t)p->k_bias % 16)
+      RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: norm 3 needs 16-byte aligned biases");
+  } else if (p->norm < 0 || p->norm > 2) {
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: norm must be 0, 1 or 2 at head_dim 128 (got %d)", p->norm);
+  }
   if (p->norm == 2 && !route->rinv_table)
     RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: norm 2 needs route->rinv_table (rsa_row_rms on every owning rank)");
   if (p->norm && (!p->q_weight || !p->k_weight)) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: norm weights are null");
@@ -579,7 +592,10 @@ extern "C" int rsa_rectified_attention_pooled_scatter(const rsa_attn_desc* d, co
   int rc = check_ws(d, workspace, bytes, &L);
   if (rc != RSA_OK) return rc;
   if ((rc = validate_route(d, route, false, true)) != RSA_OK) return rc;
-  if (d->head_dim != RSA_HEAD_DIM) RSA_FAIL(RSA_ERR_UNSUPPORTED, "the scatter epilogue is built for head_dim 128");
+  // result rows are [heads_total, head_dim]: the epilogue places head h at (head0 + h) * head_dim of the kernel
+  // instantiation, so 64-column heads must run the 64-column one (not the debug dump or attention flag 4)
+  if (d->head_dim == 64 && (g_attention_dbg || (g_attention_dbg_flags & 4)))
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_rectified_attention_pooled_scatter: head_dim 64 runs the 64-column kernel 4 only");
   if (!q || !k || !v) RSA_FAIL(RSA_ERR_ARG, "rsa_rectified_attention_pooled_scatter: null tensor");
   char* ws = (char*)workspace;
   cudaStream_t s = (cudaStream_t)stream;

@@ -133,42 +133,51 @@ def wan_rope_tables(emb, n):
     return _wan_rope_cache[key][1]
 
 
-def head_norm_params(mod):
+def head_norm_params(mod, head_dim=128):
     """dict(q_weight-style kwargs) for a per-head norm kernel 0 fuses: RMSNorm(128) (HunyuanVideo / Flux) or
-    LayerNorm(128) with bias (CogVideoX), bf16 parameters; else None.  Returns (weight, bias or None, eps)."""
-    r = rms_params(mod)
+    LayerNorm(head_dim) with bias (CogVideoX: head_dim 128 or 64), bf16 parameters; else None.  Returns (weight, bias or
+    None, eps)."""
+    r = rms_params(mod) if head_dim == 128 else None     # kernel 0 has no RMSNorm at 64 columns
     if r is not None:
         return r[0], None, r[1]
     w, b, eps = getattr(mod, "weight", None), getattr(mod, "bias", None), getattr(mod, "eps", None)
     if mod is None or w is None or b is None or eps is None or "LayerNorm" not in type(mod).__name__:
         return None
-    if w.dtype != torch.bfloat16 or b.dtype != torch.bfloat16 or w.numel() != 128 or b.numel() != 128 or not w.is_cuda:
+    if (w.dtype != torch.bfloat16 or b.dtype != torch.bfloat16 or w.numel() != head_dim or b.numel() != head_dim
+            or not w.is_cuda):
         return None
     return w, b, float(eps)
 
 
-def rope_tables(emb, n):
-    """(cos, sin) fp32 [>= n, 128] tables as diffusers passes them (`image_rotary_emb`), or None if `emb` has another form."""
+def rope_tables(emb, n, head_dim=128):
+    """(cos, sin) fp32 [>= n, head_dim] tables as diffusers passes them (`image_rotary_emb`), or None if `emb` has
+    another form."""
     if not (isinstance(emb, (tuple, list)) and len(emb) == 2):
         return None
     cos, sin = emb
-    ok = all(isinstance(t, torch.Tensor) and t.dim() == 2 and t.shape[1] == 128 and t.shape[0] >= n for t in (cos, sin))
+    ok = all(isinstance(t, torch.Tensor) and t.dim() == 2 and t.shape[1] == head_dim and t.shape[0] >= n
+             for t in (cos, sin))
     return (cos, sin) if ok else None
 
 
 def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k, p_remain, nbr, image_rotary_emb,
                          rope_text, mask_cache=None):
     """The fused form of a joint-text processor's middle section (kernel 0 + kernels 3a-4): projections ->
-    rsa_qkv_prep (head split, RMSNorm, RoPE, re-layout, pooling) -> rsa_rectified_attention_pooled.  Returns
+    rsa_qkv_prep (head split, RMSNorm / LayerNorm, RoPE, re-layout, pooling) -> rsa_rectified_attention_pooled.  Returns
     [B, S, H*D], or None when this layer does not have the shape kernel 0 fuses (the caller then runs the op-by-op path).
+    D (head_dim) is read from `to_q`'s output width: 128, or 64 (CogVideoX, LayerNorm only).
     `rope_text`: Flux rotates the text tokens too (their table rows follow the image rows); HunyuanVideo does not."""
     from rsa_b200 import ops
     heads = attn.heads
     if not hidden_states.is_cuda or hidden_states.dtype != torch.bfloat16:
         return None
+    inner = getattr(attn.to_q, "out_features", None)
+    hd = inner // heads if isinstance(inner, int) and inner % heads == 0 else 0
+    if hd not in (128, 64):
+        return None
     dual = getattr(attn, "add_q_proj", None) is not None and encoder_hidden_states is not None
     def pair(nq, nk):
-        a, c = head_norm_params(getattr(attn, nq, None)), head_norm_params(getattr(attn, nk, None))
+        a, c = head_norm_params(getattr(attn, nq, None), hd), head_norm_params(getattr(attn, nk, None), hd)
         if a is None or c is None or a[2] != c[2] or (a[1] is None) != (c[1] is None):
             return None
         return dict(q_weight=a[0], k_weight=c[0], q_bias=a[1], k_bias=c[1], eps=a[2])
@@ -185,11 +194,11 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
     nv = geo.vis_len or geo.nq_blocks * 128
     rope = None
     if image_rotary_emb is not None:
-        rope = rope_tables(image_rotary_emb, s if rope_text else nv)
+        rope = rope_tables(image_rotary_emb, s if rope_text else nv, hd)
         if rope is None:
             return None
     lat = [f(hidden_states) for f in (attn.to_q, attn.to_k, attn.to_v)]
-    if lat[0].shape[2] != heads * 128:
+    if lat[0].shape[2] != heads * hd:
         return None
     enc = None
     if dual:
@@ -199,7 +208,7 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
     elif lat[0].shape[1] != s:
         return None
     # every "this layer does not fit" exit is above: from here on the call is made
-    q, k, v = (torch.empty(b, heads, s, 128, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
+    q, k, v = (torch.empty(b, heads, s, hd, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
     plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, mask_cache=mask_cache)
     cut = lambda r, a, z: None if r is None else (r[0][a:z], r[1][a:z])
     if dual:
@@ -213,7 +222,7 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
                           **lat_norm)
         else:
             plan.qkv_prep(*lat, dst_row=0, rope=rope, rope_rows=n_rope, **lat_norm)
-    return plan.run_pooled().view(b, s, heads * 128)
+    return plan.run_pooled().view(b, s, heads * hd)
 
 
 class ProcessorBase:

@@ -72,7 +72,7 @@ EXPORTS = [
 _lib = None
 
 
-ABI_VERSION = 106
+ABI_VERSION = 107
 
 
 def lib():

@@ -128,8 +128,8 @@ COMPACT_ROPE = os.environ.get("RSA_COMPACT_ROPE", "1") != "0"     # tests switch
 def _compact_rope(cos_in, sin_in, cos, sin):
     """diffusers builds its real rotary tables with repeat_interleave(2): both elements of a pair see the same cos and
     the same sin.  When that holds (checked ONCE per table pair -- one host sync -- and remembered; the tables are
-    constants of a generation) the kernel is given one [rows, 64] table of (cos_i, sin_i) pairs instead of two
-    [rows, 128] tables.  Returns None for tables of any other form."""
+    constants of a generation) the kernel is given one [rows, head_dim / 2] table of (cos_i, sin_i) pairs instead of
+    two [rows, head_dim] tables.  Returns None for tables of any other form."""
     if not COMPACT_ROPE:
         return None
     # Keyed by storage, offset and version, and the entry keeps the caller's tensors (hence their storage) alive, so
@@ -257,16 +257,20 @@ class Plan:
     def qkv_prep(self, q_src, k_src, v_src, dst_row=0, q_weight=None, k_weight=None, eps=1e-6, rope=None,
                  rope_rows=None, pool=True, q_bias=None, k_bias=None):
         """Kernel 0: fills rows [dst_row, dst_row + rows) of this plan's q, k, v from projection outputs
-        [B, rows, H*128] (head split, per-head RMSNorm with bf16 weights, rotary embedding on the first `rope_rows`
-        tokens, re-layout) and, with pool=True, the pooled statistics of those blocks."""
+        [B, rows, H*head_dim] (head split, per-head RMSNorm or LayerNorm with bf16 parameters, rotary embedding on the
+        first `rope_rows` tokens, re-layout) and, with pool=True, the pooled statistics of those blocks.  head_dim 128
+        takes every norm; head_dim 64 (CogVideoX) takes LayerNorm only (q_weight, k_weight, q_bias, k_bias)."""
         b, h, s, d = self.shape
-        if self.q.dtype != torch.bfloat16 or d != 128:
-            raise RuntimeError("kernel 0 follows diffusers' bf16 rounding points and is built for 128 columns: "
-                               "bfloat16, head_dim 128 only")
+        if self.q.dtype != torch.bfloat16 or d not in (128, 64):
+            raise RuntimeError("kernel 0 follows diffusers' bf16 rounding points and is built for bfloat16 with "
+                               "head_dim 128 or 64")
+        if d == 64 and (q_weight is None or q_bias is None):
+            raise RuntimeError("kernel 0 at head_dim 64 is built for CogVideoX's LayerNorm: q_weight, k_weight, "
+                               "q_bias and k_bias are needed")
         for t, n in ((q_src, "q_src"), (k_src, "k_src"), (v_src, "v_src")):
             _need_cuda(t, n)
             if t.dtype != torch.bfloat16 or t.dim() != 3 or t.shape[0] != b or t.shape[2] != h * d or t.stride(2) != 1:
-                raise RuntimeError(f"{n} must be a bfloat16 [B, rows, H*128] tensor with contiguous channels")
+                raise RuntimeError(f"{n} must be a bfloat16 [B, rows, H*{d}] tensor with contiguous channels")
         rows = q_src.shape[1]
         if k_src.shape[1] != rows or v_src.shape[1] != rows:
             raise RuntimeError("q/k/v sources differ in length")

@@ -89,18 +89,20 @@ class FusedUlysses:
     """Ulysses sequence parallelism without data collectives (one process per GPU of one NVSwitch box).
 
     Rank r owns the consecutive tokens [r * rows, min((r + 1) * rows, S)), rows = ceil(S / P) (`self.local_rows` of
-    them: the last rank may hold fewer).  It writes its Q/K/V projection outputs [B, local_rows, H*128] into
+    them: the last rank may hold fewer).  It writes its Q/K/V projection outputs [B, local_rows, H*D] into
     peer-visible buffers (`self.q_src`, `self.k_src`, `self.v_src`); `run()` then
       1. barrier (one-element all_reduce: every rank's sources are written),
       2. kernel 0 in gather form: reads, for this rank's H/P heads, every token's rows straight from the owning rank's
-         buffer over NVLink, applies head split / RMSNorm / rotary embedding, stores local [B, H/P, S, 128] and pools,
+         buffer over NVLink, applies head split / RMSNorm or LayerNorm / rotary embedding, stores local [B, H/P, S, D]
+         and pools,
       3. kernels 3a-3c, kernel 4 with the scatter epilogue: every output row is stored straight into the owning rank's
-         result buffer [B, rows, H, 128],
+         result buffer [B, rows, H, D],
       4. barrier (every rank's scatter has landed),
-    and returns this rank's rows of the result, [B, rows, H*128] -- what `ulysses_attention` computes with two
-    all-to-alls (233 + 78 MB per GPU at C3a, P = 8) and two staging copies around the call."""
+    and returns this rank's rows of the result, [B, rows, H*D] -- what `ulysses_attention` computes with two
+    all-to-alls (233 + 78 MB per GPU at C3a, P = 8) and two staging copies around the call.
+    D = head_dim: 128, or 64 (CogVideoX; run() then needs the LayerNorm parameters q_weight, k_weight, q_bias, k_bias)."""
 
-    def __init__(self, batch, heads_total, geo, top_k, p_remain, nbr=None, group=None):
+    def __init__(self, batch, heads_total, geo, top_k, p_remain, nbr=None, group=None, head_dim=128):
         from . import native as N
         from . import ops
         import ctypes as C
@@ -110,6 +112,9 @@ class FusedUlysses:
             raise ValueError("at most 8 ranks (one NVSwitch box)")
         if heads_total < self.world:
             raise ValueError("every rank must compute at least one head")
+        if head_dim not in (128, 64):
+            raise ValueError("head_dim must be 128 or 64")
+        self.head_dim = hd = head_dim
         # heads need not divide by the ranks: the first (H mod P) ranks take one head more (12 heads on 8 ranks:
         # 2,2,2,2,1,1,1,1); this rank computes heads [head0, head0 + heads)
         base, extra = divmod(heads_total, self.world)
@@ -124,7 +129,7 @@ class FusedUlysses:
         self.device = torch.device("cuda", torch.cuda.current_device())
         L = N.lib()
         self._lib, self._own, self._opened = L, [], []
-        n_elems = batch * self.rows * heads_total * 128
+        n_elems = batch * self.rows * heads_total * hd
         ptrs = []
         # q, k, v sources, the result, and the per-token RMS statistics of q and k (Wan's norm across heads: every rank
         # computes them from the full rows of ITS tokens, the gathering ranks read them over NVLink)
@@ -149,11 +154,11 @@ class FusedUlysses:
                     self._opened.append(pp.value)
                     table[t, r] = pp.value
         self._table = table.to(self.device)
-        shape = (batch, self.rows, heads_total * 128)
+        shape = (batch, self.rows, heads_total * hd)
         # views of this rank's own rows (the buffers themselves hold `rows` rows on every rank)
         self.q_src, self.k_src, self.v_src, self.out = (_peer_tensor(p, shape)[:, :self.local_rows] for p in self._own[:4])
         self._flag = torch.zeros(1, device=self.device)
-        q, k, v = (torch.empty(batch, self.heads, self.seq, 128, dtype=torch.bfloat16, device=self.device)
+        q, k, v = (torch.empty(batch, self.heads, self.seq, hd, dtype=torch.bfloat16, device=self.device)
                    for _ in range(3))
         self.plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, private_workspace=True)
         route = N.PeerRoute()
@@ -161,27 +166,38 @@ class FusedUlysses:
         route.head0 = self.head0
         route.src_table = self._table[:3].data_ptr()
         route.out_table = self._table[3].data_ptr()
-        route.src_stride[0], route.src_stride[1] = self.rows * heads_total * 128, heads_total * 128
-        route.out_stride[0], route.out_stride[1] = self.rows * heads_total * 128, heads_total * 128
+        route.src_stride[0], route.src_stride[1] = self.rows * heads_total * hd, heads_total * hd
+        route.out_stride[0], route.out_stride[1] = self.rows * heads_total * hd, heads_total * hd
         route.rinv_table = self._table[4:6].data_ptr()
         self.route = route
 
     def _barrier(self):
         dist.all_reduce(self._flag, group=self.group)       # stream-ordered, one element: nothing but a barrier
 
-    def run(self, q_weight=None, k_weight=None, eps=1e-6, rope=None, rope_rows=None):
+    def run(self, q_weight=None, k_weight=None, eps=1e-6, rope=None, rope_rows=None, q_bias=None, k_bias=None):
+        """q_weight / k_weight: RMSNorm weights ([128] per head, or [heads_total*128] across heads); with q_bias /
+        k_bias: LayerNorm over head_dim (CogVideoX), the only norm at head_dim 64."""
         from . import native as N
         from . import ops
         import ctypes as C
         plan = self.plan
+        hd = self.head_dim
         p = N.PrepDesc()
         p.rows, p.dst_row = self.seq, 0
         keep = []
+        if hd == 64 and (q_weight is None or q_bias is None):
+            raise RuntimeError("head_dim 64 is built for CogVideoX's LayerNorm: q_weight, k_weight, q_bias, k_bias")
         if q_weight is not None:
             ws_ = [w.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for w in (q_weight, k_weight)]
             keep += ws_
             p.norm, p.eps, p.q_weight, p.k_weight = 1, float(eps), ws_[0].data_ptr(), ws_[1].data_ptr()
-            if all(w.numel() == self.heads_total * 128 for w in ws_):
+            if q_bias is not None or k_bias is not None:    # LayerNorm over head_dim (CogVideoX)
+                bs_ = [x.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for x in (q_bias, k_bias)]
+                if any(x.numel() != hd for x in ws_ + bs_):
+                    raise RuntimeError("LayerNorm weights and biases must have head_dim elements")
+                keep += bs_
+                p.norm, p.q_bias, p.k_bias = 3, bs_[0].data_ptr(), bs_[1].data_ptr()
+            elif all(w.numel() == self.heads_total * 128 for w in ws_):
                 # RMSNorm over all heads*128 channels of a token (Wan, rectified_wan21_attn.py:423-426): the statistic
                 # needs whole rows, which only the owning rank holds -> computed here, before the barrier
                 p.norm = 2

@@ -1,4 +1,5 @@
-"""Multi-GPU check + measurement of the fused Ulysses exchange (run under torchrun on 2, 4 or 8 GPUs of one box):
+"""Multi-GPU check + measurement of the fused Ulysses exchange (run under torchrun on 2, 4 or 8 GPUs of one box;
+workload name as the argument: a bench.py workload, or "odd" / "cog" below):
   * rank r holds tokens [r*S/P, (r+1)*S/P) of the projection outputs; FusedUlysses.run() must return exactly the rows a
     single-GPU call over all heads produces (heads are independent, same kernels => bit-identical),
   * the NCCL form (two all-to-alls around kernel 0 + the pooled call, rsa_b200.parallel.ulysses_attention-style) gives
@@ -28,35 +29,45 @@ if name == "odd":
     # fewer rows, the first rank(s) compute one head more
     bench.WORKLOADS["odd"] = dict(desc="uneven token and head shards", fam="wan", grid=(5, 9, 23), text=0, text_valid=0,
                                   heads=3, drop=0.6, ffb=True)
+if name == "cog":
+    # CogVideoX form: 64-column heads, LayerNorm(64) with bias, rotary embedding on the video tokens; 2 x 8 x 24 = 384
+    # video + 227 text = 611 tokens and 3 heads, so neither divides by 2 ranks
+    bench.WORKLOADS["cog"] = dict(desc="CogVideoX form, uneven token and head shards", fam="cog", grid=(2, 8, 24),
+                                  text=227, text_valid=227, heads=3, drop=0.5, ffb=False)
 wp = bench.workload_params(name)
 heads, s, nv = wp["heads"], wp["s"], wp["nv"]
+cog = wp["fam"] == "cog"
+hd = 64 if cog else 128                             # head_dim
 geo = bench.product_geometry(wp)
 t, h, w = wp["grid"]
 nbr = ops.gilbert_block_neighbors(t, h, w)
 rows, hl = -(-s // world), heads // world          # rows per rank (the last rank may own fewer)
 even = rows * world == s and hl * world == heads      # the NCCL form below is written for even shards only
 g = torch.Generator(device=dev).manual_seed(1234)                       # same stream on every rank: the full tensors
-full = [torch.randn(1, s, heads * 128, generator=g, device=dev).to(torch.bfloat16) for _ in range(3)]
+full = [torch.randn(1, s, heads * hd, generator=g, device=dev).to(torch.bfloat16) for _ in range(3)]
 if wp["fam"] != "wan":                                                   # give the pooled scores some structure
-    mu = torch.cumsum(torch.randn(1, (s + 127) // 128, heads * 128, generator=g, device=dev) * 0.35, dim=1)
+    mu = torch.cumsum(torch.randn(1, (s + 127) // 128, heads * hd, generator=g, device=dev) * 0.35, dim=1)
     for x in full[:2]:
         x.add_(mu.repeat_interleave(128, dim=1)[:, :s].to(torch.bfloat16))
 wan = wp["fam"] == "wan"     # Wan: RMSNorm over all heads*128 channels of a token, rotary embedding on every token
-nw = heads * 128 if wan else 128
+nw = heads * 128 if wan else hd
 wq = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(torch.bfloat16)
 wk = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(torch.bfloat16)
-ang = torch.outer(torch.arange(nv, dtype=torch.float32, device=dev), 1.0 / (256.0 ** (torch.arange(0, 128, 2, device=dev) / 128)))
+# CogVideoX: LayerNorm(head_dim) with bias on q and k
+norm_kw = dict(q_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(torch.bfloat16),
+               k_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(torch.bfloat16)) if cog else {}
+ang = torch.outer(torch.arange(nv, dtype=torch.float32, device=dev), 1.0 / (256.0 ** (torch.arange(0, hd, 2, device=dev) / hd)))
 rope = (ang.cos().repeat_interleave(2, 1).contiguous(), ang.sin().repeat_interleave(2, 1).contiguous())
 mine = slice(rank * rows, min((rank + 1) * rows, s))
 
-fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr)
+fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr, head_dim=hd)
 for dst, src in zip((fu.q_src, fu.k_src, fu.v_src), full):
     dst.copy_(src[:, mine])
-out = fu.run(wq, wk, 1e-6, rope, nv).clone()
+out = fu.run(wq, wk, 1e-6, rope, nv, **norm_kw).clone()
 torch.cuda.synchronize()
 
 # NCCL form: all-to-all the projection rows to head shards, kernel 0 + pooled call locally, all-to-all the result back
-q, k, v = (torch.empty(1, max(hl, 1), s, 128, dtype=torch.bfloat16, device=dev) for _ in range(3))
+q, k, v = (torch.empty(1, max(hl, 1), s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
 plan = ops.Plan(q, k, v, geo, wp["top_k"], bench.P_REMAIN, nbr)
 
 
@@ -72,19 +83,19 @@ def nccl_form():
         loc = x[:, mine]
         if wan and i < 2:      # the norm needs whole rows: before the exchange, on the tokens this rank owns
             loc = wan_norm(loc, wq if i == 0 else wk)
-        loc = loc.reshape(1, rows, world, hl * 128).permute(2, 0, 1, 3).contiguous()   # [P(dst), 1, rows, hl*128]
+        loc = loc.reshape(1, rows, world, hl * hd).permute(2, 0, 1, 3).contiguous()    # [P(dst), 1, rows, hl*hd]
         rcv = torch.empty_like(loc)
         dist.all_to_all_single(rcv, loc)
-        srcs.append(rcv.permute(1, 0, 2, 3).reshape(1, s, hl * 128))                         # all tokens, my heads
+        srcs.append(rcv.permute(1, 0, 2, 3).reshape(1, s, hl * hd))                          # all tokens, my heads
     if wan:
         plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv)
     elif geo.gap:
         plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope)
         plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6)
     else:
-        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv)
-    o = plan.run_pooled()                                                                     # [1, S, hl, 128]
-    return parallel.head_to_seq_shard(o).reshape(1, rows, heads * 128)
+        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, **norm_kw)
+    o = plan.run_pooled()                                                                     # [1, S, hl, hd]
+    return parallel.head_to_seq_shard(o).reshape(1, rows, heads * hd)
 
 
 # (the NCCL form below is written for even shards; with uneven ones the single-GPU call is the only reference)
@@ -97,14 +108,14 @@ frac_equal_nccl = float((out.view(torch.int16) == ref.view(torch.int16)).float()
 same_as_single = None
 if check and (rank == 0 or not even):       # uneven shards: every rank checks its own rows (the shapes are small)
     # one GPU, all heads, no exchange at all
-    qa, ka, va = (torch.empty(1, heads, s, 128, dtype=torch.bfloat16, device=dev) for _ in range(3))
+    qa, ka, va = (torch.empty(1, heads, s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
     pa = ops.Plan(qa, ka, va, geo, wp["top_k"], bench.P_REMAIN, nbr)
     if geo.gap:
         pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope)
         pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6)
     else:
-        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv)
-    single = pa.run_pooled().reshape(1, s, heads * 128)[:, mine]
+        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, **norm_kw)
+    single = pa.run_pooled().reshape(1, s, heads * hd)[:, mine]
     torch.cuda.synchronize()
     same_as_single = bool(torch.equal(out.view(torch.int16), single.view(torch.int16)))
     del qa, ka, va, pa
@@ -127,16 +138,16 @@ def timed(fn, n=10):
     return float(tt.item())
 
 
-ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, nv))
+ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, nv, **norm_kw))
 ms_nccl = timed(nccl_form) if even else None
 oks = [None] * world
 dist.all_gather_object(oks, same_as_nccl)
 singles = [None] * world
 dist.all_gather_object(singles, same_as_single)
 if rank == 0:
-    print(json.dumps({"workload": name, "n_gpus": world, "tokens": s, "heads": heads,
+    print(json.dumps({"workload": name, "n_gpus": world, "tokens": s, "heads": heads, "head_dim": hd,
                       "fused_ms_per_layer_attention": ms_fused, "nccl_all_to_all_form_ms": ms_nccl,
-                      "norm": "across heads (Wan)" if wan else "per head",
+                      "norm": "across heads (Wan)" if wan else ("LayerNorm per head (CogVideoX)" if cog else "per head"),
                       "fused_equals_nccl_form_bitwise_all_ranks": all(oks),
                       "fraction_of_elements_equal_to_nccl_form_rank0": frac_equal_nccl,
                       "fused_equals_single_gpu_bitwise_rank0": same_as_single,
