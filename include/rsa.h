@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define RSA_VERSION 107 /* 107: kernel 0 and the fused Ulysses exchange take head_dim 64 (norm 3) */
+#define RSA_VERSION 108 /* 108: rsa_dense_attention, rsa_dense_attention_scatter (kernel 4 without lists) */
 #define RSA_BLOCK 128
 #define RSA_HEAD_DIM 128
 #define RSA_MAX_ENTRIES 2048 /* max sortable entries per query block: NQ (+1 for the text aggregate) */
@@ -350,6 +350,25 @@ int rsa_masked_attention(const void* q, const void* k, const void* v, void* out,
                          const int64_t v_stride[2], const int64_t o_stride[2], const uint8_t* block_mask,
                          int n_q_blocks, int n_kv_blocks, void* workspace, size_t workspace_bytes, void* stream,
                          int dtype /* enum rsa_dtype */, int head_dim /* 128 or 64 */);
+
+/* Dense attention: kernel 4 walking every key block of every query tile, without lists, mask or workspace.  Replaces
+ * fullattn(mode="flash") (attn.py:107-120, flash_attn_varlen_func) with the cu_seqlens the processors pass,
+ * [0, q_valid, S] for the queries and [0, kv_len, S] for the keys: query rows >= q_valid are written as zeros, keys
+ * >= kv_len are never attended.  Flash-attn's arithmetic (the fp32 scores are scaled; what RSA_ATTN_FP32_SCALE selects
+ * in rsa_masked_attention), and the result is bit-identical to rsa_masked_attention on an all-ones mask with that flag
+ * (rows >= q_valid zeroed): the walk is the pair schedule of all-ones lists in closed form.
+ * Reads only batch, heads, seq (= query rows), head_dim (128 or 64), the four stride triples and dtype (bf16 or fp16)
+ * of `d`; the block-geometry fields are neither read nor validated.  q is [batch, heads, seq, head_dim], k and v are
+ * [batch, heads, seq_kv, head_dim] (seq_kv may differ from seq), out is [batch, heads, seq, head_dim], all through the
+ * descriptor's strides (multiples of 8 elements, 16-byte aligned bases).  Needs 1 <= q_valid <= seq and
+ * 1 <= kv_len <= seq_kv.  RSA_TC5_POLY and the debug dump do not apply to this form. */
+int rsa_dense_attention(const rsa_attn_desc* d, const void* q, const void* k, const void* v, void* out, int seq_kv,
+                        int q_valid, int kv_len, void* stream);
+/* The same with the fused Ulysses scatter epilogue of rsa_rectified_attention_pooled_scatter: every output row is stored
+ * into the owning rank's result buffer (route->out_table); seq_kv = seq (q, k, v come from rsa_qkv_prep_gather with
+ * pool = 0).  The route is validated as there, and head_dim 64 is refused under the debug dump or attention flag 4. */
+int rsa_dense_attention_scatter(const rsa_attn_desc* d, const void* q, const void* k, const void* v,
+                                const rsa_peer_route* route, int q_valid, int kv_len, void* stream);
 
 /* Bring-up hook (tests only): while non-null, the tcgen05 kernel's CTA for query tile 0 of batch*head 0 writes, as
  * fp32, S of its first kept block [128x128], the un-normalised O [128x128], the row sums l [128] and the row

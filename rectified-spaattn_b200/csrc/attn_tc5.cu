@@ -107,7 +107,11 @@ constexpr int kTraceBase = 33024, kTraceSteps = 64, kTraceSlots = 16;
 // 64 can still run here: its tensor maps zero-fill the second granule).  64 (CogVideoX): one granule per tile, S = Q K^T
 // over 4 k-steps instead of 8, O = P V as N = 64 MMAs into 64 TMEM columns -- 640 instead of 1024 tensor-pipe cycles
 // per kept pair, half the K/V bytes; the softmax side is the same, so this form is MUFU-bound rather than tensor-bound.
-template <bool kDebug, int kPolyPairs, bool kF16 = false, int kD = 128>
+// kDense: every query tile walks key blocks 0 .. ceil(kv_len/128) - 1 and no list, schedule, R or C is read (dense
+// attention, rsa_dense_attention).  The walk is what pair_schedule_kernel makes of all-ones lists, in closed form: the
+// lists are ascending, a pair of two tiles shares all of them (nsh), and partner pairs share all of them too (nq4), so
+// the result is bit-identical to the listed form on an all-ones mask.
+template <bool kDebug, int kPolyPairs, bool kF16 = false, int kD = 128, bool kDense = false>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                 const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmQt,
@@ -128,13 +132,14 @@ attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   const int64_t lrow0 = (int64_t)bh * a.nqt + tile0;
   // counts and prefix length are clamped so that a workspace that never saw a build (mask re-use misused) yields
   // garbage values, not an unbounded walk; out-of-range block numbers read as zero tiles through TMA
-  const int cnt0 = min(max(a.kept_cnt[lrow0], 0), a.nb);
-  const int cnt1 = tile1 < a.nqt ? min(max(a.kept_cnt[lrow0 + 1], 0), a.nb) : 0;
+  const int ndense = kDense ? (a.kv_len + 127) / 128 : 0;
+  const int cnt0 = kDense ? ndense : min(max(a.kept_cnt[lrow0], 0), a.nb);
+  const int cnt1 = tile1 < a.nqt ? (kDense ? ndense : min(max(a.kept_cnt[lrow0 + 1], 0), a.nb)) : 0;
   // the pair schedule (rsa_api.cu: pair_schedule_kernel): both lists start with the nsh blocks the two tiles have in
   // common, in the same order, so over rounds [0, nsh) one K tile and one V tile serve both slots
-  const uint16_t* __restrict__ list0 = (repair ? a.kept_idx : a.sched_idx) + lrow0 * a.nb;
-  const uint16_t* __restrict__ list1 = list0 + a.nb;
-  const int nsh = repair ? min(cnt0, cnt1)
+  const uint16_t* __restrict__ list0 = kDense ? nullptr : (repair ? a.kept_idx : a.sched_idx) + lrow0 * a.nb;
+  const uint16_t* __restrict__ list1 = kDense ? nullptr : list0 + a.nb;
+  const int nsh = (kDense || repair) ? min(cnt0, cnt1)
                          : min(max(a.pair_shared[(int64_t)bh * n_pairs + pair], 0), min(cnt0, cnt1));
   const int rounds = max(cnt0, cnt1);
   // The common prefix of the two partner pairs (pair, pair ^ 1; see the header) is walked by every pair, but only a
@@ -146,7 +151,9 @@ attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   if (kD == 128 && !kDebug && !(a.dbg_flags & 32) && !repair && pair < vis_pairs && (pair ^ 1) < vis_pairs && ((int)blockIdx.x ^ 1) < total_ctas) {
     const GridSlot gp = attention_grid_slot((int)blockIdx.x ^ 1, a.nqt, a.nq_vis, a.batch * a.heads, a.front_text_heads,
                                             (a.dbg_flags & 16) != 0);
-    if (!gp.repaired && gp.bh == bh && gp.pair == (pair ^ 1)) {
+    if (kDense && !gp.repaired && gp.bh == bh && gp.pair == (pair ^ 1)) {
+      nq4 = ndense;  // both pairs have two tiles (pair, pair ^ 1 < vis_pairs), so every block is common to all four
+    } else if (!kDense && !gp.repaired && gp.bh == bh && gp.pair == (pair ^ 1)) {
       const int64_t prow = (int64_t)bh * a.nqt + gp.tile0;
       const int pc0 = min(max(a.kept_cnt[prow], 0), a.nb), pc1 = min(max(a.kept_cnt[prow + 1], 0), a.nb);
       const int pnsh = min(max(a.pair_shared[(int64_t)bh * n_pairs + gp.pair], 0), min(pc0, pc1));
@@ -224,8 +231,8 @@ attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       int mine0 = 0, mine1 = 0, prev0 = 0, prev1 = 0;
       for (int r = 0; r <= rounds; ++r) {
         if ((r & 31) == 0) {
-          mine0 = (r + lane < cnt0) ? (int)list0[r + lane] : 0;
-          mine1 = (r + lane < cnt1) ? (int)list1[r + lane] : 0;
+          mine0 = (r + lane < cnt0) ? (kDense ? r + lane : (int)list0[r + lane]) : 0;
+          mine1 = (r + lane < cnt1) ? (kDense ? r + lane : (int)list1[r + lane]) : 0;
         }
         const int cur0 = __shfl_sync(0xffffffffu, mine0, r & 31);
         const int cur1 = __shfl_sync(0xffffffffu, mine1, r & 31);
@@ -397,7 +404,7 @@ attn_tc5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         RSA_TRACE(tr, i, 0);
         // valid keys in this block (the schedule is not ascending): the end of the valid keys, and the end of the
         // visual tokens inside the last visual block (zero rows that pad it are never attended)
-        const int blk = (int)list[i];
+        const int blk = kDense ? i : (int)list[i];
         int lim = a.kv_len - blk * 128;
         if (blk < a.nq_vis) lim = min(lim, a.vis_len - blk * 128);
         mbar_wait(bar(B_SFULL + s), i & 1);
@@ -654,11 +661,11 @@ struct Maps {
   CUtensorMap q, k, v, qt, kt, vt;
 };
 
-template <bool kDebug, int kPolyPairs, bool kF16 = false, int kD = 128>
+template <bool kDebug, int kPolyPairs, bool kF16 = false, int kD = 128, bool kDense = false>
 int launch(dim3 grid, cudaStream_t s, const Maps& m, const AttnArgs& a) {
   static bool configured = false;  // one flag per instantiation
   if (!configured) {
-    RSA_CUDA_CHECK(cudaFuncSetAttribute(attn_tc5_kernel<kDebug, kPolyPairs, kF16, kD>,
+    RSA_CUDA_CHECK(cudaFuncSetAttribute(attn_tc5_kernel<kDebug, kPolyPairs, kF16, kD, kDense>,
                                         cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
     configured = true;
   }
@@ -675,7 +682,7 @@ int launch(dim3 grid, cudaStream_t s, const Maps& m, const AttnArgs& a) {
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  RSA_CUDA_CHECK(cudaLaunchKernelEx(&cfg, attn_tc5_kernel<kDebug, kPolyPairs, kF16, kD>, m.q, m.k, m.v, m.qt, m.kt, m.vt, a));
+  RSA_CUDA_CHECK(cudaLaunchKernelEx(&cfg, attn_tc5_kernel<kDebug, kPolyPairs, kF16, kD, kDense>, m.q, m.k, m.v, m.qt, m.kt, m.vt, a));
   return RSA_OK;
 }
 
@@ -688,9 +695,20 @@ int poly_pairs(int dflt = kDefaultPolyPairs) {
   return v >= 0 ? v : dflt;
 }
 
+// The list-free dense form (kDense): flash-attn's arithmetic (q_round = 0), default polynomial setting, no debug dump.
+// With attention flag 4 a 64-column tensor runs the 128-column form, as in launch_attention_tc5.
+static int launch_dense(const Maps& m, const AttnArgs& a, cudaStream_t s) {
+  const dim3 grid((unsigned)((a.nqt + 1) / 2) * (unsigned)(a.batch * a.heads));
+  if (a.head_dim == 64 && !(a.dbg_flags & 4))
+    return a.f16 ? launch<false, kDefaultPolyPairs64, true, 64, true>(grid, s, m, a)
+                 : launch<false, kDefaultPolyPairs64, false, 64, true>(grid, s, m, a);
+  return a.f16 ? launch<false, kDefaultPolyPairs, true, 128, true>(grid, s, m, a)
+               : launch<false, kDefaultPolyPairs, false, 128, true>(grid, s, m, a);
+}
+
 }  // namespace
 
-int launch_attention_tc5(const AttnArgs& a, cudaStream_t s) {
+int launch_attention_tc5(const AttnArgs& a, cudaStream_t s, bool dense) {
   if (a.nqt == 0) return RSA_OK;
   Maps m;
   int rc;
@@ -706,6 +724,7 @@ int launch_attention_tc5(const AttnArgs& a, cudaStream_t s) {
     if ((rc = make_map(&m.kt, a.k + (int64_t)vis_kv * a.ks[2], a.batch, a.heads, a.seq_kv - vis_kv, a.ks, a.f16 != 0, a.head_dim)) != RSA_OK) return rc;
     if ((rc = make_map(&m.vt, a.v + (int64_t)vis_kv * a.vs[2], a.batch, a.heads, a.seq_kv - vis_kv, a.vs, a.f16 != 0, a.head_dim)) != RSA_OK) return rc;
   }
+  if (dense) return launch_dense(m, a, s);
   const dim3 grid((unsigned)((a.nqt + 1) / 2) * (unsigned)(a.batch * a.heads));
   if (a.head_dim == 64 && !a.dbg && !(a.dbg_flags & 4)) {  // the 64-column instantiations (the debug kernel stays 128 wide)
     if (a.f16) return launch<false, kDefaultPolyPairs64, true, 64>(grid, s, m, a);

@@ -728,3 +728,88 @@ extern "C" int rsa_masked_attention(const void* q, const void* k, const void* v,
   a.dbg_flags = g_attention_dbg_flags;
   return launch_attention(a, s);
 }
+
+// Dense attention without lists (kernel 4's kDense form): only batch, heads, seq, head_dim, the strides and dtype of the
+// descriptor are read.  Every refusal happens here, before any CUDA call.
+static int validate_dense(const rsa_attn_desc* d, const void* q, const void* k, const void* v, const void* out,
+                          bool scatter, int seq_kv, int q_valid, int kv_len, const char* fn) {
+  if (!d || !q || !k || !v || (!scatter && !out)) RSA_FAIL(RSA_ERR_ARG, "%s: null pointer", fn);
+  if (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "%s: head_dim must be 128 or 64 (got %d)", fn, d->head_dim);
+  if (d->dtype != RSA_DTYPE_BF16 && d->dtype != RSA_DTYPE_F16)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "%s: dtype %d is not one of rsa_dtype (bf16, fp16)", fn, d->dtype);
+  if (d->batch <= 0 || d->heads <= 0 || d->seq <= 0 || seq_kv <= 0)
+    RSA_FAIL(RSA_ERR_ARG, "%s: batch/heads/seq/seq_kv must be positive", fn);
+  if ((int64_t)d->batch * d->heads > 65535) RSA_FAIL(RSA_ERR_UNSUPPORTED, "%s: batch*heads > 65535", fn);
+  if (q_valid < 1 || q_valid > d->seq) RSA_FAIL(RSA_ERR_ARG, "%s: q_valid=%d out of [1, seq=%d]", fn, q_valid, d->seq);
+  if (kv_len < 1 || kv_len > seq_kv) RSA_FAIL(RSA_ERR_ARG, "%s: kv_len=%d out of [1, seq_kv=%d]", fn, kv_len, seq_kv);
+  const int64_t* st[4] = {d->q_stride, d->k_stride, d->v_stride, d->o_stride};
+  for (int t = 0; t < (scatter ? 3 : 4); ++t)
+    for (int i = 0; i < 3; ++i)
+      if (st[t][i] < 0 || st[t][i] % 8)
+        RSA_FAIL(RSA_ERR_UNSUPPORTED, "%s: strides must be non-negative multiples of 8 elements (16 bytes)", fn);
+  if (((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)(scatter ? nullptr : out)) % 16)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "%s: q/k/v/out must be 16-byte aligned", fn);
+  return RSA_OK;
+}
+
+static void fill_dense_args(const rsa_attn_desc* d, const void* q, const void* k, const void* v, void* out, int seq_kv,
+                            int q_valid, int kv_len, AttnArgs* a) {
+  memset(a, 0, sizeof(*a));
+  a->q = (const __nv_bfloat16*)q;
+  a->k = (const __nv_bfloat16*)k;
+  a->v = (const __nv_bfloat16*)v;
+  a->o = (__nv_bfloat16*)out;
+  a->batch = d->batch;
+  a->heads = d->heads;
+  for (int i = 0; i < 3; ++i) {
+    a->qs[i] = d->q_stride[i];
+    a->ks[i] = d->k_stride[i];
+    a->vs[i] = d->v_stride[i];
+    a->os[i] = d->o_stride[i];
+  }
+  a->seq_q = d->seq;
+  a->seq_kv = seq_kv;
+  a->kv_len = kv_len;
+  a->q_valid = q_valid;
+  a->vis_len = 1 << 30;  // no text segment: every block is "visual", nothing is shifted (as rsa_masked_attention)
+  a->nq_vis = 1 << 20;
+  a->gap = 0;
+  a->nqt = (d->seq + RSA_BLOCK - 1) / RSA_BLOCK;
+  a->nb = (seq_kv + RSA_BLOCK - 1) / RSA_BLOCK;
+  a->scale_log2 = (float)((1.0 / sqrt((double)d->head_dim)) * 1.44269504);
+  a->head_dim = d->head_dim;
+  a->rescale_thr = attention_rescale_threshold(d->dtype == RSA_DTYPE_F16);
+  a->front_text_heads = 0;
+  a->f16 = d->dtype == RSA_DTYPE_F16;
+  a->q_round = 0;        // flash-attn's arithmetic: the fp32 scores are scaled, q is not rounded
+  a->dbg = nullptr;      // the dense form has no debug dump
+  a->dbg_flags = g_attention_dbg_flags;
+}
+
+extern "C" int rsa_dense_attention(const rsa_attn_desc* d, const void* q, const void* k, const void* v, void* out,
+                                   int seq_kv, int q_valid, int kv_len, void* stream) {
+  int rc = validate_dense(d, q, k, v, out, false, seq_kv, q_valid, kv_len, "rsa_dense_attention");
+  if (rc != RSA_OK) return rc;
+  AttnArgs a;
+  fill_dense_args(d, q, k, v, out, seq_kv, q_valid, kv_len, &a);
+  return launch_attention_tc5(a, (cudaStream_t)stream, true);
+}
+
+extern "C" int rsa_dense_attention_scatter(const rsa_attn_desc* d, const void* q, const void* k, const void* v,
+                                           const rsa_peer_route* route, int q_valid, int kv_len, void* stream) {
+  int rc = validate_dense(d, q, k, v, nullptr, true, d ? d->seq : 0, q_valid, kv_len, "rsa_dense_attention_scatter");
+  if (rc != RSA_OK) return rc;
+  if ((rc = validate_route(d, route, false, true)) != RSA_OK) return rc;
+  // as rsa_rectified_attention_pooled_scatter: the epilogue places head h at (head0 + h) * head_dim of the instantiation
+  if (d->head_dim == 64 && (g_attention_dbg || (g_attention_dbg_flags & 4)))
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_dense_attention_scatter: head_dim 64 runs the 64-column kernel 4 only");
+  AttnArgs a;
+  fill_dense_args(d, q, k, v, nullptr, d->seq, q_valid, kv_len, &a);
+  a.o_table = (__nv_bfloat16* const*)route->out_table;
+  a.peer_rows = route->rows_per_rank;
+  a.peer_head0 = route->head0;
+  a.peer_os[0] = route->out_stride[0];
+  a.peer_os[1] = route->out_stride[1];
+  return launch_attention_tc5(a, (cudaStream_t)stream, true);
+}

@@ -164,7 +164,9 @@ struct AttnArgs {
 };
 
 int launch_attention_mma(const AttnArgs& a, cudaStream_t s);      // mma.sync cross-check kernel: tests/xcheck only, not in the product library
-int launch_attention_tc5(const AttnArgs& a, cudaStream_t s);      // tcgen05 / TMEM / TMA kernel
+// tcgen05 / TMEM / TMA kernel; dense = true: the list-free form (every tile walks blocks 0 .. ceil(kv_len/128) - 1;
+// kept_idx, kept_cnt, sched_idx, pair_shared, quad_shared, R and C are not read)
+int launch_attention_tc5(const AttnArgs& a, cudaStream_t s, bool dense = false);
 int launch_pair_schedule(const AttnArgs& a, cudaStream_t s);  // kept lists -> sched_idx / pair_shared
 int launch_mask_to_lists(const uint8_t* mask, int bh, int nq, int nkv, int kv_blocks_valid, uint16_t* kept_idx,
                          int32_t* kept_cnt, cudaStream_t s);

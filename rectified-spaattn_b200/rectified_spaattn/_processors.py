@@ -161,12 +161,15 @@ def rope_tables(emb, n, head_dim=128):
 
 
 def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k, p_remain, nbr, image_rotary_emb,
-                         rope_text, mask_cache=None):
+                         rope_text, mask_cache=None, dense=False):
     """The fused form of a joint-text processor's middle section (kernel 0 + kernels 3a-4): projections ->
     rsa_qkv_prep (head split, RMSNorm / LayerNorm, RoPE, re-layout, pooling) -> rsa_rectified_attention_pooled.  Returns
     [B, S, H*D], or None when this layer does not have the shape kernel 0 fuses (the caller then runs the op-by-op path).
     D (head_dim) is read from `to_q`'s output width: 128, or 64 (CogVideoX, LayerNorm only).
-    `rope_text`: Flux rotates the text tokens too (their table rows follow the image rows); HunyuanVideo does not."""
+    `rope_text`: Flux rotates the text tokens too (their table rows follow the image rows); HunyuanVideo does not.
+    `dense`: the call the op-by-op path sends to fullattn(mode="flash") -- kernel 0 without pooling, then dense
+    attention over the first `geo.kv_len - geo.gap` memory rows (num_true for HunyuanVideo, S otherwise) as queries
+    and keys; top_k, p_remain, nbr and mask_cache are not used."""
     from rsa_b200 import ops
     heads = attn.heads
     if not hidden_states.is_cuda or hidden_states.dtype != torch.bfloat16:
@@ -209,19 +212,23 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
         return None
     # every "this layer does not fit" exit is above: from here on the call is made
     q, k, v = (torch.empty(b, heads, s, hd, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
-    plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, mask_cache=mask_cache)
+    plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, mask_cache=None if dense else mask_cache)
     cut = lambda r, a, z: None if r is None else (r[0][a:z], r[1][a:z])
+    pool = not dense
     if dual:
-        plan.qkv_prep(*lat, dst_row=0, rope=cut(rope, 0, nv), **lat_norm)
-        plan.qkv_prep(*enc, dst_row=nv, rope=cut(rope, nv, s) if rope_text else None, **enc_norm)
+        plan.qkv_prep(*lat, dst_row=0, rope=cut(rope, 0, nv), pool=pool, **lat_norm)
+        plan.qkv_prep(*enc, dst_row=nv, rope=cut(rope, nv, s) if rope_text else None, pool=pool, **enc_norm)
     else:
         n_rope = 0 if rope is None else (s if rope_text else nv)
         if geo.gap:     # ragged visual segment: the two segments are separate block ranges
-            plan.qkv_prep(*(t[:, :nv] for t in lat), dst_row=0, rope=cut(rope, 0, nv), **lat_norm)
+            plan.qkv_prep(*(t[:, :nv] for t in lat), dst_row=0, rope=cut(rope, 0, nv), pool=pool, **lat_norm)
             plan.qkv_prep(*(t[:, nv:] for t in lat), dst_row=nv, rope=cut(rope, nv, s) if rope_text else None,
-                          **lat_norm)
+                          pool=pool, **lat_norm)
         else:
-            plan.qkv_prep(*lat, dst_row=0, rope=rope, rope_rows=n_rope, **lat_norm)
+            plan.qkv_prep(*lat, dst_row=0, rope=rope, rope_rows=n_rope, pool=pool, **lat_norm)
+    if dense:
+        n_valid = geo.kv_len - geo.gap      # memory rows: kv_len counts the gap rows of a ragged visual segment
+        return plan.run_dense(n_valid, n_valid).view(b, s, heads * hd)
     return plan.run_pooled().view(b, s, heads * hd)
 
 
@@ -231,6 +238,9 @@ class ProcessorBase:
 
     steps_per_cycle = 50  # `current_step` wraps to 0 after this many calls
     fuse_prep = True      # joint-text processors: run head split / QK norm / RoPE / pooling as kernel 0 when the layer allows
+    # the same for the calls that go to fullattn(mode="flash") (warm-up calls, dense layers, mode "flash"): kernel 0
+    # without pooling, then kernel 4's list-free dense form.  Off by default: the op-by-op route stays the reference's.
+    fuse_prep_dense = False
 
     def __init__(self, mode, select_block_num, block_neighbor_list, p_remain_rates, processor_id=0):
         self.mode = mode
@@ -292,10 +302,11 @@ class WanProcessorBase(ProcessorBase):
     def sparse_now(self) -> bool:
         raise NotImplementedError
 
-    def _fused(self, attn, hidden_states, rotary_emb, enc_img):
+    def _fused(self, attn, hidden_states, rotary_emb, enc_img, dense=False):
         """Kernel 0 form of the middle section (reference rectified_wan21_attn.py:419-470): projections -> RMSNorm across
         heads + rotary embedding + head split + pooling in one pass -> kernels 3a-4.  None when the layer does not have
-        the shape kernel 0 fuses."""
+        the shape kernel 0 fuses.  `dense`: a warm-up call or dense layer -- kernel 0 without pooling, then dense
+        attention over all S tokens."""
         from rsa_b200 import geometry as G
         from rsa_b200 import ops
         heads = attn.heads
@@ -315,9 +326,9 @@ class WanProcessorBase(ProcessorBase):
             return None
         q, k, v = (torch.empty(b, heads, s, 128, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
         plan = ops.Plan(q, k, v, G.wan(s, self.first_frame_blocks), self.select_block_num, self.p_remain_rates,
-                        self.block_neighbor_list, mask_cache=self._mask_cache())
-        plan.qkv_prep(*src, dst_row=0, q_weight=nq_[0], k_weight=nk_[0], eps=nq_[1], rope=rope)
-        out = plan.run_pooled().view(b, s, heads * 128)
+                        self.block_neighbor_list, mask_cache=None if dense else self._mask_cache())
+        plan.qkv_prep(*src, dst_row=0, q_weight=nq_[0], k_weight=nk_[0], eps=nq_[1], rope=rope, pool=not dense)
+        out = (plan.run_dense(s, s) if dense else plan.run_pooled()).view(b, s, heads * 128)
         if enc_img is not None:
             out = out + image_cross_attention(attn, q, enc_img)
         return out
@@ -332,6 +343,12 @@ class WanProcessorBase(ProcessorBase):
             encoder_hidden_states = hidden_states
         if self.mode == "sparse" and self.sparse_now() and self.fuse_prep and encoder_hidden_states is hidden_states:
             fused = self._fused(attn, hidden_states, rotary_emb, enc_img)
+            if fused is not None:
+                self._tick()
+                return attn.to_out[1](attn.to_out[0](fused))
+        if (self.mode == "flash" or (self.mode == "sparse" and not self.sparse_now())) and self.fuse_prep_dense \
+                and encoder_hidden_states is hidden_states and attention_mask is None:
+            fused = self._fused(attn, hidden_states, rotary_emb, enc_img, dense=True)
             if fused is not None:
                 self._tick()
                 return attn.to_out[1](attn.to_out[0](fused))

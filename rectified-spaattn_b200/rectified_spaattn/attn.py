@@ -1,7 +1,7 @@
 """Mirror of the reference rectified_spaattn/attn.py (dense attention helper).
 
 `fullattn(..., mode="flash")` -- the only mode on the sparse path (text rows, warm-up layers/steps; reference
-attn.py:107-120 calls flash_attn_varlen_func) -- runs on kernel 4 with every KV block kept (dense tiles), so the
+attn.py:107-120 calls flash_attn_varlen_func) -- runs on kernel 4's list-free dense form (rsa_dense_attention), so the
 package has no flash-attn dependency.  Modes "torch" and "vanilla" are the reference's A/B-comparison switches
 (scripts --mode), not part of the hot path; they are kept as plain PyTorch for completeness.
 """
@@ -42,12 +42,11 @@ def _flash_like(q, k, v, cu_seqlens_q, cu_seqlens_kv, batch_size):
     if cu_seqlens_kv is not None:
         ck = cu_seqlens_kv.tolist() if isinstance(cu_seqlens_kv, torch.Tensor) else list(cu_seqlens_kv)
         kv_len = min(skv, int(ck[1]))
-    nqb, nkb = (sq + 127) // 128, (skv + 127) // 128
-    mask = torch.ones(b, h, nqb, nkb, dtype=torch.bool, device=q.device)
-    out = _ops.masked_attention(q, k, v, mask, kv_len, fp32_scale=True)   # flash-attn's arithmetic: no q~ rounding
-    if q_valid < sq:
-        out[:, :, q_valid:] = 0
-    return out
+    if q_valid < 1:
+        return torch.zeros_like(q, memory_format=torch.contiguous_format)
+    # kernel 4 walking every block without lists: bit-identical to the masked form on an all-ones mask with
+    # fp32_scale=True (flash-attn's arithmetic), with no mask, no workspace and rows >= q_valid written as zeros
+    return _ops.dense_attention(q, k, v, q_valid, kv_len)
 
 
 def fullattn(q, k, v, mode="flash", drop_rate=0, attn_mask=None, causal=False, cu_seqlens_q=None,

@@ -57,12 +57,14 @@ class RectifiedCogVideoXVideoSpaAttnProcessor2_0(_P.ProcessorBase):
         if attention_mask is not None:
             attention_mask = attn.prepare_attention_mask(attention_mask, s, b)
             attention_mask = attention_mask.view(b, attn.heads, -1, attention_mask.shape[-1])
-        if (self.mode == "sparse" and self.current_step >= 5 and self.fuse_prep and attention_mask is None
+        sparse = self.mode == "sparse" and self.current_step >= 5     # otherwise fullattn(mode="flash") below
+        if ((self.fuse_prep if sparse else self.fuse_prep_dense) and attention_mask is None
                 and not getattr(attn, "is_cross_attention", False)):
             # kernel 0: head split + LayerNorm + RoPE + pooling in one pass (reference :443-469), then kernels 3a-4
             fused = _P.fused_prep_attention(attn, hidden_states, None, _G.cogvideo(s, n_txt), self.select_block_num,
                                             self.p_remain_rates, self.block_neighbor_list, image_rotary_emb,
-                                            rope_text=False, mask_cache=self._mask_cache())
+                                            rope_text=False, mask_cache=self._mask_cache() if sparse else None,
+                                            dense=not sparse)
             if fused is not None:
                 self._tick()
                 hidden_states = attn.to_out[1](attn.to_out[0](fused))

@@ -55,14 +55,16 @@ class RectifiedFluxSpaAttnProcessor2_0(_P.ProcessorBase):
 
     def __call__(self, attn, hidden_states, encoder_hidden_states=None, attention_mask=None, image_rotary_emb=None):
         sparse = self.mode == "sparse" and (self.processor_id < 37 or self.processor_id >= 57)
-        if sparse and self.fuse_prep and attention_mask is None:
+        # every call that is not sparse goes to fullattn(mode="flash") below: single-stream blocks 37-56, other modes
+        if (self.fuse_prep if sparse else self.fuse_prep_dense) and attention_mask is None:
             # kernel 0: everything between the projections and the attention in one pass (reference :431-486)
             s = hidden_states.shape[1] + (encoder_hidden_states.shape[1] if encoder_hidden_states is not None else 0)
             fused = None
             if s % 128 == 0 and s > self.text_length:
                 fused = _P.fused_prep_attention(attn, hidden_states, encoder_hidden_states, _G.flux(s, self.text_length),
                                                 self.select_block_num, self.p_remain_rates, self.block_neighbor_list,
-                                                image_rotary_emb, rope_text=True, mask_cache=self._mask_cache())
+                                                image_rotary_emb, rope_text=True,
+                                                mask_cache=self._mask_cache() if sparse else None, dense=not sparse)
             if fused is not None:
                 self._tick()
                 if encoder_hidden_states is None:

@@ -72,14 +72,17 @@ class RectifiedHunyuanVideoSpaAttnProcessor2_0(_P.ProcessorBase):
         single_stream = getattr(attn, "add_q_proj", None) is None and encoder_hidden_states is not None
         if single_stream:
             hidden_states = torch.cat([hidden_states, encoder_hidden_states], dim=1)
-        if self.mode == "sparse" and self.fuse_prep and encoder_hidden_states is not None:
+        sparse = self.mode == "sparse"
+        if ((sparse and self.fuse_prep) or (self.mode == "flash" and self.fuse_prep_dense)) \
+                and encoder_hidden_states is not None:
             # kernel 0: everything between the projections and the attention in one pass (reference :448-498)
             s = hidden_states.shape[1] + (0 if single_stream else encoder_hidden_states.shape[1])
             num_true = self.num_true if self.num_true is not None else _P.kv_valid(attention_mask, s)
             fused = _P.fused_prep_attention(attn, hidden_states, None if single_stream else encoder_hidden_states,
                                             _G.hunyuan(s, int(num_true), encoder_hidden_states.shape[1]),
                                             self.select_block_num, self.p_remain_rates, self.block_neighbor_list,
-                                            image_rotary_emb, rope_text=False, mask_cache=self._mask_cache())
+                                            image_rotary_emb, rope_text=False,
+                                            mask_cache=self._mask_cache() if sparse else None, dense=not sparse)
             if fused is not None:
                 n_txt = encoder_hidden_states.shape[1]
                 hidden_states, encoder_hidden_states = fused[:, :-n_txt], fused[:, -n_txt:]

@@ -67,12 +67,13 @@ EXPORTS = [
     "rsa_rectified_attention_pooled_scatter", "rsa_rectified_attention_reuse",
     "rsa_debug_attention_grid_slot", "rsa_debug_front_text_heads", "rsa_gilbert_xyz2d_r",
     "rsa_attn_desc_size", "rsa_prep_desc_size", "rsa_peer_route_size", "rsa_row_rms",
+    "rsa_dense_attention", "rsa_dense_attention_scatter",
 ]
 
 _lib = None
 
 
-ABI_VERSION = 107
+ABI_VERSION = 108
 
 
 def lib():
@@ -122,6 +123,8 @@ def lib():
     L.rsa_qkv_prep_gather.argtypes = [C.POINTER(PrepDesc), C.POINTER(AttnDesc), C.POINTER(PeerRoute), p, p, p, i32, p,
                                       sz, p]
     L.rsa_rectified_attention_pooled_scatter.argtypes = [C.POINTER(AttnDesc), p, p, p, C.POINTER(PeerRoute), p, sz, p]
+    L.rsa_dense_attention.argtypes = [C.POINTER(AttnDesc), p, p, p, p, i32, i32, i32, p]
+    L.rsa_dense_attention_scatter.argtypes = [C.POINTER(AttnDesc), p, p, p, C.POINTER(PeerRoute), i32, i32, p]
     L.rsa_row_rms.argtypes = [p, p, i32, i32, i32, C.POINTER(i64), C.POINTER(i64), C.c_float, p, p, p]
     L.rsa_peer_alloc.argtypes = [sz, C.POINTER(p)]
     L.rsa_peer_free.argtypes = [p]

@@ -246,6 +246,15 @@ class Plan:
             self.mask_cache.ran(mask_mode)
         return self.out
 
+    def run_dense(self, q_valid, kv_len):
+        """Dense attention over this plan's q, k, v into its [B, S, H, D] output (rsa_dense_attention): query rows
+        >= q_valid are zeros, keys >= kv_len are not attended.  No block selection, no workspace."""
+        with torch.cuda.device(self.device):
+            N.check(N.lib().rsa_dense_attention(C.byref(self.desc), self.q.data_ptr(), self.k.data_ptr(),
+                                                self.v.data_ptr(), self.out.data_ptr(), self.shape[2], int(q_valid),
+                                                int(kv_len), _stream(self.device)), "rsa_dense_attention")
+        return self.out
+
     def _reuse(self, mask_mode, pooled):
         L = N.lib()
         with torch.cuda.device(self.device):
@@ -544,6 +553,52 @@ def masked_attention(q, k, v, block_mask, kv_len, sm_scale=None, out=None, fp32_
                                        (N.DTYPE_F16 if q.dtype == torch.float16 else N.DTYPE_BF16)
                                        | (N.ATTN_FP32_SCALE if fp32_scale else 0), d),
                 "rsa_masked_attention")
+    return out
+
+
+def dense_attention(q, k, v, q_valid, kv_len, out=None):
+    """Dense attention on kernel 4 without lists (rsa_dense_attention): q [B,H,S,D], k / v [B,H,S_kv,D] views with any
+    strides (D contiguous), bf16 or fp16, D = 128 or 64.  Query rows >= q_valid are zeros, keys >= kv_len are not
+    attended; flash-attn's arithmetic.  `out`: a [B,H,S,D] tensor or view, or a [B,S,H,D] tensor written through its
+    permuted view (the processors' layout); returned as given (a new contiguous [B,H,S,D] tensor when None)."""
+    _need_cuda(q, "q")
+    if q.dtype not in (torch.bfloat16, torch.float16) or k.dtype != q.dtype or v.dtype != q.dtype:
+        raise RuntimeError("q, k, v must all be bfloat16 or all float16")
+    b, h, s, d = q.shape
+    if d not in (64, 128):
+        raise AssertionError("head_dim must be 128 or 64")
+    skv = k.shape[2]
+    if k.shape != (b, h, skv, d) or v.shape != k.shape:
+        raise RuntimeError("key/value must be [B, H, S_kv, D] with the query's B, H and D")
+
+    def ready(t):       # the kernel reads through TMA: strides multiples of 8 elements, 16-byte aligned base
+        if t.stride(3) != 1 or any(x % 8 for x in t.stride()[:3]) or t.data_ptr() % 16:
+            t = t.contiguous()
+        return t
+
+    q, k, v = ready(q), ready(k), ready(v)
+    if out is None:
+        out = torch.empty((b, h, s, d), dtype=q.dtype, device=q.device)
+    if out.dtype != q.dtype or out.device != q.device:
+        raise RuntimeError("out must have the dtype and device of q")
+    if tuple(out.shape) == (b, h, s, d):
+        o4 = out
+    elif tuple(out.shape) == (b, s, h, d):
+        o4 = out.permute(0, 2, 1, 3)
+    else:
+        raise RuntimeError("out must be [B, H, S, D] or [B, S, H, D]")
+    if o4.stride(3) != 1:
+        raise RuntimeError("out must have a contiguous head_dim")
+    desc = N.AttnDesc()
+    desc.batch, desc.heads, desc.seq, desc.head_dim = b, h, s, d
+    for name, t in zip(("q_stride", "k_stride", "v_stride", "o_stride"), (q, k, v, o4)):
+        arr = getattr(desc, name)
+        for i in range(3):
+            arr[i] = t.stride(i)
+    desc.dtype = N.DTYPE_F16 if q.dtype == torch.float16 else N.DTYPE_BF16
+    with torch.cuda.device(q.device):
+        N.check(N.lib().rsa_dense_attention(C.byref(desc), q.data_ptr(), k.data_ptr(), v.data_ptr(), o4.data_ptr(), skv,
+                                            int(q_valid), int(kv_len), _stream(q.device)), "rsa_dense_attention")
     return out
 
 

@@ -100,6 +100,8 @@ class FusedUlysses:
       4. barrier (every rank's scatter has landed),
     and returns this rank's rows of the result, [B, rows, H*D] -- what `ulysses_attention` computes with two
     all-to-alls (233 + 78 MB per GPU at C3a, P = 8) and two staging copies around the call.
+    run(dense=True) is the form for calls that attend densely (warm-up steps, dense layers): kernel 0 gathers without
+    pooling and kernel 4's list-free dense form scatters, between the same two barriers.
     D = head_dim: 128, or 64 (CogVideoX; run() then needs the LayerNorm parameters q_weight, k_weight, q_bias, k_bias)."""
 
     def __init__(self, batch, heads_total, geo, top_k, p_remain, nbr=None, group=None, head_dim=128):
@@ -174,19 +176,23 @@ class FusedUlysses:
     def _barrier(self):
         dist.all_reduce(self._flag, group=self.group)       # stream-ordered, one element: nothing but a barrier
 
-    def run(self, q_weight=None, k_weight=None, eps=1e-6, rope=None, rope_rows=None, q_bias=None, k_bias=None):
+    def run(self, q_weight=None, k_weight=None, eps=1e-6, rope=None, rope_rows=None, q_bias=None, k_bias=None,
+            dense=False):
         """q_weight / k_weight: RMSNorm weights ([128] per head, or [heads_total*128] across heads); with q_bias /
-        k_bias: LayerNorm over head_dim (CogVideoX), the only norm at head_dim 64."""
+        k_bias: LayerNorm over head_dim (CogVideoX), the only norm at head_dim 64.  dense=True: dense attention over the
+        geometry's valid tokens (memory rows: num_true for HunyuanVideo, S otherwise) instead of the sparse call."""
         from . import native as N
         from . import ops
         import ctypes as C
+        if not isinstance(dense, bool):
+            raise TypeError("dense must be True or False")
         plan = self.plan
         hd = self.head_dim
+        if hd == 64 and (q_weight is None or q_bias is None):
+            raise RuntimeError("head_dim 64 is built for CogVideoX's LayerNorm: q_weight, k_weight, q_bias, k_bias")
         p = N.PrepDesc()
         p.rows, p.dst_row = self.seq, 0
         keep = []
-        if hd == 64 and (q_weight is None or q_bias is None):
-            raise RuntimeError("head_dim 64 is built for CogVideoX's LayerNorm: q_weight, k_weight, q_bias, k_bias")
         if q_weight is not None:
             ws_ = [w.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for w in (q_weight, k_weight)]
             keep += ws_
@@ -223,21 +229,28 @@ class FusedUlysses:
         self._barrier()
         st = ops._stream(self.device)
         gap = plan.desc.vis_len and plan.desc.nq_blocks * 128 - plan.desc.vis_len
+        pool = 0 if dense else 1
         with torch.cuda.device(self.device):
             if gap:     # ragged visual segment: the block structure restarts at the text tokens -> two gathers
                 nv = plan.desc.vis_len
                 p.rows, p.dst_row = nv, 0
                 p.rope_rows = min(p.rope_rows, nv)
                 N.check(self._lib.rsa_qkv_prep_gather(C.byref(p), C.byref(plan.desc), C.byref(self.route),
-                                                      plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), 1,
+                                                      plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), pool,
                                                       plan.ws.data_ptr(), plan.ws_bytes, st), "rsa_qkv_prep_gather")
                 p.rows, p.dst_row, p.rope_rows = self.seq - nv, nv, 0
             N.check(self._lib.rsa_qkv_prep_gather(C.byref(p), C.byref(plan.desc), C.byref(self.route), plan.q.data_ptr(),
-                                                  plan.k.data_ptr(), plan.v.data_ptr(), 1, plan.ws.data_ptr(),
+                                                  plan.k.data_ptr(), plan.v.data_ptr(), pool, plan.ws.data_ptr(),
                                                   plan.ws_bytes, st), "rsa_qkv_prep_gather")
-            N.check(self._lib.rsa_rectified_attention_pooled_scatter(
-                C.byref(plan.desc), plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), C.byref(self.route),
-                plan.ws.data_ptr(), plan.ws_bytes, st), "rsa_rectified_attention_pooled_scatter")
+            if dense:
+                n_valid = plan.desc.kv_len - gap    # the geometry's kv_len counts the gap rows of a ragged segment
+                N.check(self._lib.rsa_dense_attention_scatter(
+                    C.byref(plan.desc), plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), C.byref(self.route),
+                    n_valid, n_valid, st), "rsa_dense_attention_scatter")
+            else:
+                N.check(self._lib.rsa_rectified_attention_pooled_scatter(
+                    C.byref(plan.desc), plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), C.byref(self.route),
+                    plan.ws.data_ptr(), plan.ws_bytes, st), "rsa_rectified_attention_pooled_scatter")
         self._barrier()
         self._keep = keep
         return self.out

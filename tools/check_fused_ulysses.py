@@ -1,5 +1,6 @@
 """Multi-GPU check + measurement of the fused Ulysses exchange (run under torchrun on 2, 4 or 8 GPUs of one box;
-workload name as the argument: a bench.py workload, or "odd" / "cog" below):
+workload name as the argument: a bench.py workload, or "odd" / "cog" below; --dense: the dense form, FusedUlysses.run(
+dense=True) against kernel 0 without pooling + Plan.run_dense):
   * rank r holds tokens [r*S/P, (r+1)*S/P) of the projection outputs; FusedUlysses.run() must return exactly the rows a
     single-GPU call over all heads produces (heads are independent, same kernels => bit-identical),
   * the NCCL form (two all-to-alls around kernel 0 + the pooled call, rsa_b200.parallel.ulysses_attention-style) gives
@@ -18,8 +19,9 @@ sys.argv, argv = [sys.argv[0]], sys.argv[1:]
 import bench  # noqa: E402
 from rsa_b200 import ops, parallel  # noqa: E402
 
-name = argv[0] if argv else "c3a"
+name = next((a for a in argv if not a.startswith("--")), "c3a")
 check = "--no-check" not in argv
+dense = "--dense" in argv
 rank, world, lrank = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(lrank)
 dev = torch.device("cuda", lrank)
@@ -63,12 +65,18 @@ mine = slice(rank * rows, min((rank + 1) * rows, s))
 fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr, head_dim=hd)
 for dst, src in zip((fu.q_src, fu.k_src, fu.v_src), full):
     dst.copy_(src[:, mine])
-out = fu.run(wq, wk, 1e-6, rope, nv, **norm_kw).clone()
+out = fu.run(wq, wk, 1e-6, rope, nv, dense=dense, **norm_kw).clone()
 torch.cuda.synchronize()
 
 # NCCL form: all-to-all the projection rows to head shards, kernel 0 + pooled call locally, all-to-all the result back
 q, k, v = (torch.empty(1, max(hl, 1), s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
 plan = ops.Plan(q, k, v, geo, wp["top_k"], bench.P_REMAIN, nbr)
+
+
+def finish(pl):
+    """The attention after kernel 0: the pooled sparse call, or dense attention over the valid memory rows."""
+    n_valid = geo.kv_len - geo.gap
+    return pl.run_dense(n_valid, n_valid) if dense else pl.run_pooled()
 
 
 def wan_norm(x, w):
@@ -88,13 +96,15 @@ def nccl_form():
         dist.all_to_all_single(rcv, loc)
         srcs.append(rcv.permute(1, 0, 2, 3).reshape(1, s, hl * hd))                          # all tokens, my heads
     if wan:
-        plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv)
+        plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv, pool=not dense)
     elif geo.gap:
-        plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope)
-        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6)
+        plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
+                      pool=not dense)
+        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense)
     else:
-        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, **norm_kw)
-    o = plan.run_pooled()                                                                     # [1, S, hl, hd]
+        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
+                      **norm_kw)
+    o = finish(plan)                                                                     # [1, S, hl, hd]
     return parallel.head_to_seq_shard(o).reshape(1, rows, heads * hd)
 
 
@@ -111,11 +121,13 @@ if check and (rank == 0 or not even):       # uneven shards: every rank checks i
     qa, ka, va = (torch.empty(1, heads, s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
     pa = ops.Plan(qa, ka, va, geo, wp["top_k"], bench.P_REMAIN, nbr)
     if geo.gap:
-        pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope)
-        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6)
+        pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
+                    pool=not dense)
+        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense)
     else:
-        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, **norm_kw)
-    single = pa.run_pooled().reshape(1, s, heads * hd)[:, mine]
+        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
+                    **norm_kw)
+    single = finish(pa).reshape(1, s, heads * hd)[:, mine]
     torch.cuda.synchronize()
     same_as_single = bool(torch.equal(out.view(torch.int16), single.view(torch.int16)))
     del qa, ka, va, pa
@@ -138,14 +150,14 @@ def timed(fn, n=10):
     return float(tt.item())
 
 
-ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, nv, **norm_kw))
+ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, nv, dense=dense, **norm_kw))
 ms_nccl = timed(nccl_form) if even else None
 oks = [None] * world
 dist.all_gather_object(oks, same_as_nccl)
 singles = [None] * world
 dist.all_gather_object(singles, same_as_single)
 if rank == 0:
-    print(json.dumps({"workload": name, "n_gpus": world, "tokens": s, "heads": heads, "head_dim": hd,
+    print(json.dumps({"workload": name, "dense": dense, "n_gpus": world, "tokens": s, "heads": heads, "head_dim": hd,
                       "fused_ms_per_layer_attention": ms_fused, "nccl_all_to_all_form_ms": ms_nccl,
                       "norm": "across heads (Wan)" if wan else ("LayerNorm per head (CogVideoX)" if cog else "per head"),
                       "fused_equals_nccl_form_bitwise_all_ranks": all(oks),
@@ -153,7 +165,7 @@ if rank == 0:
                       "fused_equals_single_gpu_bitwise_rank0": same_as_single,
                       "fused_equals_single_gpu_bitwise_checked_ranks": [x for x in singles if x is not None],
                       "rows_per_rank": rows, "rows_last_rank": s - (world - 1) * rows, "heads_rank0": fu.heads,
-                      "note": "both forms run kernel 0 + kernels 3a-4; fused = gather inside kernel 0 and scatter inside "
+                      "note": "both forms run kernel 0 + kernels 3a-4 (--dense: kernel 0 without pooling + dense kernel 4); fused = gather inside kernel 0 and scatter inside "
                               "kernel 4's epilogue over peer memory, barriers only; nccl = all_to_all_single x4 + staging copies"}))
 fu.close()
 dist.destroy_process_group()
