@@ -76,12 +76,12 @@ constexpr int kDefaultPolyPairs64 = 1;  // CogVideoX1.5 shape, kernel 4: 8.30 / 
 __device__ __forceinline__ float u2f(uint32_t u) { return __uint_as_float(u); }
 __device__ __forceinline__ uint32_t f2u(float f) { return __float_as_uint(f); }
 
-// 2^x for x <= ~8 on the FMA pipe, two lanes at a time: x = n + f, n = round(x), f in [-0.5, 0.5];
-// 2^f ~ c0 + f (c1 + f (c2 + f c3)); the integer n is added into the exponent field.
+// 2^x for x <= 127 on the FMA pipe, two lanes at a time: x = n + f, n = round(x), f in [-0.5, 0.5];
+// 2^f ~ c0 + f (c1 + f (c2 + f c3)); the integer n is added into the exponent field, which is valid for n >= -125.
+// Below that, -inf (a key >= kv_len) included, the result is +0 as with ex2.approx.ftz, which differs only in returning
+// values under 2^-125 for x in [-126, -125): a key that must not be attended gets weight exactly zero.
 __device__ __forceinline__ float2 exp2_poly2(float2 x) {
   const float kMagic = 12582912.f;  // 1.5 * 2^23: adding it leaves round(x) in the low mantissa bits
-  x.x = fmaxf(x.x, -125.f);
-  x.y = fmaxf(x.y, -125.f);
   const float2 t = __fadd2_rn(x, make_float2(kMagic, kMagic));
   const float2 r = __fadd2_rn(t, make_float2(-kMagic, -kMagic));
   const float2 f = __ffma2_rn(r, make_float2(-1.f, -1.f), x);
@@ -89,8 +89,8 @@ __device__ __forceinline__ float2 exp2_poly2(float2 x) {
                         make_float2(0.24261151254177094f, 0.24261151254177094f));
   p = __ffma2_rn(p, f, make_float2(0.6932601928710938f, 0.6932601928710938f));
   p = __ffma2_rn(p, f, make_float2(0.9999279975891113f, 0.9999279975891113f));
-  p.x = __int_as_float(__float_as_int(p.x) + (__float_as_int(t.x) << 23));
-  p.y = __int_as_float(__float_as_int(p.y) + (__float_as_int(t.y) << 23));
+  p.x = x.x < -125.f ? 0.f : __int_as_float(__float_as_int(p.x) + (__float_as_int(t.x) << 23));
+  p.y = x.y < -125.f ? 0.f : __int_as_float(__float_as_int(p.y) + (__float_as_int(t.y) << 23));
   return p;
 }
 
