@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define RSA_VERSION 108 /* 108: rsa_dense_attention, rsa_dense_attention_scatter (kernel 4 without lists) */
+#define RSA_VERSION 109 /* 109: kernel 0 (rsa_qkv_prep, rsa_qkv_prep_gather) in fp16; rsa_row_rms_dtype */
 #define RSA_BLOCK 128
 #define RSA_HEAD_DIM 128
 #define RSA_MAX_ENTRIES 2048 /* max sortable entries per query block: NQ (+1 for the text aggregate) */
@@ -122,7 +122,7 @@ typedef struct rsa_attn_desc {
                                        /* strides always describe the tensors as they lie in memory.        */
   int32_t dtype;                       /* enum rsa_dtype of query / key / value / out (kernels 2 and 4; pooled   */
                                        /* statistics, scores and selection are fp32 either way).  Kernel 0       */
-                                       /* (rsa_qkv_prep*) follows diffusers' bf16 rounding points: bf16 only.    */
+                                       /* (rsa_qkv_prep*) follows diffusers' rounding points in this dtype.      */
 } rsa_attn_desc;
 
 /* Pointers into the caller's workspace (all device memory, fp32 unless noted). */
@@ -226,7 +226,11 @@ int rsa_rectified_attention_reuse(const rsa_attn_desc* d, const void* q, const v
  * descriptor's workspace and every visual / text block must be produced by such calls before
  * rsa_rectified_attention_pooled runs.
  * head_dim 128 takes every norm; head_dim 64 (CogVideoX1.5: 48 heads x 64) takes norm 3 only (RSA_ERR_UNSUPPORTED
- * otherwise), with the pooled statistics' columns 64..127 written as zeros, as rsa_pool_stats computes them. */
+ * otherwise), with the pooled statistics' columns 64..127 written as zeros, as rsa_pool_stats computes them.
+ * The 16-bit tensors -- sources, destinations, norm weights and biases -- are all in the descriptor's dtype, bf16 or fp16
+ * (an fp16 model, e.g. CogVideoX-2B, runs the same diffusers sequence in fp16).  Every rounding point rounds to that
+ * format to nearest even: in fp16 an overflow becomes +-inf, as .to(torch.float16) gives, and results below 2^-14 stay
+ * subnormal.  The same norms and head dims are built in both dtypes. */
 typedef struct rsa_prep_desc {
   int32_t rows;             /* tokens in the source tensors                                                   */
   int32_t dst_row;          /* memory row of the destination the first source token goes to: 0 or the visual  */
@@ -236,7 +240,8 @@ typedef struct rsa_prep_desc {
                             /* heads*128 channels of a token (Wan2.1 / Wan2.2, rectified_wan21_attn.py:423-426)*/
                             /* 3 = LayerNorm over head_dim with weight and bias (CogVideoX, cogvideo :452-455) */
   float eps;
-  const void* q_weight;     /* DEVICE bf16 [head_dim] (norms 1, 3) or [heads*128] (norm 2): norm_q.weight      */
+  const void* q_weight;     /* DEVICE [head_dim] (norms 1, 3) or [heads*128] (norm 2), in the descriptor's      */
+                            /* dtype: norm_q.weight                                                            */
   const void* k_weight;     /* likewise norm_k.weight                                                          */
   int32_t rope_rows;        /* source tokens [0, rope_rows) are rotated; 0 = no rotary embedding               */
   int32_t rope_compact;     /* 0: cos and sin are two tables.  1: `cos` is ONE table [rope_rows, head_dim/2] of */
@@ -247,7 +252,7 @@ typedef struct rsa_prep_desc {
   const float* cos;         /* DEVICE fp32 [rope_rows, head_dim] (diffusers' repeat-interleaved cos table)     */
   const float* sin;
   float* row_scratch;       /* norm 2 only: DEVICE scratch of 2*batch*rows floats for the per-token statistics  */
-  const void* q_bias;       /* norm 3 only: DEVICE bf16 [head_dim] (norm_q.bias)                                */
+  const void* q_bias;       /* norm 3 only: DEVICE [head_dim] in the descriptor's dtype (norm_q.bias)           */
   const void* k_bias;
 } rsa_prep_desc;
 
@@ -309,10 +314,11 @@ typedef struct rsa_peer_route {
   int32_t head0;                /* this rank's first head: it computes heads [head0, head0 + desc->heads)          */
   int32_t reserved;             /* 0                                                                               */
   const void* const* src_table; /* DEVICE array [3][n_ranks] (q, k, v): every rank's projection output,           */
-                                /* [batch, rows_per_rank, heads_total*head_dim] bf16, as mapped in THIS process     */
+                                /* [batch, rows_per_rank, heads_total*head_dim] in the descriptor's dtype, as      */
+                                /* mapped in THIS process                                                           */
   int64_t src_stride[2];        /* (batch, token) element strides of those buffers                                 */
   void* const* out_table;       /* DEVICE array [n_ranks]: every rank's result buffer [batch, rows_per_rank,       */
-                                /* heads_total, head_dim] bf16, as mapped in this process                          */
+                                /* heads_total, head_dim] in the descriptor's dtype, as mapped in this process      */
   int64_t out_stride[2];        /* (batch, token) element strides of those buffers                                 */
   const float* const* rinv_table; /* prep norm 2 (Wan: RMSNorm over all heads_total*128 channels of a token) only:  */
                                 /* DEVICE array [2][n_ranks] (q, k): every rank's per-token statistics              */
@@ -326,6 +332,9 @@ typedef struct rsa_peer_route {
  * Ulysses exchange every rank runs it on the tokens it owns so that the gathering ranks need not see whole rows. */
 int rsa_row_rms(const void* q_src, const void* k_src, int batch, int rows, int channels, const int64_t q_stride[2],
                 const int64_t k_stride[2], float eps, float* rinv_q, float* rinv_k, void* stream);
+/* The same for rows in `dtype` (enum rsa_dtype: bf16 or fp16; the statistic is fp32 either way).  rsa_row_rms reads bf16. */
+int rsa_row_rms_dtype(const void* q_src, const void* k_src, int batch, int rows, int channels, const int64_t q_stride[2],
+                      const int64_t k_stride[2], float eps, float* rinv_q, float* rinv_k, int dtype, void* stream);
 
 int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* d, const rsa_peer_route* route, void* q, void* k,
                         void* v, int pool, void* workspace, size_t workspace_bytes, void* stream);

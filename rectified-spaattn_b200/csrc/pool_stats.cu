@@ -21,6 +21,9 @@
 // in rectified_flux_attn.py): unflatten/transpose, attn.norm_q / attn.norm_k (diffusers RMSNorm(head_dim, eps):
 // x * rsqrt(mean(x^2) + eps) in fp32 -> bf16 -> * weight -> bf16) and diffusers apply_rotary_emb(use_real=True,
 // use_real_unbind_dim=-1): out = x * cos + rotate_pairs(x) * sin in fp32 (two products and a sum, each rounded) -> bf16.
+// An fp16 model runs the same sequence in fp16 (diffusers rounds at the same points in either format): kernel 0's kF16
+// forms round with cvt.rn.f16x2.f32 -- no .satfinite, so an overflow becomes +-inf as in .to(torch.float16), and results
+// below 2^-14 stay fp16 subnormals -- and pool the fp16 rows they store, exactly as kernel 2's fp16 form reads them.
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -32,13 +35,13 @@ namespace {
 
 constexpr int kThreads = 256;
 
-struct PrepArgs {
+struct PrepArgs {  // 16-bit tensors are in the descriptor's dtype (bf16, or fp16 in the kF16 forms)
   const __nv_bfloat16* src[3];  // q, k, v projection outputs [B, rows, H*D], D = head_dim (128, or 64 with layer_norm)
   int64_t src_stride[3][2];     // (batch, token) element strides
   __nv_bfloat16* dst[3];        // [B, H, S, D] views
   int64_t dst_stride[3][3];     // (batch, head, token)
-  const __nv_bfloat16* w[2];    // norm weights of q, k (bf16 [D], or [H*128] with w_head_stride = 128) or nullptr
-  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k (bf16 [D]) -- layer_norm only
+  const __nv_bfloat16* w[2];    // norm weights of q, k ([D], or [H*128] with w_head_stride = 128) or nullptr
+  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k ([D]) -- layer_norm only
   int layer_norm;               // 1: LayerNorm over head_dim (CogVideoX: mean removed, bias added, one rounding)
   int w_head_stride;            // 0: one weight vector per tensor (norm over head_dim); 128: norm across heads (Wan)
   const float* row_rinv[2];     // norm across heads: rsqrt(mean(x^2) + eps) per (batch, source row), from row_rms_kernel
@@ -90,6 +93,28 @@ __device__ __forceinline__ uint4 ld_global_v4(const void* p) {
   return r;
 }
 
+// Kernel 0's rounding points: two fp32 values rounded to the 16-bit format as one packed pair.  fp16 takes
+// cvt.rn.f16x2.f32 without .satfinite (overflow -> +-inf, as .to(torch.float16)); neither form flushes subnormals.
+template <bool kF16>
+struct Pair16 {
+  using T = __nv_bfloat162;
+  static __device__ __forceinline__ T pack(float a, float b) { return __floats2bfloat162_rn(a, b); }
+};
+template <>
+struct Pair16<true> {
+  using T = __half2;
+  static __device__ __forceinline__ T pack(float a, float b) {
+    uint32_t u;
+    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(u) : "f"(b), "f"(a));  // a -> low half, b -> high half
+    return *reinterpret_cast<const __half2*>(&u);
+  }
+};
+template <bool kF16>
+__device__ __forceinline__ float2 round2(float a, float b) {
+  if constexpr (kF16) return __half22float2(Pair16<true>::pack(a, b));
+  else return __bfloat1622float2(__floats2bfloat162_rn(a, b));
+}
+
 // Kernel 0 front end: rows of one 128-token block of one head, normalised / rotated / rounded to bf16, stored to the
 // destination and returned in the same register layout the pooling sweep uses.  All eight source rows of a thread are
 // requested before the first is used, and the rotary-table row of step it + 1 is requested before step it is
@@ -120,8 +145,8 @@ __device__ __forceinline__ RopeRow load_rope(const PrepArgs& p, int r, int col, 
 // kGather: rows come from peer-mapped buffers.  kCompact: one (cos, sin)-pair table.  Compile-time so that each form
 // carries only its own code and registers (with all of them behind run-time flags the HunyuanVideo form lost 40 %).
 // kD: head_dim.  At 64 (CogVideoX, LayerNorm only) a thread's 8 columns belong to one of two adjacent heads h, h + 1
-// (see qkv_prep_stream_kernel); `heads` tells whether head h + 1 exists.
-template <int kNorm, bool kCompact, bool kGather, int kD = 128>
+// (see qkv_prep_stream_kernel); `heads` tells whether head h + 1 exists.  kF16: the rows, weights and biases are fp16.
+template <int kNorm, bool kCompact, bool kGather, int kD = 128, bool kF16 = false>
 __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
                                              uint4 (&raw)[8], int heads = 0);
 
@@ -159,7 +184,7 @@ __device__ __forceinline__ void prep_rows(const PrepArgs& p, int which, int b, i
 // raw[it] = source row jblk * 128 + 16 warp + 2 it + (lane >> 4), columns 8 (lane & 15) .. +7 of head h (kD = 64:
 // columns 8 (lane & 7) .. +7 of head h + ((lane >> 3) & 1)), zeros beyond the source: normalise / rotate / round, store
 // to the destination, and leave the rounded values in raw (zeros for the lanes of a head that does not exist).
-template <int kNorm, bool kCompact, bool kGather, int kD>
+template <int kNorm, bool kCompact, bool kGather, int kD, bool kF16>
 __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
                                              uint4 (&raw)[8], int heads) {
   static_assert(kD == 128 || (kD == 64 && kNorm == 3), "the 64-column form is built for LayerNorm (CogVideoX) only");
@@ -179,10 +204,10 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
   float wgt[8];
   // (src_head0: under the fused Ulysses gather this rank's head h is head src_head0 + h of the token's row; else 0)
   if constexpr (kNorm != 0)
-    unpack8(__ldg(reinterpret_cast<const uint4*>(p.w[which] + (p.src_head0 + h) * p.w_head_stride + col)), wgt);
+    unpack8<kF16>(__ldg(reinterpret_cast<const uint4*>(p.w[which] + (p.src_head0 + h) * p.w_head_stride + col)), wgt);
   const float* rinv_rows = (kNorm == 2 && !kGather) ? p.row_rinv[which] + (int64_t)b * p.rows : nullptr;
   float bia[8];
-  if constexpr (kNorm == 3) unpack8(__ldg(reinterpret_cast<const uint4*>(p.bias[which] + col)), bia);
+  if constexpr (kNorm == 3) unpack8<kF16>(__ldg(reinterpret_cast<const uint4*>(p.bias[which] + col)), bia);
   RopeRow next = load_rope<kCompact, kD>(p, r0, col, r0 < p.rows && r0 < p.rope_rows);
 #pragma unroll
   for (int it = 0; it < 8; ++it) {
@@ -192,9 +217,9 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
     const RopeRow t = next;
     if (it < 7) next = load_rope<kCompact, kD>(p, r + 2, col, r + 2 < p.rows && r + 2 < p.rope_rows);
     float f[8];
-    unpack8(raw[it], f);
+    unpack8<kF16>(raw[it], f);
     if constexpr (kNorm == 3) {
-      // torch.nn.LayerNorm(head_dim) on a bf16 tensor: statistics and affine in fp32, ONE rounding to bf16
+      // torch.nn.LayerNorm(head_dim) on a bf16 / fp16 tensor: statistics and affine in fp32, ONE rounding
       // (cogvideo :452-455; two-pass variance, fixed butterfly order over the kD / 8 lanes that share the (row, head))
       float sm = 0.f;
 #pragma unroll
@@ -213,8 +238,8 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
       const float rstd = rsqrtf(__fadd_rn(__fmul_rn(ss, 1.0f / kD), p.eps));
 #pragma unroll
       for (int c = 0; c < 8; c += 2) {
-        const float2 y = __bfloat1622float2(__floats2bfloat162_rn(__fmaf_rn(wgt[c], __fmul_rn(rstd, f[c]), bia[c]),
-                                                                  __fmaf_rn(wgt[c + 1], __fmul_rn(rstd, f[c + 1]), bia[c + 1])));
+        const float2 y = round2<kF16>(__fmaf_rn(wgt[c], __fmul_rn(rstd, f[c]), bia[c]),
+                                      __fmaf_rn(wgt[c + 1], __fmul_rn(rstd, f[c + 1]), bia[c + 1]));
         f[c] = y.x;
         f[c + 1] = y.y;
       }
@@ -238,8 +263,8 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
       }
 #pragma unroll
       for (int c = 0; c < 8; c += 2) {  // packed conversions: one F2FP per pair, the scalar cvt runs on the XU pipe
-        const float2 xn = __bfloat1622float2(__floats2bfloat162_rn(__fmul_rn(f[c], rinv), __fmul_rn(f[c + 1], rinv)));
-        const float2 y = __bfloat1622float2(__floats2bfloat162_rn(__fmul_rn(xn.x, wgt[c]), __fmul_rn(xn.y, wgt[c + 1])));
+        const float2 xn = round2<kF16>(__fmul_rn(f[c], rinv), __fmul_rn(f[c + 1], rinv));
+        const float2 y = round2<kF16>(__fmul_rn(xn.x, wgt[c]), __fmul_rn(xn.y, wgt[c + 1]));
         f[c] = y.x;
         f[c + 1] = y.y;
       }
@@ -256,9 +281,9 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
 #pragma unroll
       for (int c = 0; c < 8; ++c) f[c] = g[c];
     }
-    __nv_bfloat162 o2[4];
+    typename Pair16<kF16>::T o2[4];
 #pragma unroll
-    for (int c = 0; c < 4; ++c) o2[c] = __floats2bfloat162_rn(f[2 * c], f[2 * c + 1]);
+    for (int c = 0; c < 4; ++c) o2[c] = Pair16<kF16>::pack(f[2 * c], f[2 * c + 1]);
     const uint4 u = *reinterpret_cast<const uint4*>(o2);
     if (live && head_live) *reinterpret_cast<uint4*>(dst + (int64_t)(p.dst_row0 + r) * p.dst_stride[which][2]) = u;
     raw[it] = live && head_live ? u : make_uint4(0, 0, 0, 0);
@@ -267,7 +292,9 @@ __device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b
 
 // RMSNorm across heads (Wan: attn.norm_q / norm_k = RMSNorm(heads*head_dim), rectified_wan21_attn.py:423-426): one warp
 // per source row computes rsqrt(mean(x^2) + eps) over all H*128 channels.  Order (replicated by the oracle): lane l
-// runs one fma chain over its columns 8(l + 32 j) .. +7, j = 0, 1, ..; then a butterfly over the lanes.
+// runs one fma chain over its columns 8(l + 32 j) .. +7, j = 0, 1, ..; then a butterfly over the lanes.  kF16: fp16 rows
+// (the statistic is fp32 either way).
+template <bool kF16>
 __global__ void __launch_bounds__(256) row_rms_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
                                                       int64_t qsb, int64_t qst, int64_t ksb, int64_t kst, int rows,
                                                       int inner, float eps, float* __restrict__ rq, float* __restrict__ rk) {
@@ -278,7 +305,7 @@ __global__ void __launch_bounds__(256) row_rms_kernel(const __nv_bfloat16* __res
   float ss = 0.f;
   for (int c0 = 8 * lane; c0 < inner; c0 += 256) {
     float f[8];
-    unpack8(__ldg(reinterpret_cast<const uint4*>(x + c0)), f);
+    unpack8<kF16>(__ldg(reinterpret_cast<const uint4*>(x + c0)), f);
 #pragma unroll
     for (int c = 0; c < 8; ++c) ss = __fmaf_rn(f[c], f[c], ss);
   }
@@ -666,7 +693,8 @@ __global__ void __launch_bounds__(kThreads, 2) pool_stats_stream_kernel(const Po
 // each half-warp take head h, lanes 8-15 head h + 1; an odd head count leaves the last pair half empty (128-byte
 // copies, nothing stored for the missing head).  Every lane stays busy: the kernel is bound by issue slots, and one
 // head per item would idle half of them.  n_bh counts pairs then (B * ceil(H / 2)).
-template <int kNorm, bool kGather, bool kCompact, int kD = 128>
+// kF16: fp16 rows (every form above has one); the rounding points, the copies and the pooling order are the same.
+template <int kNorm, bool kGather, bool kCompact, int kD = 128, bool kF16 = false>
 __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const PoolArgs a, const PrepArgs p, const int n_blocks,
                                                                       const int n_bh) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -758,7 +786,7 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
       raw[i] = make_uint4(0, 0, 0, 0);
       if (rloc + 2 * i < rows && lane_live) raw[i] = tp[i * 32];
     }
-    process_rows<kNorm, kCompact, kGather, kD>(p, which, b, h, jblk, warp, lane, raw, a.heads);
+    process_rows<kNorm, kCompact, kGather, kD, kF16>(p, which, b, h, jblk, warp, lane, raw, a.heads);
     const bool visual = blk < a.nq_vis;
     bool pooled = false;
     if (p.pool) {
@@ -775,7 +803,7 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
           const int t = (blk - a.nq_vis) * 128 + rloc + 2 * i;  // text token index
           if (t < a.text_keys && lane_live) {
             float f[8];
-            unpack8<false>(raw[i], f);
+            unpack8<kF16>(raw[i], f);
             // kD = 64: head bh0 + (col >> 6), its columns (col & 63) .. +7, and zeros in the 64 columns it lacks
             const int row_bh = kD == 128 ? bh : bh0 + (col >> 6), row_col = kD == 128 ? col : col & 63;
             float* dstk = a.mean[1] + ((int64_t)row_bh * a.out_rows[1] + a.n_blk[1] + t) * 128 + row_col;
@@ -793,7 +821,7 @@ __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const Pool
     if (pooled) {
       float2 f[8][4];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) unpack_row<false>(raw[i], f[i]);
+      for (int i = 0; i < 8; ++i) unpack_row<kF16>(raw[i], f[i]);
       pool_block<kD>(a, f, which, bh0, blk, s_part, s_mean, tid, warp, lane, [&]() {
         if (n + kPoolStages < n_mine) issue(n + kPoolStages);
       }, live_cols);
@@ -886,10 +914,11 @@ int launch_pool_stats(const rsa_attn_desc* d, const void* q, const void* k, cons
 }
 
 int launch_row_rms(const void* q_src, const void* k_src, int batch, int rows, int channels, const int64_t* qs,
-                   const int64_t* ks, float eps, float* rq, float* rk, cudaStream_t s) {
+                   const int64_t* ks, float eps, float* rq, float* rk, bool f16, cudaStream_t s) {
   dim3 g((rows + 7) / 8, batch, 2);
-  row_rms_kernel<<<g, 256, 0, s>>>((const __nv_bfloat16*)q_src, (const __nv_bfloat16*)k_src, qs[0], qs[1], ks[0], ks[1], rows,
-                                   channels, eps, rq, rk);
+  auto kernel = f16 ? row_rms_kernel<true> : row_rms_kernel<false>;
+  kernel<<<g, 256, 0, s>>>((const __nv_bfloat16*)q_src, (const __nv_bfloat16*)k_src, qs[0], qs[1], ks[0], ks[1], rows,
+                           channels, eps, rq, rk);
   RSA_CUDA_CHECK(cudaGetLastError());
   return RSA_OK;
 }
@@ -917,14 +946,13 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
   pa.bias[0] = (const __nv_bfloat16*)p->q_bias;
   pa.bias[1] = (const __nv_bfloat16*)p->k_bias;
   pa.row_rinv[0] = pa.row_rinv[1] = nullptr;
+  const bool f16 = d->dtype == RSA_DTYPE_F16;
   if (p->norm == 2 && !route) {
     float* rq = p->row_scratch;
     float* rk = rq + (int64_t)d->batch * p->rows;
-    dim3 g((p->rows + 7) / 8, d->batch, 2);
-    row_rms_kernel<<<g, 256, 0, s>>>((const __nv_bfloat16*)q_src, (const __nv_bfloat16*)k_src, p->src_stride[0][0],
-                                     p->src_stride[0][1], p->src_stride[1][0], p->src_stride[1][1], p->rows,
-                                     d->heads * 128, p->eps, rq, rk);
-    RSA_CUDA_CHECK(cudaGetLastError());
+    const int rc = launch_row_rms(q_src, k_src, d->batch, p->rows, d->heads * 128, p->src_stride[0], p->src_stride[1],
+                                  p->eps, rq, rk, f16, s);
+    if (rc != RSA_OK) return rc;
     pa.row_rinv[0] = rq;
     pa.row_rinv[1] = rk;
   }
@@ -981,17 +1009,23 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
   const int sgrid = (int)(items < 2 * sms ? items : 2 * sms);
   dim3 grid(3 * d->batch * d->heads, blocks);
   // per-block form: 2 CTAs per SM (about 100 registers): capping at 3 or 4 CTAs spills and is no faster (1.24 / 1.25 / 2.17 ms at C3b)
-#define RSA_PREP_STREAM(NORM, GATHER, COMPACT, D)                                                                       \
+#define RSA_PREP_STREAM_F(NORM, GATHER, COMPACT, D, F16)                                                                \
   do {                                                                                                                  \
     static bool cfg = false;                                                                                            \
     if (!cfg) {                                                                                                         \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D>,                              \
+      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16>,                         \
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));                     \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D>,                              \
+      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16>,                         \
                                           cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
       cfg = true;                                                                                                       \
     }                                                                                                                   \
-    qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D><<<sgrid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);            \
+    qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16><<<sgrid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);       \
+  } while (0)
+#define RSA_PREP_STREAM(NORM, GATHER, COMPACT, D) RSA_PREP_STREAM_F(NORM, GATHER, COMPACT, D, false)
+#define RSA_PREP_F16(NORM, GATHER, D)                                    \
+  do {                                                                   \
+    if (compact) RSA_PREP_STREAM_F(NORM, GATHER, true, D, true);         \
+    else RSA_PREP_STREAM_F(NORM, GATHER, false, D, true);                \
   } while (0)
 #define RSA_PREP_LAUNCH(NORM, GATHER)                                                               \
   do {                                                                                              \
@@ -1001,29 +1035,50 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
     } else if (compact) pool_stats_kernel<true, 2, NORM, GATHER, true><<<grid, kThreads, 0, s>>>(a, pa);   \
     else pool_stats_kernel<true, 2, NORM, GATHER, false><<<grid, kThreads, 0, s>>>(a, pa);          \
   } while (0)
-  if (hd64) {
-    // 64-column heads: CogVideoX's LayerNorm only (rsa_api.cu refuses the other norms), always the streaming kernel
-    if (route) {
-      if (compact) RSA_PREP_STREAM(3, true, true, 64);
-      else RSA_PREP_STREAM(3, true, false, 64);
-    } else if (compact) {
-      RSA_PREP_STREAM(3, false, true, 64);
+  if (!f16) {
+    if (hd64) {
+      // 64-column heads: CogVideoX's LayerNorm only (rsa_api.cu refuses the other norms), always the streaming kernel
+      if (route) {
+        if (compact) RSA_PREP_STREAM(3, true, true, 64);
+        else RSA_PREP_STREAM(3, true, false, 64);
+      } else if (compact) {
+        RSA_PREP_STREAM(3, false, true, 64);
+      } else {
+        RSA_PREP_STREAM(3, false, false, 64);
+      }
+    } else if (route) {
+      if (p->norm == 1) RSA_PREP_LAUNCH(1, true);
+      else if (p->norm == 2) RSA_PREP_LAUNCH(2, true);
+      else RSA_PREP_LAUNCH(0, true);
     } else {
-      RSA_PREP_STREAM(3, false, false, 64);
+      switch (p->norm) {
+        case 1: RSA_PREP_LAUNCH(1, false); break;
+        case 2: RSA_PREP_LAUNCH(2, false); break;
+        case 3: RSA_PREP_LAUNCH(3, false); break;
+        default: RSA_PREP_LAUNCH(0, false); break;
+      }
     }
-  } else if (route) {
-    if (p->norm == 1) RSA_PREP_LAUNCH(1, true);
-    else if (p->norm == 2) RSA_PREP_LAUNCH(2, true);
-    else RSA_PREP_LAUNCH(0, true);
   } else {
-    switch (p->norm) {
-      case 1: RSA_PREP_LAUNCH(1, false); break;
-      case 2: RSA_PREP_LAUNCH(2, false); break;
-      case 3: RSA_PREP_LAUNCH(3, false); break;
-      default: RSA_PREP_LAUNCH(0, false); break;
+    // fp16: the streaming kernel only (RSA_PREP_FORM=0 selects the per-block form for bf16), the same norms as bf16
+    if (hd64) {
+      if (route) RSA_PREP_F16(3, true, 64);
+      else RSA_PREP_F16(3, false, 64);
+    } else if (route) {
+      if (p->norm == 1) RSA_PREP_F16(1, true, 128);
+      else if (p->norm == 2) RSA_PREP_F16(2, true, 128);
+      else RSA_PREP_F16(0, true, 128);
+    } else {
+      switch (p->norm) {
+        case 1: RSA_PREP_F16(1, false, 128); break;
+        case 2: RSA_PREP_F16(2, false, 128); break;
+        case 3: RSA_PREP_F16(3, false, 128); break;
+        default: RSA_PREP_F16(0, false, 128); break;
+      }
     }
   }
+#undef RSA_PREP_STREAM_F
 #undef RSA_PREP_STREAM
+#undef RSA_PREP_F16
 #undef RSA_PREP_LAUNCH
   RSA_CUDA_CHECK(cudaGetLastError());
   return RSA_OK;

@@ -486,7 +486,9 @@ extern "C" int rsa_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, cons
   int rc = validate_desc(d);
   if (rc != RSA_OK) return rc;
   if (!p) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep: descriptor is null");
-  if (d->dtype != RSA_DTYPE_BF16) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep follows diffusers' bf16 rounding points: bf16 only");
+  // diffusers' rounding points in the descriptor's dtype: bf16 or fp16 (validate_desc has refused any other)
+  if (d->dtype != RSA_DTYPE_BF16 && d->dtype != RSA_DTYPE_F16)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: dtype %d is not bf16 or fp16", d->dtype);
   if (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: head_dim must be 128 or 64 (got %d)", d->head_dim);
   if (d->head_dim == 64 && p->norm != 3)
     RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: head_dim 64 is built for norm 3 (LayerNorm, CogVideoX) only, not norm %d", p->norm);
@@ -544,8 +546,10 @@ extern "C" int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* 
   if (rc != RSA_OK) return rc;
   if ((rc = validate_route(d, route, true, false)) != RSA_OK) return rc;
   if (!p || !q || !k || !v) RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: null pointer");
-  if (d->dtype != RSA_DTYPE_BF16 || (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64))
-    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: bf16 and head_dim 128 or 64 only");
+  if (d->dtype != RSA_DTYPE_BF16 && d->dtype != RSA_DTYPE_F16)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: dtype %d is not bf16 or fp16", d->dtype);
+  if (d->head_dim != RSA_HEAD_DIM && d->head_dim != 64)
+    RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: head_dim must be 128 or 64 (got %d)", d->head_dim);
   // like rsa_qkv_prep: the whole sequence in one call, or -- ragged visual segment -- the visual tokens (dst_row 0) and
   // the text tokens (dst_row = visual token count) in two; source token = dst_row + row either way
   const RowMap rm = row_map(d);
@@ -575,14 +579,23 @@ extern "C" int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* 
                          (cudaStream_t)stream);
 }
 
-extern "C" int rsa_row_rms(const void* q_src, const void* k_src, int batch, int rows, int channels,
-                           const int64_t q_stride[2], const int64_t k_stride[2], float eps, float* rinv_q, float* rinv_k,
-                           void* stream) {
+extern "C" int rsa_row_rms_dtype(const void* q_src, const void* k_src, int batch, int rows, int channels,
+                                 const int64_t q_stride[2], const int64_t k_stride[2], float eps, float* rinv_q,
+                                 float* rinv_k, int dtype, void* stream) {
   if (!q_src || !k_src || !rinv_q || !rinv_k || !q_stride || !k_stride) RSA_FAIL(RSA_ERR_ARG, "rsa_row_rms: null pointer");
+  if (dtype != RSA_DTYPE_BF16 && dtype != RSA_DTYPE_F16) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_row_rms: dtype %d is not bf16 or fp16", dtype);
   if (batch < 1 || rows < 1 || channels < 8 || channels % 8) RSA_FAIL(RSA_ERR_ARG, "rsa_row_rms: bad sizes");
   if (((uintptr_t)q_src | (uintptr_t)k_src) % 16 || q_stride[1] % 8 || k_stride[1] % 8 || q_stride[0] % 8 || k_stride[0] % 8)
     RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_row_rms: rows must be 16-byte aligned");
-  return launch_row_rms(q_src, k_src, batch, rows, channels, q_stride, k_stride, eps, rinv_q, rinv_k, (cudaStream_t)stream);
+  return launch_row_rms(q_src, k_src, batch, rows, channels, q_stride, k_stride, eps, rinv_q, rinv_k,
+                        dtype == RSA_DTYPE_F16, (cudaStream_t)stream);
+}
+
+extern "C" int rsa_row_rms(const void* q_src, const void* k_src, int batch, int rows, int channels,
+                           const int64_t q_stride[2], const int64_t k_stride[2], float eps, float* rinv_q, float* rinv_k,
+                           void* stream) {
+  return rsa_row_rms_dtype(q_src, k_src, batch, rows, channels, q_stride, k_stride, eps, rinv_q, rinv_k, RSA_DTYPE_BF16,
+                           stream);
 }
 
 extern "C" int rsa_rectified_attention_pooled_scatter(const rsa_attn_desc* d, const void* q, const void* k,

@@ -123,7 +123,7 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
                     const void* v_src, const rsa_peer_route* route, void* q, void* k, void* v, char* ws,
                     const WsLayout* L, cudaStream_t s);
 int launch_row_rms(const void* q_src, const void* k_src, int batch, int rows, int channels, const int64_t* qs,
-                   const int64_t* ks, float eps, float* rq, float* rk, cudaStream_t s);
+                   const int64_t* ks, float eps, float* rq, float* rk, bool f16, cudaStream_t s);
 int launch_block_scores(const rsa_attn_desc* d, char* ws, const WsLayout& L, cudaStream_t s);
 int launch_block_select(const rsa_attn_desc* d, char* ws, const WsLayout& L, cudaStream_t s, bool keep_lists = false);
 int launch_rect_c(const rsa_attn_desc* d, char* ws, const WsLayout& L, cudaStream_t s);

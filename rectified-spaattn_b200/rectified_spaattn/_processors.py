@@ -83,23 +83,24 @@ def dense(fullattn, query, key, value, mode, attention_mask, s_k):
     return out.transpose(1, 2).reshape(b, s_q, -1)
 
 
-def rms_params(mod):
-    """(weight, eps) if `mod` is an RMSNorm over head_dim = 128 with a bf16 weight and no bias -- the form kernel 0
-    fuses (diffusers RMSNorm of HunyuanVideo / Flux `norm_q`, `norm_k`, `norm_added_q`, `norm_added_k`); else None."""
+def rms_params(mod, dtype=torch.bfloat16):
+    """(weight, eps) if `mod` is an RMSNorm over head_dim = 128 with a weight of `dtype` (the activations' dtype: a
+    weight of another dtype rounds elsewhere in diffusers) and no bias -- the form kernel 0 fuses (diffusers RMSNorm of
+    HunyuanVideo / Flux `norm_q`, `norm_k`, `norm_added_q`, `norm_added_k`); else None."""
     w, eps = getattr(mod, "weight", None), getattr(mod, "eps", None)
     if mod is None or w is None or eps is None or getattr(mod, "bias", None) is not None:
         return None
-    if "RMSNorm" not in type(mod).__name__ or w.dtype != torch.bfloat16 or w.numel() != 128 or not w.is_cuda:
+    if "RMSNorm" not in type(mod).__name__ or w.dtype != dtype or w.numel() != 128 or not w.is_cuda:
         return None
     return w, float(eps)
 
 
-def wan_rms_params(mod, heads):
-    """(weight, eps) if `mod` is an RMSNorm over all heads*128 channels with a bf16 weight (Wan norm_q / norm_k)."""
+def wan_rms_params(mod, heads, dtype=torch.bfloat16):
+    """(weight, eps) if `mod` is an RMSNorm over all heads*128 channels with a weight of `dtype` (Wan norm_q / norm_k)."""
     w, eps = getattr(mod, "weight", None), getattr(mod, "eps", None)
     if mod is None or w is None or eps is None or getattr(mod, "bias", None) is not None:
         return None
-    if "RMSNorm" not in type(mod).__name__ or w.dtype != torch.bfloat16 or w.numel() != heads * 128 or not w.is_cuda:
+    if "RMSNorm" not in type(mod).__name__ or w.dtype != dtype or w.numel() != heads * 128 or not w.is_cuda:
         return None
     return w, float(eps)
 
@@ -133,17 +134,17 @@ def wan_rope_tables(emb, n):
     return _wan_rope_cache[key][1]
 
 
-def head_norm_params(mod, head_dim=128):
+def head_norm_params(mod, head_dim=128, dtype=torch.bfloat16):
     """dict(q_weight-style kwargs) for a per-head norm kernel 0 fuses: RMSNorm(128) (HunyuanVideo / Flux) or
-    LayerNorm(head_dim) with bias (CogVideoX: head_dim 128 or 64), bf16 parameters; else None.  Returns (weight, bias or
-    None, eps)."""
-    r = rms_params(mod) if head_dim == 128 else None     # kernel 0 has no RMSNorm at 64 columns
+    LayerNorm(head_dim) with bias (CogVideoX: head_dim 128 or 64), parameters of `dtype`; else None.  Returns (weight,
+    bias or None, eps)."""
+    r = rms_params(mod, dtype) if head_dim == 128 else None     # kernel 0 has no RMSNorm at 64 columns
     if r is not None:
         return r[0], None, r[1]
     w, b, eps = getattr(mod, "weight", None), getattr(mod, "bias", None), getattr(mod, "eps", None)
     if mod is None or w is None or b is None or eps is None or "LayerNorm" not in type(mod).__name__:
         return None
-    if (w.dtype != torch.bfloat16 or b.dtype != torch.bfloat16 or w.numel() != head_dim or b.numel() != head_dim
+    if (w.dtype != dtype or b.dtype != dtype or w.numel() != head_dim or b.numel() != head_dim
             or not w.is_cuda):
         return None
     return w, b, float(eps)
@@ -160,8 +161,13 @@ def rope_tables(emb, n, head_dim=128):
     return (cos, sin) if ok else None
 
 
+def prep_dtype_ok(x, fp16):
+    """Kernel 0 runs on bf16 activations, and on fp16 ones when the processor's fuse_prep_fp16 switch is set."""
+    return x.dtype == torch.bfloat16 or (fp16 and x.dtype == torch.float16)
+
+
 def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k, p_remain, nbr, image_rotary_emb,
-                         rope_text, mask_cache=None, dense=False):
+                         rope_text, mask_cache=None, dense=False, fp16=False):
     """The fused form of a joint-text processor's middle section (kernel 0 + kernels 3a-4): projections ->
     rsa_qkv_prep (head split, RMSNorm / LayerNorm, RoPE, re-layout, pooling) -> rsa_rectified_attention_pooled.  Returns
     [B, S, H*D], or None when this layer does not have the shape kernel 0 fuses (the caller then runs the op-by-op path).
@@ -169,18 +175,20 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
     `rope_text`: Flux rotates the text tokens too (their table rows follow the image rows); HunyuanVideo does not.
     `dense`: the call the op-by-op path sends to fullattn(mode="flash") -- kernel 0 without pooling, then dense
     attention over the first `geo.kv_len - geo.gap` memory rows (num_true for HunyuanVideo, S otherwise) as queries
-    and keys; top_k, p_remain, nbr and mask_cache are not used."""
+    and keys; top_k, p_remain, nbr and mask_cache are not used.
+    `fp16`: fp16 activations take kernel 0 too (ProcessorBase.fuse_prep_fp16); the norm parameters must then be fp16."""
     from rsa_b200 import ops
     heads = attn.heads
-    if not hidden_states.is_cuda or hidden_states.dtype != torch.bfloat16:
+    if not hidden_states.is_cuda or not prep_dtype_ok(hidden_states, fp16):
         return None
+    dt = hidden_states.dtype
     inner = getattr(attn.to_q, "out_features", None)
     hd = inner // heads if isinstance(inner, int) and inner % heads == 0 else 0
     if hd not in (128, 64):
         return None
     dual = getattr(attn, "add_q_proj", None) is not None and encoder_hidden_states is not None
     def pair(nq, nk):
-        a, c = head_norm_params(getattr(attn, nq, None), hd), head_norm_params(getattr(attn, nk, None), hd)
+        a, c = head_norm_params(getattr(attn, nq, None), hd, dt), head_norm_params(getattr(attn, nk, None), hd, dt)
         if a is None or c is None or a[2] != c[2] or (a[1] is None) != (c[1] is None):
             return None
         return dict(q_weight=a[0], k_weight=c[0], q_bias=a[1], k_bias=c[1], eps=a[2])
@@ -211,10 +219,11 @@ def fused_prep_attention(attn, hidden_states, encoder_hidden_states, geo, top_k,
     elif lat[0].shape[1] != s:
         return None
     # every "this layer does not fit" exit is above: from here on the call is made
-    q, k, v = (torch.empty(b, heads, s, hd, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
+    q, k, v = (torch.empty(b, heads, s, hd, dtype=dt, device=hidden_states.device) for _ in range(3))
     plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, mask_cache=None if dense else mask_cache)
     cut = lambda r, a, z: None if r is None else (r[0][a:z], r[1][a:z])
     pool = not dense
+    lat_norm, enc_norm = (None if n is None else dict(n, allow_fp16=fp16) for n in (lat_norm, enc_norm))
     if dual:
         plan.qkv_prep(*lat, dst_row=0, rope=cut(rope, 0, nv), pool=pool, **lat_norm)
         plan.qkv_prep(*enc, dst_row=nv, rope=cut(rope, nv, s) if rope_text else None, pool=pool, **enc_norm)
@@ -241,6 +250,10 @@ class ProcessorBase:
     # the same for the calls that go to fullattn(mode="flash") (warm-up calls, dense layers, mode "flash"): kernel 0
     # without pooling, then kernel 4's list-free dense form.  Off by default: the op-by-op route stays the reference's.
     fuse_prep_dense = False
+    # kernel 0 for fp16 layers too (fp16 models such as CogVideoX-2B): with fuse_prep on their sparse calls, with
+    # fuse_prep_dense on their dense calls as well.  The norm parameters must be fp16 like the activations.  Off by
+    # default: until it is switched on, an fp16 model runs its pre-attention op by op exactly as before.
+    fuse_prep_fp16 = False
 
     def __init__(self, mode, select_block_num, block_neighbor_list, p_remain_rates, processor_id=0):
         self.mode = mode
@@ -302,17 +315,19 @@ class WanProcessorBase(ProcessorBase):
     def sparse_now(self) -> bool:
         raise NotImplementedError
 
-    def _fused(self, attn, hidden_states, rotary_emb, enc_img, dense=False):
+    def _fused(self, attn, hidden_states, rotary_emb, enc_img, dense=False, fp16=False):
         """Kernel 0 form of the middle section (reference rectified_wan21_attn.py:419-470): projections -> RMSNorm across
         heads + rotary embedding + head split + pooling in one pass -> kernels 3a-4.  None when the layer does not have
         the shape kernel 0 fuses.  `dense`: a warm-up call or dense layer -- kernel 0 without pooling, then dense
-        attention over all S tokens."""
+        attention over all S tokens.  `fp16`: fp16 activations (and fp16 norm weights) take kernel 0 too."""
         from rsa_b200 import geometry as G
         from rsa_b200 import ops
         heads = attn.heads
-        if not hidden_states.is_cuda or hidden_states.dtype != torch.bfloat16:
+        if not hidden_states.is_cuda or not prep_dtype_ok(hidden_states, fp16):
             return None
-        nq_, nk_ = wan_rms_params(getattr(attn, "norm_q", None), heads), wan_rms_params(getattr(attn, "norm_k", None), heads)
+        dt = hidden_states.dtype
+        nq_ = wan_rms_params(getattr(attn, "norm_q", None), heads, dt)
+        nk_ = wan_rms_params(getattr(attn, "norm_k", None), heads, dt)
         if nq_ is None or nk_ is None or nq_[1] != nk_[1]:
             return None
         b, s, _ = hidden_states.shape
@@ -324,10 +339,11 @@ class WanProcessorBase(ProcessorBase):
         src = [f(hidden_states) for f in (attn.to_q, attn.to_k, attn.to_v)]
         if src[0].shape[2] != heads * 128:
             return None
-        q, k, v = (torch.empty(b, heads, s, 128, dtype=torch.bfloat16, device=hidden_states.device) for _ in range(3))
+        q, k, v = (torch.empty(b, heads, s, 128, dtype=dt, device=hidden_states.device) for _ in range(3))
         plan = ops.Plan(q, k, v, G.wan(s, self.first_frame_blocks), self.select_block_num, self.p_remain_rates,
                         self.block_neighbor_list, mask_cache=None if dense else self._mask_cache())
-        plan.qkv_prep(*src, dst_row=0, q_weight=nq_[0], k_weight=nk_[0], eps=nq_[1], rope=rope, pool=not dense)
+        plan.qkv_prep(*src, dst_row=0, q_weight=nq_[0], k_weight=nk_[0], eps=nq_[1], rope=rope, pool=not dense,
+                      allow_fp16=fp16)
         out = (plan.run_dense(s, s) if dense else plan.run_pooled()).view(b, s, heads * 128)
         if enc_img is not None:
             out = out + image_cross_attention(attn, q, enc_img)
@@ -342,13 +358,13 @@ class WanProcessorBase(ProcessorBase):
         if encoder_hidden_states is None:
             encoder_hidden_states = hidden_states
         if self.mode == "sparse" and self.sparse_now() and self.fuse_prep and encoder_hidden_states is hidden_states:
-            fused = self._fused(attn, hidden_states, rotary_emb, enc_img)
+            fused = self._fused(attn, hidden_states, rotary_emb, enc_img, fp16=self.fuse_prep_fp16)
             if fused is not None:
                 self._tick()
                 return attn.to_out[1](attn.to_out[0](fused))
         if (self.mode == "flash" or (self.mode == "sparse" and not self.sparse_now())) and self.fuse_prep_dense \
                 and encoder_hidden_states is hidden_states and attention_mask is None:
-            fused = self._fused(attn, hidden_states, rotary_emb, enc_img, dense=True)
+            fused = self._fused(attn, hidden_states, rotary_emb, enc_img, dense=True, fp16=self.fuse_prep_fp16)
             if fused is not None:
                 self._tick()
                 return attn.to_out[1](attn.to_out[0](fused))

@@ -64,7 +64,7 @@ class RectifiedCogVideoXVideoSpaAttnProcessor2_0(_P.ProcessorBase):
             fused = _P.fused_prep_attention(attn, hidden_states, None, _G.cogvideo(s, n_txt), self.select_block_num,
                                             self.p_remain_rates, self.block_neighbor_list, image_rotary_emb,
                                             rope_text=False, mask_cache=self._mask_cache() if sparse else None,
-                                            dense=not sparse)
+                                            dense=not sparse, fp16=self.fuse_prep_fp16)
             if fused is not None:
                 self._tick()
                 hidden_states = attn.to_out[1](attn.to_out[0](fused))

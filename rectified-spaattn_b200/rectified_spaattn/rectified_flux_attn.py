@@ -64,7 +64,7 @@ class RectifiedFluxSpaAttnProcessor2_0(_P.ProcessorBase):
                 fused = _P.fused_prep_attention(attn, hidden_states, encoder_hidden_states, _G.flux(s, self.text_length),
                                                 self.select_block_num, self.p_remain_rates, self.block_neighbor_list,
                                                 image_rotary_emb, rope_text=True,
-                                                mask_cache=self._mask_cache() if sparse else None, dense=not sparse)
+                                                mask_cache=self._mask_cache() if sparse else None, dense=not sparse, fp16=self.fuse_prep_fp16)
             if fused is not None:
                 self._tick()
                 if encoder_hidden_states is None:

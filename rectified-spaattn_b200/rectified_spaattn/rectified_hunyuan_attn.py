@@ -82,7 +82,7 @@ class RectifiedHunyuanVideoSpaAttnProcessor2_0(_P.ProcessorBase):
                                             _G.hunyuan(s, int(num_true), encoder_hidden_states.shape[1]),
                                             self.select_block_num, self.p_remain_rates, self.block_neighbor_list,
                                             image_rotary_emb, rope_text=False,
-                                            mask_cache=self._mask_cache() if sparse else None, dense=not sparse)
+                                            mask_cache=self._mask_cache() if sparse else None, dense=not sparse, fp16=self.fuse_prep_fp16)
             if fused is not None:
                 n_txt = encoder_hidden_states.shape[1]
                 hidden_states, encoder_hidden_states = fused[:, :-n_txt], fused[:, -n_txt:]

@@ -67,13 +67,13 @@ EXPORTS = [
     "rsa_rectified_attention_pooled_scatter", "rsa_rectified_attention_reuse",
     "rsa_debug_attention_grid_slot", "rsa_debug_front_text_heads", "rsa_gilbert_xyz2d_r",
     "rsa_attn_desc_size", "rsa_prep_desc_size", "rsa_peer_route_size", "rsa_row_rms",
-    "rsa_dense_attention", "rsa_dense_attention_scatter",
+    "rsa_dense_attention", "rsa_dense_attention_scatter", "rsa_row_rms_dtype",
 ]
 
 _lib = None
 
 
-ABI_VERSION = 108
+ABI_VERSION = 109
 
 
 def lib():
@@ -126,6 +126,7 @@ def lib():
     L.rsa_dense_attention.argtypes = [C.POINTER(AttnDesc), p, p, p, p, i32, i32, i32, p]
     L.rsa_dense_attention_scatter.argtypes = [C.POINTER(AttnDesc), p, p, p, C.POINTER(PeerRoute), i32, i32, p]
     L.rsa_row_rms.argtypes = [p, p, i32, i32, i32, C.POINTER(i64), C.POINTER(i64), C.c_float, p, p, p]
+    L.rsa_row_rms_dtype.argtypes = [p, p, i32, i32, i32, C.POINTER(i64), C.POINTER(i64), C.c_float, p, p, i32, p]
     L.rsa_peer_alloc.argtypes = [sz, C.POINTER(p)]
     L.rsa_peer_free.argtypes = [p]
     L.rsa_peer_export.argtypes = [p, p]

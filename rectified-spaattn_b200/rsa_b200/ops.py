@@ -264,22 +264,30 @@ class Plan:
                     "rsa_rectified_attention_reuse")
 
     def qkv_prep(self, q_src, k_src, v_src, dst_row=0, q_weight=None, k_weight=None, eps=1e-6, rope=None,
-                 rope_rows=None, pool=True, q_bias=None, k_bias=None):
+                 rope_rows=None, pool=True, q_bias=None, k_bias=None, allow_fp16=False):
         """Kernel 0: fills rows [dst_row, dst_row + rows) of this plan's q, k, v from projection outputs
-        [B, rows, H*head_dim] (head split, per-head RMSNorm or LayerNorm with bf16 parameters, rotary embedding on the
-        first `rope_rows` tokens, re-layout) and, with pool=True, the pooled statistics of those blocks.  head_dim 128
-        takes every norm; head_dim 64 (CogVideoX) takes LayerNorm only (q_weight, k_weight, q_bias, k_bias)."""
+        [B, rows, H*head_dim] (head split, per-head RMSNorm or LayerNorm, rotary embedding on the first `rope_rows`
+        tokens, re-layout) and, with pool=True, the pooled statistics of those blocks.  head_dim 128 takes every norm;
+        head_dim 64 (CogVideoX) takes LayerNorm only (q_weight, k_weight, q_bias, k_bias).
+        The sources have the plan's dtype and the norm parameters are converted to it: kernel 0 rounds where diffusers
+        rounds, in bf16 or fp16.  An fp16 plan takes kernel 0 only with allow_fp16=True (the switch
+        ProcessorBase.fuse_prep_fp16 sets), so that an fp16 caller keeps the op-by-op sequence unless it opts in."""
         b, h, s, d = self.shape
-        if self.q.dtype != torch.bfloat16 or d not in (128, 64):
-            raise RuntimeError("kernel 0 follows diffusers' bf16 rounding points and is built for bfloat16 with "
+        dt = self.q.dtype
+        if dt == torch.float16 and not allow_fp16:
+            raise RuntimeError("kernel 0 in float16 is opt-in: pass allow_fp16=True")
+        if dt not in (torch.bfloat16, torch.float16) or d not in (128, 64):
+            raise RuntimeError("kernel 0 follows diffusers' rounding points and is built for bfloat16 or float16 with "
                                "head_dim 128 or 64")
         if d == 64 and (q_weight is None or q_bias is None):
             raise RuntimeError("kernel 0 at head_dim 64 is built for CogVideoX's LayerNorm: q_weight, k_weight, "
                                "q_bias and k_bias are needed")
         for t, n in ((q_src, "q_src"), (k_src, "k_src"), (v_src, "v_src")):
             _need_cuda(t, n)
-            if t.dtype != torch.bfloat16 or t.dim() != 3 or t.shape[0] != b or t.shape[2] != h * d or t.stride(2) != 1:
-                raise RuntimeError(f"{n} must be a bfloat16 [B, rows, H*{d}] tensor with contiguous channels")
+            if t.dtype != dt:
+                raise RuntimeError(f"{n} is {t.dtype} but the plan is {dt}: kernel 0 reads its sources in the plan's dtype")
+            if t.dim() != 3 or t.shape[0] != b or t.shape[2] != h * d or t.stride(2) != 1:
+                raise RuntimeError(f"{n} must be a [B, rows, H*{d}] tensor with contiguous channels")
         rows = q_src.shape[1]
         if k_src.shape[1] != rows or v_src.shape[1] != rows:
             raise RuntimeError("q/k/v sources differ in length")
@@ -291,9 +299,9 @@ class Plan:
         if q_weight is not None or k_weight is not None:
             if q_weight is None or k_weight is None:
                 raise RuntimeError("both norm weights are needed")
-            ws_ = [w.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for w in (q_weight, k_weight)]
+            ws_ = [w.detach().to(device=self.device, dtype=dt).contiguous() for w in (q_weight, k_weight)]
             if q_bias is not None or k_bias is not None:    # LayerNorm over head_dim (CogVideoX)
-                bs_ = [x.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for x in (q_bias, k_bias)]
+                bs_ = [x.detach().to(device=self.device, dtype=dt).contiguous() for x in (q_bias, k_bias)]
                 if any(w.numel() != d for w in ws_ + bs_):
                     raise RuntimeError("LayerNorm weights and biases must have head_dim elements")
                 keep += bs_

@@ -81,8 +81,8 @@ class _RawDevice:
         self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 3}
 
 
-def _peer_tensor(ptr, shape):
-    return torch.as_tensor(_RawDevice(ptr, shape), device="cuda").view(torch.bfloat16)
+def _peer_tensor(ptr, shape, dtype=torch.bfloat16):
+    return torch.as_tensor(_RawDevice(ptr, shape), device="cuda").view(dtype)
 
 
 class FusedUlysses:
@@ -102,12 +102,17 @@ class FusedUlysses:
     all-to-alls (233 + 78 MB per GPU at C3a, P = 8) and two staging copies around the call.
     run(dense=True) is the form for calls that attend densely (warm-up steps, dense layers): kernel 0 gathers without
     pooling and kernel 4's list-free dense form scatters, between the same two barriers.
-    D = head_dim: 128, or 64 (CogVideoX; run() then needs the LayerNorm parameters q_weight, k_weight, q_bias, k_bias)."""
+    D = head_dim: 128, or 64 (CogVideoX; run() then needs the LayerNorm parameters q_weight, k_weight, q_bias, k_bias).
+    dtype: torch.bfloat16 or torch.float16, the dtype of the peer buffers, of the plan's tensors and of the norm
+    parameters (converted to it in run()); kernel 0 rounds where diffusers rounds, in that format."""
 
-    def __init__(self, batch, heads_total, geo, top_k, p_remain, nbr=None, group=None, head_dim=128):
+    def __init__(self, batch, heads_total, geo, top_k, p_remain, nbr=None, group=None, head_dim=128,
+                 dtype=torch.bfloat16):
         from . import native as N
         from . import ops
         import ctypes as C
+        if dtype not in (torch.bfloat16, torch.float16):
+            raise ValueError(f"dtype must be torch.bfloat16 or torch.float16 (got {dtype})")
         self.group = group
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
         if self.world > 8:
@@ -117,6 +122,7 @@ class FusedUlysses:
         if head_dim not in (128, 64):
             raise ValueError("head_dim must be 128 or 64")
         self.head_dim = hd = head_dim
+        self.dtype = dtype
         # heads need not divide by the ranks: the first (H mod P) ranks take one head more (12 heads on 8 ranks:
         # 2,2,2,2,1,1,1,1); this rank computes heads [head0, head0 + heads)
         base, extra = divmod(heads_total, self.world)
@@ -158,9 +164,10 @@ class FusedUlysses:
         self._table = table.to(self.device)
         shape = (batch, self.rows, heads_total * hd)
         # views of this rank's own rows (the buffers themselves hold `rows` rows on every rank)
-        self.q_src, self.k_src, self.v_src, self.out = (_peer_tensor(p, shape)[:, :self.local_rows] for p in self._own[:4])
+        self.q_src, self.k_src, self.v_src, self.out = (_peer_tensor(p, shape, dtype)[:, :self.local_rows]
+                                                        for p in self._own[:4])
         self._flag = torch.zeros(1, device=self.device)
-        q, k, v = (torch.empty(batch, self.heads, self.seq, hd, dtype=torch.bfloat16, device=self.device)
+        q, k, v = (torch.empty(batch, self.heads, self.seq, hd, dtype=dtype, device=self.device)
                    for _ in range(3))
         self.plan = ops.Plan(q, k, v, geo, top_k, p_remain, nbr, private_workspace=True)
         route = N.PeerRoute()
@@ -194,11 +201,11 @@ class FusedUlysses:
         p.rows, p.dst_row = self.seq, 0
         keep = []
         if q_weight is not None:
-            ws_ = [w.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for w in (q_weight, k_weight)]
+            ws_ = [w.detach().to(device=self.device, dtype=self.dtype).contiguous() for w in (q_weight, k_weight)]
             keep += ws_
             p.norm, p.eps, p.q_weight, p.k_weight = 1, float(eps), ws_[0].data_ptr(), ws_[1].data_ptr()
             if q_bias is not None or k_bias is not None:    # LayerNorm over head_dim (CogVideoX)
-                bs_ = [x.detach().to(device=self.device, dtype=torch.bfloat16).contiguous() for x in (q_bias, k_bias)]
+                bs_ = [x.detach().to(device=self.device, dtype=self.dtype).contiguous() for x in (q_bias, k_bias)]
                 if any(x.numel() != hd for x in ws_ + bs_):
                     raise RuntimeError("LayerNorm weights and biases must have head_dim elements")
                 keep += bs_
@@ -212,13 +219,15 @@ class FusedUlysses:
                     # the statistics buffers are [batch, rows] like every peer buffer; rsa_row_rms packs its output as
                     # [batch, its row count], so a short last shard is done one batch element at a time
                     even = self.local_rows == self.rows
+                    dtc = N.DTYPE_F16 if self.dtype == torch.float16 else N.DTYPE_BF16
                     for b in range(1 if even else self.batch):
                         off = b * self.rows
-                        N.check(self._lib.rsa_row_rms(self._own[0] + off * self.heads_total * 256,
-                                                      self._own[1] + off * self.heads_total * 256,
-                                                      self.batch if even else 1, self.local_rows, self.heads_total * 128,
-                                                      st2, st2, float(eps), self._own[4] + off * 4, self._own[5] + off * 4,
-                                                      ops._stream(self.device)), "rsa_row_rms")
+                        N.check(self._lib.rsa_row_rms_dtype(self._own[0] + off * self.heads_total * 256,
+                                                            self._own[1] + off * self.heads_total * 256,
+                                                            self.batch if even else 1, self.local_rows,
+                                                            self.heads_total * 128, st2, st2, float(eps),
+                                                            self._own[4] + off * 4, self._own[5] + off * 4, dtc,
+                                                            ops._stream(self.device)), "rsa_row_rms_dtype")
             elif any(w.numel() != 128 for w in ws_):
                 raise RuntimeError("norm weights must have 128 (per head) or heads*128 (across heads) elements")
         if rope is not None:

@@ -1,6 +1,7 @@
 """Multi-GPU check + measurement of the fused Ulysses exchange (run under torchrun on 2, 4 or 8 GPUs of one box;
 workload name as the argument: a bench.py workload, or "odd" / "cog" below; --dense: the dense form, FusedUlysses.run(
-dense=True) against kernel 0 without pooling + Plan.run_dense):
+dense=True) against kernel 0 without pooling + Plan.run_dense; --dtype float16: fp16 projection rows, norm parameters and
+results, FusedUlysses(dtype=torch.float16)):
   * rank r holds tokens [r*S/P, (r+1)*S/P) of the projection outputs; FusedUlysses.run() must return exactly the rows a
     single-GPU call over all heads produces (heads are independent, same kernels => bit-identical),
   * the NCCL form (two all-to-alls around kernel 0 + the pooled call, rsa_b200.parallel.ulysses_attention-style) gives
@@ -19,9 +20,11 @@ sys.argv, argv = [sys.argv[0]], sys.argv[1:]
 import bench  # noqa: E402
 from rsa_b200 import ops, parallel  # noqa: E402
 
-name = next((a for a in argv if not a.startswith("--")), "c3a")
+name = next((a for i, a in enumerate(argv) if not a.startswith("--") and (i == 0 or argv[i - 1] != "--dtype")), "c3a")
 check = "--no-check" not in argv
 dense = "--dense" in argv
+dt = {"bfloat16": torch.bfloat16, "float16": torch.float16}[argv[argv.index("--dtype") + 1] if "--dtype" in argv else "bfloat16"]
+f16 = dict(allow_fp16=True) if dt == torch.float16 else {}     # Plan.qkv_prep takes fp16 plans on request
 rank, world, lrank = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(lrank)
 dev = torch.device("cuda", lrank)
@@ -46,30 +49,30 @@ nbr = ops.gilbert_block_neighbors(t, h, w)
 rows, hl = -(-s // world), heads // world          # rows per rank (the last rank may own fewer)
 even = rows * world == s and hl * world == heads      # the NCCL form below is written for even shards only
 g = torch.Generator(device=dev).manual_seed(1234)                       # same stream on every rank: the full tensors
-full = [torch.randn(1, s, heads * hd, generator=g, device=dev).to(torch.bfloat16) for _ in range(3)]
+full = [torch.randn(1, s, heads * hd, generator=g, device=dev).to(dt) for _ in range(3)]
 if wp["fam"] != "wan":                                                   # give the pooled scores some structure
     mu = torch.cumsum(torch.randn(1, (s + 127) // 128, heads * hd, generator=g, device=dev) * 0.35, dim=1)
     for x in full[:2]:
-        x.add_(mu.repeat_interleave(128, dim=1)[:, :s].to(torch.bfloat16))
+        x.add_(mu.repeat_interleave(128, dim=1)[:, :s].to(dt))
 wan = wp["fam"] == "wan"     # Wan: RMSNorm over all heads*128 channels of a token, rotary embedding on every token
 nw = heads * 128 if wan else hd
-wq = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(torch.bfloat16)
-wk = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(torch.bfloat16)
+wq = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(dt)
+wk = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(dt)
 # CogVideoX: LayerNorm(head_dim) with bias on q and k
-norm_kw = dict(q_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(torch.bfloat16),
-               k_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(torch.bfloat16)) if cog else {}
+norm_kw = dict(q_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(dt),
+               k_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(dt)) if cog else {}
 ang = torch.outer(torch.arange(nv, dtype=torch.float32, device=dev), 1.0 / (256.0 ** (torch.arange(0, hd, 2, device=dev) / hd)))
 rope = (ang.cos().repeat_interleave(2, 1).contiguous(), ang.sin().repeat_interleave(2, 1).contiguous())
 mine = slice(rank * rows, min((rank + 1) * rows, s))
 
-fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr, head_dim=hd)
+fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr, head_dim=hd, dtype=dt)
 for dst, src in zip((fu.q_src, fu.k_src, fu.v_src), full):
     dst.copy_(src[:, mine])
 out = fu.run(wq, wk, 1e-6, rope, nv, dense=dense, **norm_kw).clone()
 torch.cuda.synchronize()
 
 # NCCL form: all-to-all the projection rows to head shards, kernel 0 + pooled call locally, all-to-all the result back
-q, k, v = (torch.empty(1, max(hl, 1), s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
+q, k, v = (torch.empty(1, max(hl, 1), s, hd, dtype=dt, device=dev) for _ in range(3))
 plan = ops.Plan(q, k, v, geo, wp["top_k"], bench.P_REMAIN, nbr)
 
 
@@ -82,7 +85,7 @@ def finish(pl):
 def wan_norm(x, w):
     """diffusers RMSNorm over the whole row (what the Wan processor does before the head split), in PyTorch."""
     var = x.float().pow(2).mean(-1, keepdim=True)
-    return (x * torch.rsqrt(var + 1e-6)).to(torch.bfloat16) * w
+    return (x * torch.rsqrt(var + 1e-6)).to(dt) * w
 
 
 def nccl_form():
@@ -96,14 +99,14 @@ def nccl_form():
         dist.all_to_all_single(rcv, loc)
         srcs.append(rcv.permute(1, 0, 2, 3).reshape(1, s, hl * hd))                          # all tokens, my heads
     if wan:
-        plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv, pool=not dense)
+        plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv, pool=not dense, **f16)
     elif geo.gap:
         plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
-                      pool=not dense)
-        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense)
+                      pool=not dense, **f16)
+        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense, **f16)
     else:
         plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
-                      **norm_kw)
+                      **norm_kw, **f16)
     o = finish(plan)                                                                     # [1, S, hl, hd]
     return parallel.head_to_seq_shard(o).reshape(1, rows, heads * hd)
 
@@ -118,15 +121,15 @@ frac_equal_nccl = float((out.view(torch.int16) == ref.view(torch.int16)).float()
 same_as_single = None
 if check and (rank == 0 or not even):       # uneven shards: every rank checks its own rows (the shapes are small)
     # one GPU, all heads, no exchange at all
-    qa, ka, va = (torch.empty(1, heads, s, hd, dtype=torch.bfloat16, device=dev) for _ in range(3))
+    qa, ka, va = (torch.empty(1, heads, s, hd, dtype=dt, device=dev) for _ in range(3))
     pa = ops.Plan(qa, ka, va, geo, wp["top_k"], bench.P_REMAIN, nbr)
     if geo.gap:
         pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
-                    pool=not dense)
-        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense)
+                    pool=not dense, **f16)
+        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense, **f16)
     else:
         pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
-                    **norm_kw)
+                    **norm_kw, **f16)
     single = finish(pa).reshape(1, s, heads * hd)[:, mine]
     torch.cuda.synchronize()
     same_as_single = bool(torch.equal(out.view(torch.int16), single.view(torch.int16)))
@@ -157,7 +160,7 @@ dist.all_gather_object(oks, same_as_nccl)
 singles = [None] * world
 dist.all_gather_object(singles, same_as_single)
 if rank == 0:
-    print(json.dumps({"workload": name, "dense": dense, "n_gpus": world, "tokens": s, "heads": heads, "head_dim": hd,
+    print(json.dumps({"workload": name, "dense": dense, "dtype": str(dt).replace("torch.", ""), "n_gpus": world, "tokens": s, "heads": heads, "head_dim": hd,
                       "fused_ms_per_layer_attention": ms_fused, "nccl_all_to_all_form_ms": ms_nccl,
                       "norm": "across heads (Wan)" if wan else ("LayerNorm per head (CogVideoX)" if cog else "per head"),
                       "fused_equals_nccl_form_bitwise_all_ranks": all(oks),
