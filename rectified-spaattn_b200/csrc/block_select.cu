@@ -12,7 +12,6 @@
 // Outputs: kept-block bitmask, ascending u16 kept-block index list + count (what kernel 4 walks), n_needed, R,
 // W = P*(1-part) for kernel 3c, optionally P itself for the parity tests.
 #include <math.h>
-#include <stdlib.h>
 
 #include "rsa_common.cuh"
 
@@ -207,10 +206,10 @@ __device__ void sort_desc(const float* s_p, int n_net, int n_ent, uint32_t* s_va
   __syncthreads();
 }
 
-// kMinBlocks: CTAs per SM the register allocation is held to (the kernel is issue-bound with long barrier waits; without
-// a bound ptxas drifted from 48 to 64 registers = 4 CTAs per SM and the kernel lost 11 %)
-template <int kMinBlocks>
-__global__ void __launch_bounds__(kThreads, kMinBlocks) block_select_kernel(const SelectArgs a) {
+// Held to 8 CTAs per SM: the kernel is issue-bound with long barrier waits; without a bound ptxas drifted from 48 to 64
+// registers = 4 CTAs per SM and the kernel lost 11 %.  At 5 / 6 / 8 CTAs per SM: C3b 0.69 / 0.63 / 0.62 ms, Flux
+// 0.23 / 0.22 / 0.21, C4 0.51 / 0.47 / 0.45 (profiles/r01_block_select_occupancy_ab.txt).
+__global__ void __launch_bounds__(kThreads, 8) block_select_kernel(const SelectArgs a) {
   __shared__ float s_p[kMaxEnt + 1];
   __shared__ uint32_t s_val[kMaxEnt + 1];  // sorted probability bit patterns
   __shared__ uint32_t s_thr;           // bit pattern of the n-th largest probability
@@ -445,14 +444,7 @@ int launch_block_select(const rsa_attn_desc* d, char* ws, const WsLayout& L, cud
   a.scale = (float)(1.0 / sqrt((double)d->head_dim));  // == float32(head_dim ** -0.5)
   if (L.nqt == 0) return RSA_OK;
   dim3 grid(L.nqt, L.bh);
-  static int occ = 0;
-  if (!occ) {
-    const char* e = getenv("RSA_SELECT_OCC");
-    occ = (e && e[0] == '5') ? 5 : (e && e[0] == '6') ? 6 : 8;  // C3b 0.69 / 0.63 / 0.62 ms, Flux 0.23 / 0.22 / 0.21, C4 0.51 / 0.47 / 0.45 for 5 / 6 / 8
-  }
-  if (occ == 5) block_select_kernel<5><<<grid, kThreads, 0, s>>>(a);
-  else if (occ == 8) block_select_kernel<8><<<grid, kThreads, 0, s>>>(a);
-  else block_select_kernel<6><<<grid, kThreads, 0, s>>>(a);
+  block_select_kernel<<<grid, kThreads, 0, s>>>(a);
   RSA_CUDA_CHECK(cudaGetLastError());
   return RSA_OK;
 }

@@ -7,14 +7,15 @@
 // Q, K, V is read from HBM exactly once (algorithmic bytes = 3*S*H*D*2) and stays in registers for the
 // second (deviation) sweep.
 //
-// One CTA (256 threads) per (block, head, tensor).  Thread (warp w, lane l) owns rows 16w + 2*it + (l>>4),
-// it = 0..7, and the eight columns 8*(l&15) .. +7.  Summation order (the oracle replicates it bit for bit):
+// The 256 threads of a CTA reduce one (block, head, tensor) at a time.  Within a block, thread (warp w, lane l) owns
+// rows 16w + 2*it + (l>>4), it = 0..7, and the eight columns 8*(l&15) .. +7.  Summation order per block (the oracle
+// replicates it bit for bit):
 //   lane chain over it = 0..7 (sequential fp32) -> half-warp pair (shfl xor 16) -> warps 0..7 (sequential).
 // Rows >= valid_rows contribute zeros; the divisor is always 128 (the reference zero-pads, wan21 :299-302).
 // Rows are counted in the padded layout (rsa_common.cuh RowMap): a visual block reads memory rows below vis_len and
 // zeros above, a text block reads memory rows shifted down by the gap.
 //
-// The same kernel has a second front end ("prep", kernel 0): instead of loading finished Q/K/V rows it builds them from
+// Kernel 0 is a second front end of the same reduction ("prep"): instead of loading finished Q/K/V rows it builds them from
 // the projection outputs [B, S, H*D] -- per-head RMSNorm, rotary embedding, re-layout to [B, H, S, D] -- stores
 // them, and pools the values it has just rounded to bf16, so the pooled statistics are bit-identical to pooling the
 // stored rows and Q, K, V are never read back.  Replaces rectified_hunyuan_attn.py:448-479 (and the same sequence
@@ -25,7 +26,6 @@
 // forms round with cvt.rn.f16x2.f32 -- no .satfinite, so an overflow becomes +-inf as in .to(torch.float16), and results
 // below 2^-14 stay fp16 subnormals -- and pool the fp16 rows they store, exactly as kernel 2's fp16 form reads them.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "ptx_sm100.cuh"
 #include "rsa_common.cuh"
@@ -36,13 +36,12 @@ namespace {
 constexpr int kThreads = 256;
 
 struct PrepArgs {  // 16-bit tensors are in the descriptor's dtype (bf16, or fp16 in the kF16 forms)
-  const __nv_bfloat16* src[3];  // q, k, v projection outputs [B, rows, H*D], D = head_dim (128, or 64 with layer_norm)
+  const __nv_bfloat16* src[3];  // q, k, v projection outputs [B, rows, H*D], D = head_dim (128, or 64 with LayerNorm)
   int64_t src_stride[3][2];     // (batch, token) element strides
   __nv_bfloat16* dst[3];        // [B, H, S, D] views
   int64_t dst_stride[3][3];     // (batch, head, token)
   const __nv_bfloat16* w[2];    // norm weights of q, k ([D], or [H*128] with w_head_stride = 128) or nullptr
-  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k ([D]) -- layer_norm only
-  int layer_norm;               // 1: LayerNorm over head_dim (CogVideoX: mean removed, bias added, one rounding)
+  const __nv_bfloat16* bias[2]; // LayerNorm biases of q, k ([D]) -- kNorm = 3 only
   int w_head_stride;            // 0: one weight vector per tensor (norm over head_dim); 128: norm across heads (Wan)
   const float* row_rinv[2];     // norm across heads: rsqrt(mean(x^2) + eps) per (batch, source row), from row_rms_kernel
   float eps;
@@ -72,7 +71,6 @@ struct PoolArgs {
   int head_dim;               // 128 or 64: columns >= head_dim do not exist in x and pool as zeros
   // text keys copied as fp32 rows behind the pooled keys
   int text_keys, text_from;   // a, memory row of the first text token (= vis_len)
-  int pool_ctas;              // kernel 2's grid: x < pool_ctas pools block x, x >= pool_ctas copies 16 text keys
 };
 
 template <bool kF16 = false>
@@ -85,12 +83,6 @@ __device__ __forceinline__ void unpack8(const uint4& u, float* f) {
     f[2 * i] = t.x;
     f[2 * i + 1] = t.y;
   }
-}
-
-__device__ __forceinline__ uint4 ld_global_v4(const void* p) {
-  uint4 r;
-  asm volatile("ld.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-  return r;
 }
 
 // Kernel 0's rounding points: two fp32 values rounded to the 16-bit format as one packed pair.  fp16 takes
@@ -115,10 +107,11 @@ __device__ __forceinline__ float2 round2(float a, float b) {
   else return __bfloat1622float2(__floats2bfloat162_rn(a, b));
 }
 
-// Kernel 0 front end: rows of one 128-token block of one head, normalised / rotated / rounded to bf16, stored to the
-// destination and returned in the same register layout the pooling sweep uses.  All eight source rows of a thread are
-// requested before the first is used, and the rotary-table row of step it + 1 is requested before step it is
-// computed: the kernel is latency-bound otherwise (first version: 2.1 ms at C3b, 26 % of DRAM throughput).
+// Kernel 0's row transform (process_rows below): rows of one 128-token block of one head, normalised / rotated / rounded
+// to the 16-bit format, stored to the destination and left in the register layout the pooling sweep uses.  The source
+// rows arrive through the shared-memory ring of qkv_prep_stream_kernel; the rotary-table row of step it + 1 is requested
+// before step it is computed.  Without loads issued ahead the kernel is latency-bound (first version, loads issued row
+// by row: 2.1 ms at C3b, 26 % of DRAM throughput).
 struct RopeRow {
   float4 c0, c1, s0, s1;
 };
@@ -146,41 +139,6 @@ __device__ __forceinline__ RopeRow load_rope(const PrepArgs& p, int r, int col, 
 // carries only its own code and registers (with all of them behind run-time flags the HunyuanVideo form lost 40 %).
 // kD: head_dim.  At 64 (CogVideoX, LayerNorm only) a thread's 8 columns belong to one of two adjacent heads h, h + 1
 // (see qkv_prep_stream_kernel); `heads` tells whether head h + 1 exists.  kF16: the rows, weights and biases are fp16.
-template <int kNorm, bool kCompact, bool kGather, int kD = 128, bool kF16 = false>
-__device__ __forceinline__ void process_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
-                                             uint4 (&raw)[8], int heads = 0);
-
-template <int kNorm, bool kGather, bool kCompact>
-__device__ __forceinline__ void prep_rows(const PrepArgs& p, int which, int b, int h, int jblk, int warp, int lane,
-                                          uint4 (&raw)[8]) {
-  const int col = 8 * (lane & 15);
-  const __nv_bfloat16* src = p.src[which] + b * p.src_stride[which][0] + (int64_t)h * 128 + col;
-  const int r0 = jblk * 128 + 16 * warp + (lane >> 4);  // source row of step 0; the 16 lanes of a half-warp share it
-  if constexpr (!kGather) {
-#pragma unroll
-    for (int it = 0; it < 8; ++it) {
-      const int r = r0 + 2 * it;
-      raw[it] = make_uint4(0, 0, 0, 0);
-      if (r < p.rows) raw[it] = __ldg(reinterpret_cast<const uint4*>(src + (int64_t)r * p.src_stride[which][1]));
-    }
-  } else {
-    // each row comes from the rank that owns it, over NVLink
-    const int64_t off = b * p.src_stride[which][0] + (int64_t)(p.src_head0 + h) * 128 + col;
-#pragma unroll
-    for (int it = 0; it < 8; ++it) {
-      const int r = r0 + 2 * it;
-      raw[it] = make_uint4(0, 0, 0, 0);
-      if (r < p.rows) {
-        const int tok = p.dst_row0 + r;  // the peer buffers hold the tokens in memory order, like the destination
-        const int owner = tok / p.src_rows;
-        const __nv_bfloat16* base = p.src_table[which * p.n_src + owner];
-        raw[it] = ld_global_v4(base + off + (int64_t)(tok - owner * p.src_rows) * p.src_stride[which][1]);
-      }
-    }
-  }
-  process_rows<kNorm, kCompact, kGather>(p, which, b, h, jblk, warp, lane, raw);
-}
-
 // raw[it] = source row jblk * 128 + 16 warp + 2 it + (lane >> 4), columns 8 (lane & 15) .. +7 of head h (kD = 64:
 // columns 8 (lane & 7) .. +7 of head h + ((lane >> 3) & 1)), zeros beyond the source: normalise / rotate / round, store
 // to the destination, and leave the rounded values in raw (zeros for the lanes of a head that does not exist).
@@ -314,146 +272,14 @@ __global__ void __launch_bounds__(256) row_rms_kernel(const __nv_bfloat16* __res
   if (lane == 0) (which ? rk : rq)[(int64_t)b * rows + row] = rsqrtf(__fadd_rn(__fdiv_rn(ss, (float)inner), eps));
 }
 
-template <bool kPrep, int kMinBlocks = 2, int kNorm = 0, bool kGather = false, bool kCompact = false, bool kF16 = false>
-__global__ void __launch_bounds__(kThreads, kMinBlocks) pool_stats_kernel(const PoolArgs a, const PrepArgs p) {
-  // Prep grid: x = (tensor, batch*head) fastest, y = token block -- the CTAs that run together read the same source
-  // rows (all heads of a token are contiguous in the projection output) and the same rotary-table rows, which are as
-  // large as L2 at the HunyuanVideo size (2 x 61 MB) and would otherwise be streamed from HBM once per head.
-  const int which = kPrep ? (int)(blockIdx.x % 3) : (int)blockIdx.z;
-  const int bh = kPrep ? (int)(blockIdx.x / 3) : (int)blockIdx.y;
-  const int jblk = kPrep ? (int)blockIdx.y : (int)blockIdx.x;
-  const int blk = kPrep ? p.blk0 + jblk : jblk;
-  const int b = bh / a.heads, h = bh % a.heads;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-  if (!kPrep && jblk >= a.pool_ctas) {
-    // the CTAs behind the pooling ones (tensor 1 only): text keys -> fp32 rows [NQ, NQ + a) of k_cat; one 16-lane
-    // group per row
-    if (which != 1) return;
-    const int rows_per_cta = kThreads / 16;
-    const int t = (jblk - a.pool_ctas) * rows_per_cta + (tid >> 4);
-    if (t < a.text_keys) {
-      const int tok = a.text_from + t;
-      const __nv_bfloat16* src = a.x[1] + b * a.stride[1][0] + h * a.stride[1][1] + (int64_t)tok * a.stride[1][2];
-      float f[8];
-      uint4 u = make_uint4(0, 0, 0, 0);
-      if (tok + a.gap < a.valid_rows[1] && 8 * (tid & 15) < a.head_dim) u = *reinterpret_cast<const uint4*>(src + 8 * (tid & 15));
-      unpack8<kF16>(u, f);
-      float* dst = a.mean[1] + ((int64_t)bh * a.out_rows[1] + a.n_blk[1] + t) * 128 + 8 * (tid & 15);
-      reinterpret_cast<float4*>(dst)[0] = make_float4(f[0], f[1], f[2], f[3]);
-      reinterpret_cast<float4*>(dst)[1] = make_float4(f[4], f[5], f[6], f[7]);
-    }
-    return;
-  }
-  __shared__ float s_part[8][128];
-  __shared__ float s_mean[128];
-
-  const int col = 8 * (lane & 15);
-  const int row0 = blk * 128 + 16 * warp + (lane >> 4);
-  const bool visual = blk < a.nq_vis;
-  const int valid = visual ? min(a.valid_rows[which], a.vis_len) : a.valid_rows[which];
-
-  uint4 raw[8];
-  if constexpr (kPrep) {
-    prep_rows<kNorm, kGather, kCompact>(p, which, b, h, jblk, warp, lane, raw);
-    if (!p.pool) return;
-    // rows the pooling counts as zeros (K, V rows >= kv_zero_from; hunyuan masked_fill_ :307-308) stay stored as they are
-#pragma unroll
-    for (int it = 0; it < 8; ++it)
-      if (row0 + 2 * it >= valid) raw[it] = make_uint4(0, 0, 0, 0);
-    if (which == 1 && !visual) {
-      // text keys scored as single tokens: fp32 rows [NQ, NQ + a) of k_cat (hunyuan :193-194)
-#pragma unroll
-      for (int it = 0; it < 8; ++it) {
-        const int t = (blk - a.nq_vis) * 128 + 16 * warp + 2 * it + (lane >> 4);  // text token index
-        if (t < a.text_keys) {
-          float f[8];
-          unpack8<kF16>(raw[it], f);
-          float* dstk = a.mean[1] + ((int64_t)bh * a.out_rows[1] + a.n_blk[1] + t) * 128 + col;
-          reinterpret_cast<float4*>(dstk)[0] = make_float4(f[0], f[1], f[2], f[3]);
-          reinterpret_cast<float4*>(dstk)[1] = make_float4(f[4], f[5], f[6], f[7]);
-        }
-      }
-    }
-    if (blk >= a.n_blk[which]) return;
-  } else {
-    if (blk >= a.n_blk[which]) return;
-    const __nv_bfloat16* base = a.x[which] + b * a.stride[which][0] + h * a.stride[which][1];
-    const int64_t ts = a.stride[which][2];
-    const int shift = visual ? 0 : a.gap;  // padded row -> memory row
-#pragma unroll
-    for (int it = 0; it < 8; ++it) {
-      const int r = row0 + 2 * it;
-      raw[it] = make_uint4(0, 0, 0, 0);
-      if (r < valid && col < a.head_dim) raw[it] = __ldg(reinterpret_cast<const uint4*>(base + (int64_t)(r - shift) * ts + col));
-    }
-  }
-
-  float acc[8];
-#pragma unroll
-  for (int c = 0; c < 8; ++c) acc[c] = 0.f;
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    float f[8];
-    unpack8<kF16>(raw[it], f);
-#pragma unroll
-    for (int c = 0; c < 8; ++c) acc[c] = __fadd_rn(acc[c], f[c]);
-  }
-#pragma unroll
-  for (int c = 0; c < 8; ++c) acc[c] = __fadd_rn(acc[c], __shfl_xor_sync(0xffffffffu, acc[c], 16));
-  if (lane < 16) {
-#pragma unroll
-    for (int c = 0; c < 8; ++c) s_part[warp][col + c] = acc[c];
-  }
-  __syncthreads();
-  if (tid < 128) {
-    float t = s_part[0][tid];
-#pragma unroll
-    for (int w = 1; w < 8; ++w) t = __fadd_rn(t, s_part[w][tid]);
-    const float m = __fmul_rn(t, 1.0f / 128.0f);
-    s_mean[tid] = m;
-    a.mean[which][((int64_t)bh * a.out_rows[which] + blk) * 128 + tid] = m;
-  }
-  if (a.mad[which] == nullptr) return;
-  __syncthreads();
-
-  float mean[8];
-#pragma unroll
-  for (int c = 0; c < 8; ++c) mean[c] = s_mean[col + c];
-#pragma unroll
-  for (int c = 0; c < 8; ++c) acc[c] = 0.f;
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    float f[8];
-    unpack8<kF16>(raw[it], f);
-#pragma unroll
-    for (int c = 0; c < 8; ++c) acc[c] = __fadd_rn(acc[c], fabsf(__fsub_rn(f[c], mean[c])));
-  }
-#pragma unroll
-  for (int c = 0; c < 8; ++c) acc[c] = __fadd_rn(acc[c], __shfl_xor_sync(0xffffffffu, acc[c], 16));
-  __syncthreads();  // s_part reuse
-  if (lane < 16) {
-#pragma unroll
-    for (int c = 0; c < 8; ++c) s_part[warp][col + c] = acc[c];
-  }
-  __syncthreads();
-  if (tid < 128) {
-    float t = s_part[0][tid];
-#pragma unroll
-    for (int w = 1; w < 8; ++w) t = __fadd_rn(t, s_part[w][tid]);
-    a.mad[which][((int64_t)bh * a.n_blk[which] + blk) * 128 + tid] = __fmul_rn(t, 1.0f / 128.0f);
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------------
-// Kernel 2, streaming form (the one rsa_pool_stats launches).  The per-block kernel above is latency-exposed: a CTA
-// requests its 32 KB, waits for them, reduces twice across three barriers and leaves -- nothing is in flight for the
-// SM while it reduces, and at C3b there are 67 000 such CTAs (0.77 of the measured copy bandwidth).  Here a persistent
-// grid (2 CTAs per SM) walks contiguous ranges of (tensor, head, block) items; an otherwise idle warp keeps
-// kPoolStages blocks in flight with bulk copies (cp.async.bulk, no tensor map: each row is head_dim * 2 contiguous
-// bytes; rows of a [B, H, S, D] tensor with token stride D are one 32 KB copy) into a shared-memory ring, and the 256
-// threads reduce block i from shared memory exactly as above -- same thread <-> row mapping, same summation order, so
-// the statistics are bit-identical -- while blocks i + 1, i + 2 land.
+// Kernel 2 (what rsa_pool_stats launches), streaming: a CTA that requests one block, waits for it, reduces it across
+// three barriers and leaves has nothing in flight for the SM while it reduces (one CTA per block reached 0.77 of the
+// measured copy bandwidth at C3b).  So a persistent grid (2 CTAs per SM) walks contiguous ranges of (tensor, head,
+// block) items; an otherwise idle warp keeps kPoolStages blocks in flight with bulk copies (cp.async.bulk, no tensor
+// map: each row is head_dim * 2 contiguous bytes; rows of a [B, H, S, D] tensor with token stride D are one 32 KB copy)
+// into a shared-memory ring, and the 256 threads reduce block i from shared memory with the thread <-> row mapping and
+// summation order given at the top of this file while blocks i + 1, i + 2 land.
 constexpr int kPoolStages = 3;
 constexpr int kPoolStageBytes = 128 * 256;
 constexpr int kPoolSmem = kPoolStages * kPoolStageBytes + 64;
@@ -678,13 +504,13 @@ __global__ void __launch_bounds__(kThreads, 2) pool_stats_stream_kernel(const Po
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Kernel 0, streaming form (what rsa_qkv_prep / rsa_qkv_prep_gather launch).  Same structure as the streaming kernel 2:
+// Kernel 0 (what rsa_qkv_prep / rsa_qkv_prep_gather launch).  Same structure as kernel 2:
 // a persistent grid, the source rows of the next blocks in flight as 256-byte bulk copies (one per token row and head:
 // the projection output is [B, rows, H*128]) into a shared-memory ring, issued by the otherwise idle warp 7; the 256
 // threads take block n from shared memory into the register layout of process_rows (normalise / rotate / round /
 // store) and pool the rounded values with pool_block.  For the fused Ulysses gather the sources are the peer-mapped
-// buffers of the owning ranks: the copies cross NVLink with three blocks (96 KB) in flight per CTA, where the per-block
-// kernel exposed one NVLink round trip (~4 us) per block.
+// buffers of the owning ranks: the copies cross NVLink with three blocks (96 KB) in flight per CTA instead of exposing
+// one NVLink round trip (~4 us) per block.
 // Items are ordered block-major, then tensor, then head: the 3 * B * H items of one token block read the same source
 // rows (all heads of a token are contiguous) and the same rotary-table rows, which therefore stay in L1 / L2 instead
 // of being streamed from HBM once per head (the table alone is as large as L2 at the HunyuanVideo size).
@@ -694,7 +520,7 @@ __global__ void __launch_bounds__(kThreads, 2) pool_stats_stream_kernel(const Po
 // copies, nothing stored for the missing head).  Every lane stays busy: the kernel is bound by issue slots, and one
 // head per item would idle half of them.  n_bh counts pairs then (B * ceil(H / 2)).
 // kF16: fp16 rows (every form above has one); the rounding points, the copies and the pooling order are the same.
-template <int kNorm, bool kGather, bool kCompact, int kD = 128, bool kF16 = false>
+template <int kNorm, bool kGather, bool kCompact, int kD, bool kF16>
 __global__ void __launch_bounds__(kThreads, 2) qkv_prep_stream_kernel(const PoolArgs a, const PrepArgs p, const int n_blocks,
                                                                       const int n_bh) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -870,32 +696,26 @@ static PoolArgs pool_args(const rsa_attn_desc* d, const void* q, const void* k, 
   a.head_dim = d->head_dim;
   a.text_keys = L.a;
   a.text_from = rm.vis_len;
-  a.pool_ctas = L.nb;
   return a;
+}
+
+// SMs of the current device, queried once: the persistent grids of kernels 0 and 2 are two CTAs per SM.
+static int sm_count(int* sms) {
+  static int n = 0;
+  if (n == 0) {
+    int dev = 0;
+    RSA_CUDA_CHECK(cudaGetDevice(&dev));
+    RSA_CUDA_CHECK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
+  }
+  *sms = n;
+  return RSA_OK;
 }
 
 int launch_pool_stats(const rsa_attn_desc* d, const void* q, const void* k, const void* v, char* ws,
                       const WsLayout& L, cudaStream_t s) {
   const PoolArgs a = pool_args(d, q, k, v, ws, L);
-  static int form = -1;  // RSA_POOL_FORM=0: the per-block kernel (A/B timing); default: the streaming kernel
-  if (form < 0) {
-    const char* e = getenv("RSA_POOL_FORM");
-    form = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (form == 0) {
-    const int text_ctas = (L.a + 15) / 16;
-    dim3 grid(L.nb + text_ctas, L.bh, 3);
-    if (d->dtype == RSA_DTYPE_F16) pool_stats_kernel<false, 3, 0, false, false, true><<<grid, kThreads, 0, s>>>(a, PrepArgs{});
-    else pool_stats_kernel<false, 3><<<grid, kThreads, 0, s>>>(a, PrepArgs{});
-    RSA_CUDA_CHECK(cudaGetLastError());
-    return RSA_OK;
-  }
-  static int sms = 0;
   static bool configured = false;
   if (!configured) {
-    int dev = 0;
-    RSA_CUDA_CHECK(cudaGetDevice(&dev));
-    RSA_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     RSA_CUDA_CHECK(cudaFuncSetAttribute(pool_stats_stream_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));
     RSA_CUDA_CHECK(cudaFuncSetAttribute(pool_stats_stream_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));
     // two CTAs of 100 KB each per SM: without the hint the driver may pick a smaller shared-memory carve-out that holds one
@@ -903,6 +723,8 @@ int launch_pool_stats(const rsa_attn_desc* d, const void* q, const void* k, cons
     RSA_CUDA_CHECK(cudaFuncSetAttribute(pool_stats_stream_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     configured = true;
   }
+  int sms = 0;
+  if (const int rc = sm_count(&sms); rc != RSA_OK) return rc;
   const int64_t items = (int64_t)L.bh * (2 * (int64_t)L.nq + L.nb);
   if (items == 0) return RSA_OK;
   if (items > 0x7fffffffLL) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_pool_stats: too many blocks");
@@ -921,6 +743,47 @@ int launch_row_rms(const void* q_src, const void* k_src, int batch, int rows, in
                            channels, eps, rq, rk);
   RSA_CUDA_CHECK(cudaGetLastError());
   return RSA_OK;
+}
+
+// One form of kernel 0.  Its shared-memory attributes are set on its first launch: two CTAs of 100 KB each per SM, as
+// for kernel 2.
+template <int kNorm, bool kGather, bool kCompact, int kD, bool kF16>
+static int launch_prep_stream(const PoolArgs& a, const PrepArgs& pa, int grid, int blocks, int n_bh, cudaStream_t s) {
+  auto kernel = qkv_prep_stream_kernel<kNorm, kGather, kCompact, kD, kF16>;
+  static bool configured = false;
+  if (!configured) {
+    RSA_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));
+    RSA_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    configured = true;
+  }
+  kernel<<<grid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);
+  RSA_CUDA_CHECK(cudaGetLastError());
+  return RSA_OK;
+}
+
+// The forms of kernel 0 that are built, for each rotary-table form (kCompact) and dtype (kF16): 128 columns with norms
+// 0-3 locally and norms 0-2 in gather form, 64 columns with norm 3 (LayerNorm, CogVideoX) in both.  rsa_qkv_prep and
+// rsa_qkv_prep_gather (rsa_api.cu) refuse every other norm and head_dim.
+template <bool kCompact, bool kF16>
+static int launch_prep_form(int norm, bool gather, int head_dim, const PoolArgs& a, const PrepArgs& pa, int grid,
+                            int blocks, int n_bh, cudaStream_t s) {
+  if (head_dim == 64) {
+    if (gather) return launch_prep_stream<3, true, kCompact, 64, kF16>(a, pa, grid, blocks, n_bh, s);
+    return launch_prep_stream<3, false, kCompact, 64, kF16>(a, pa, grid, blocks, n_bh, s);
+  }
+  if (gather) {
+    switch (norm) {
+      case 1: return launch_prep_stream<1, true, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+      case 2: return launch_prep_stream<2, true, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+      default: return launch_prep_stream<0, true, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+    }
+  }
+  switch (norm) {
+    case 1: return launch_prep_stream<1, false, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+    case 2: return launch_prep_stream<2, false, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+    case 3: return launch_prep_stream<3, false, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+    default: return launch_prep_stream<0, false, kCompact, 128, kF16>(a, pa, grid, blocks, n_bh, s);
+  }
 }
 
 int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* q_src, const void* k_src,
@@ -942,7 +805,6 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
   pa.w[0] = p->norm ? (const __nv_bfloat16*)p->q_weight : nullptr;
   pa.w[1] = p->norm ? (const __nv_bfloat16*)p->k_weight : nullptr;
   pa.w_head_stride = p->norm == 2 ? 128 : 0;
-  pa.layer_norm = p->norm == 3 ? 1 : 0;
   pa.bias[0] = (const __nv_bfloat16*)p->q_bias;
   pa.bias[1] = (const __nv_bfloat16*)p->k_bias;
   pa.row_rinv[0] = pa.row_rinv[1] = nullptr;
@@ -993,95 +855,20 @@ int launch_qkv_prep(const rsa_prep_desc* p, const rsa_attn_desc* d, const void* 
   }
   const int blocks = (p->rows + 127) / 128;
   const bool compact = pa.rope_compact && pa.rope_rows > 0;
-  static int form = -1;  // RSA_PREP_FORM=0: the per-block kernel (A/B timing); default: the streaming kernel
-  static int sms = 0;
-  if (form < 0) {
-    const char* e = getenv("RSA_PREP_FORM");
-    form = (e && e[0] == '0') ? 0 : 1;
-    int dev = 0;
-    RSA_CUDA_CHECK(cudaGetDevice(&dev));
-    RSA_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  }
   const bool hd64 = d->head_dim == 64;  // items are head pairs (qkv_prep_stream_kernel)
   const int n_bh = d->batch * (hd64 ? (d->heads + 1) / 2 : d->heads);
   const int64_t items = (int64_t)blocks * 3 * n_bh;
   if (items > 0x7fffffffLL) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep: too many blocks");
-  const int sgrid = (int)(items < 2 * sms ? items : 2 * sms);
-  dim3 grid(3 * d->batch * d->heads, blocks);
-  // per-block form: 2 CTAs per SM (about 100 registers): capping at 3 or 4 CTAs spills and is no faster (1.24 / 1.25 / 2.17 ms at C3b)
-#define RSA_PREP_STREAM_F(NORM, GATHER, COMPACT, D, F16)                                                                \
-  do {                                                                                                                  \
-    static bool cfg = false;                                                                                            \
-    if (!cfg) {                                                                                                         \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16>,                         \
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, kPoolSmem));                     \
-      RSA_CUDA_CHECK(cudaFuncSetAttribute(qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16>,                         \
-                                          cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-      cfg = true;                                                                                                       \
-    }                                                                                                                   \
-    qkv_prep_stream_kernel<NORM, GATHER, COMPACT, D, F16><<<sgrid, kThreads, kPoolSmem, s>>>(a, pa, blocks, n_bh);       \
-  } while (0)
-#define RSA_PREP_STREAM(NORM, GATHER, COMPACT, D) RSA_PREP_STREAM_F(NORM, GATHER, COMPACT, D, false)
-#define RSA_PREP_F16(NORM, GATHER, D)                                    \
-  do {                                                                   \
-    if (compact) RSA_PREP_STREAM_F(NORM, GATHER, true, D, true);         \
-    else RSA_PREP_STREAM_F(NORM, GATHER, false, D, true);                \
-  } while (0)
-#define RSA_PREP_LAUNCH(NORM, GATHER)                                                               \
-  do {                                                                                              \
-    if (form == 1) {                                                                                \
-      if (compact) RSA_PREP_STREAM(NORM, GATHER, true, 128);                                        \
-      else RSA_PREP_STREAM(NORM, GATHER, false, 128);                                               \
-    } else if (compact) pool_stats_kernel<true, 2, NORM, GATHER, true><<<grid, kThreads, 0, s>>>(a, pa);   \
-    else pool_stats_kernel<true, 2, NORM, GATHER, false><<<grid, kThreads, 0, s>>>(a, pa);          \
-  } while (0)
-  if (!f16) {
-    if (hd64) {
-      // 64-column heads: CogVideoX's LayerNorm only (rsa_api.cu refuses the other norms), always the streaming kernel
-      if (route) {
-        if (compact) RSA_PREP_STREAM(3, true, true, 64);
-        else RSA_PREP_STREAM(3, true, false, 64);
-      } else if (compact) {
-        RSA_PREP_STREAM(3, false, true, 64);
-      } else {
-        RSA_PREP_STREAM(3, false, false, 64);
-      }
-    } else if (route) {
-      if (p->norm == 1) RSA_PREP_LAUNCH(1, true);
-      else if (p->norm == 2) RSA_PREP_LAUNCH(2, true);
-      else RSA_PREP_LAUNCH(0, true);
-    } else {
-      switch (p->norm) {
-        case 1: RSA_PREP_LAUNCH(1, false); break;
-        case 2: RSA_PREP_LAUNCH(2, false); break;
-        case 3: RSA_PREP_LAUNCH(3, false); break;
-        default: RSA_PREP_LAUNCH(0, false); break;
-      }
-    }
-  } else {
-    // fp16: the streaming kernel only (RSA_PREP_FORM=0 selects the per-block form for bf16), the same norms as bf16
-    if (hd64) {
-      if (route) RSA_PREP_F16(3, true, 64);
-      else RSA_PREP_F16(3, false, 64);
-    } else if (route) {
-      if (p->norm == 1) RSA_PREP_F16(1, true, 128);
-      else if (p->norm == 2) RSA_PREP_F16(2, true, 128);
-      else RSA_PREP_F16(0, true, 128);
-    } else {
-      switch (p->norm) {
-        case 1: RSA_PREP_F16(1, false, 128); break;
-        case 2: RSA_PREP_F16(2, false, 128); break;
-        case 3: RSA_PREP_F16(3, false, 128); break;
-        default: RSA_PREP_F16(0, false, 128); break;
-      }
-    }
+  int sms = 0;
+  if (const int rc = sm_count(&sms); rc != RSA_OK) return rc;
+  const int grid = (int)(items < 2 * sms ? items : 2 * sms);
+  const bool gather = route != nullptr;
+  if (f16) {
+    if (compact) return launch_prep_form<true, true>(p->norm, gather, d->head_dim, a, pa, grid, blocks, n_bh, s);
+    return launch_prep_form<false, true>(p->norm, gather, d->head_dim, a, pa, grid, blocks, n_bh, s);
   }
-#undef RSA_PREP_STREAM_F
-#undef RSA_PREP_STREAM
-#undef RSA_PREP_F16
-#undef RSA_PREP_LAUNCH
-  RSA_CUDA_CHECK(cudaGetLastError());
-  return RSA_OK;
+  if (compact) return launch_prep_form<true, false>(p->norm, gather, d->head_dim, a, pa, grid, blocks, n_bh, s);
+  return launch_prep_form<false, false>(p->norm, gather, d->head_dim, a, pa, grid, blocks, n_bh, s);
 }
 
 }  // namespace rsa

@@ -1,5 +1,5 @@
 """Kernel 2 timing on one workload, cold (GPU idle before) and hot (right after 20 full calls, i.e. under the power cap,
-which is the state it runs in inside a denoising loop); RSA_POOL_FORM=0 selects the per-block kernel for A/B."""
+which is the state it runs in inside a denoising loop)."""
 import json, os, subprocess, sys
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO); sys.path.insert(0, os.path.join(REPO, "rectified-spaattn_b200"))
@@ -29,7 +29,7 @@ def t(fn, n):
     return e0.elapsed_time(e1) / n
 
 b = 3 * q.numel() * 2
-res = {"workload": name, "form": os.environ.get("RSA_POOL_FORM", "1")}
+res = {"workload": name}
 for _ in range(5):
     plan.pool_stats()
 torch.cuda.synchronize()
