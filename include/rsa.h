@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define RSA_VERSION 109 /* 109: kernel 0 (rsa_qkv_prep, rsa_qkv_prep_gather) in fp16; rsa_row_rms_dtype */
+#define RSA_VERSION 110 /* 110: rsa_qkv_prep_gather takes the visual / text two-call form at head_dim 64 too */
 #define RSA_BLOCK 128
 #define RSA_HEAD_DIM 128
 #define RSA_MAX_ENTRIES 2048 /* max sortable entries per query block: NQ (+1 for the text aggregate) */
@@ -304,9 +304,10 @@ int rsa_peer_close(void* ptr);
  * when the tokens do not divide (every rank must own at least one; all buffers are laid out for rows_per_rank rows).
  * This rank computes heads [head0, head0 + desc->heads) of the heads_total heads; the shards need not be even (12 heads
  * on 8 ranks: 2,2,2,2,1,1,1,1), every rank states its own first head and its own count.  Prep norm 0, 1, or 2 (2 needs
- * rinv_table) at head_dim 128; norm 3 (LayerNorm, CogVideoX) over the whole sequence at head_dim 64.  A ragged visual segment (HunyuanVideo 129
- * frames) takes two gather calls like rsa_qkv_prep: the visual tokens (dst_row 0) and the text tokens (dst_row = visual
- * token count); the source token of row r is dst_row + r in both. */
+ * rinv_table) at head_dim 128; norm 3 (LayerNorm, CogVideoX) at head_dim 64.  A ragged visual segment (HunyuanVideo 129
+ * frames, Flux 1360x768, CogVideoX 49 frames at 480x720) takes two gather calls like rsa_qkv_prep, at either head_dim:
+ * the visual tokens (dst_row 0) and the text tokens (dst_row = visual token count); the source token of row r is
+ * dst_row + r in both. */
 typedef struct rsa_peer_route {
   int32_t n_ranks, rank;
   int32_t rows_per_rank;

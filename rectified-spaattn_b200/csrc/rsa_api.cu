@@ -558,11 +558,10 @@ extern "C" int rsa_qkv_prep_gather(const rsa_prep_desc* p, const rsa_attn_desc* 
   const bool txt = p->dst_row == rm.vis_len && p->rows == d->seq - rm.vis_len && d->family == RSA_FAMILY_JOINT;
   if (!whole && !vis && !txt)
     RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: rows / dst_row must name the whole sequence, the visual tokens or the text tokens");
-  // head_dim 128: norms 0-2; head_dim 64 (CogVideoX): LayerNorm (norm 3) over the whole sequence (no gap in its geometry)
+  // head_dim 128: norms 0-2; head_dim 64 (CogVideoX): LayerNorm (norm 3), in the same one- or two-call forms
   if (d->head_dim == 64) {
     if (p->norm != 3)
       RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: head_dim 64 is built for norm 3 (LayerNorm, CogVideoX) only, not norm %d", p->norm);
-    if (!whole) RSA_FAIL(RSA_ERR_UNSUPPORTED, "rsa_qkv_prep_gather: head_dim 64 takes the whole sequence in one call");
     if (!p->q_bias || !p->k_bias || (uintptr_t)p->q_bias % 16 || (uintptr_t)p->k_bias % 16)
       RSA_FAIL(RSA_ERR_ARG, "rsa_qkv_prep_gather: norm 3 needs 16-byte aligned biases");
   } else if (p->norm < 0 || p->norm > 2) {

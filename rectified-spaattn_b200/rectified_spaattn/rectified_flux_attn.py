@@ -1,5 +1,6 @@
 """Drop-in mirror of the reference rectified_spaattn/rectified_flux_attn.py (Flux.1-dev joint attention: image
-tokens first, `text_length` text tokens last, no padding).  See rectified_wan21_attn.py for the symbol map."""
+tokens first, `text_length` text tokens last; image token counts that do not fill whole blocks -- 1360x768, 1280x720,
+832x1216, 1920x1088 -- take the padded layout of geometry.flux, which the reference does not have).  See rectified_wan21_attn.py for the symbol map."""
 import torch
 
 from rsa_b200 import geometry as _G
@@ -60,7 +61,7 @@ class RectifiedFluxSpaAttnProcessor2_0(_P.ProcessorBase):
             # kernel 0: everything between the projections and the attention in one pass (reference :431-486)
             s = hidden_states.shape[1] + (encoder_hidden_states.shape[1] if encoder_hidden_states is not None else 0)
             fused = None
-            if s % 128 == 0 and s > self.text_length:
+            if s > self.text_length:    # a ragged S takes the padded layout of _G.flux (two kernel-0 calls)
                 fused = _P.fused_prep_attention(attn, hidden_states, encoder_hidden_states, _G.flux(s, self.text_length),
                                                 self.select_block_num, self.p_remain_rates, self.block_neighbor_list,
                                                 image_rotary_emb, rope_text=True,

@@ -73,7 +73,7 @@ EXPORTS = [
 _lib = None
 
 
-ABI_VERSION = 109
+ABI_VERSION = 110
 
 
 def lib():

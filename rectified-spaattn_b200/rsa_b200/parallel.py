@@ -242,12 +242,16 @@ class FusedUlysses:
         with torch.cuda.device(self.device):
             if gap:     # ragged visual segment: the block structure restarts at the text tokens -> two gathers
                 nv = plan.desc.vis_len
+                n_rope = p.rope_rows
                 p.rows, p.dst_row = nv, 0
-                p.rope_rows = min(p.rope_rows, nv)
+                p.rope_rows = min(n_rope, nv)
                 N.check(self._lib.rsa_qkv_prep_gather(C.byref(p), C.byref(plan.desc), C.byref(self.route),
                                                       plan.q.data_ptr(), plan.k.data_ptr(), plan.v.data_ptr(), pool,
                                                       plan.ws.data_ptr(), plan.ws_bytes, st), "rsa_qkv_prep_gather")
-                p.rows, p.dst_row, p.rope_rows = self.seq - nv, nv, 0
+                # text tokens: rotated with table rows [nv, rope_rows) when the tables reach past the visual tokens (Flux)
+                p.rows, p.dst_row, p.rope_rows = self.seq - nv, nv, max(0, n_rope - nv)
+                if p.rope_rows:
+                    p.cos, p.sin = p.cos + nv * hd * 4, p.sin + nv * hd * 4
             N.check(self._lib.rsa_qkv_prep_gather(C.byref(p), C.byref(plan.desc), C.byref(self.route), plan.q.data_ptr(),
                                                   plan.k.data_ptr(), plan.v.data_ptr(), pool, plan.ws.data_ptr(),
                                                   plan.ws_bytes, st), "rsa_qkv_prep_gather")

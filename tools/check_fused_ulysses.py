@@ -1,5 +1,5 @@
 """Multi-GPU check + measurement of the fused Ulysses exchange (run under torchrun on 2, 4 or 8 GPUs of one box;
-workload name as the argument: a bench.py workload, or "odd" / "cog" below; --dense: the dense form, FusedUlysses.run(
+workload name as the argument: a bench.py workload, or "odd" / "cog" / "cog_ragged" / "flux_ragged" below; --dense: the dense form, FusedUlysses.run(
 dense=True) against kernel 0 without pooling + Plan.run_dense; --dtype float16: fp16 projection rows, norm parameters and
 results, FusedUlysses(dtype=torch.float16)):
   * rank r holds tokens [r*S/P, (r+1)*S/P) of the projection outputs; FusedUlysses.run() must return exactly the rows a
@@ -39,6 +39,16 @@ if name == "cog":
     # video + 227 text = 611 tokens and 3 heads, so neither divides by 2 ranks
     bench.WORKLOADS["cog"] = dict(desc="CogVideoX form, uneven token and head shards", fam="cog", grid=(2, 8, 24),
                                   text=227, text_valid=227, heads=3, drop=0.5, ffb=False)
+if name == "cog_ragged":
+    # CogVideoX form with a ragged visual segment: 3 x 10 x 35 = 1050 video tokens (8 blocks + 26) + 226 text -> the
+    # padded layout of geometry.cogvideo (gap 102), two gathers per tensor
+    bench.WORKLOADS["cog_ragged"] = dict(desc="CogVideoX form, ragged visual segment", fam="cog", grid=(3, 10, 35),
+                                         text=226, text_valid=226, heads=3, drop=0.5, ffb=False)
+if name == "flux_ragged":
+    # Flux form with a ragged visual segment: 1 x 25 x 41 = 1025 image tokens + 512 text (gap 127); the rotary
+    # embedding covers the text tokens too, so the text gather rotates with table rows [nv, S)
+    bench.WORKLOADS["flux_ragged"] = dict(desc="Flux form, ragged visual segment", fam="flux", grid=(1, 25, 41),
+                                          text=512, text_valid=512, heads=3, drop=0.5, ffb=False)
 wp = bench.workload_params(name)
 heads, s, nv = wp["heads"], wp["s"], wp["nv"]
 cog = wp["fam"] == "cog"
@@ -61,14 +71,17 @@ wk = (1 + 0.1 * torch.randn(nw, generator=g, device=dev)).to(dt)
 # CogVideoX: LayerNorm(head_dim) with bias on q and k
 norm_kw = dict(q_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(dt),
                k_bias=(0.05 * torch.randn(hd, generator=g, device=dev)).to(dt)) if cog else {}
-ang = torch.outer(torch.arange(nv, dtype=torch.float32, device=dev), 1.0 / (256.0 ** (torch.arange(0, hd, 2, device=dev) / hd)))
+n_rope = s if wp["fam"] == "flux" else nv            # Flux rotates every token, the others the visual tokens only
+ang = torch.outer(torch.arange(n_rope, dtype=torch.float32, device=dev), 1.0 / (256.0 ** (torch.arange(0, hd, 2, device=dev) / hd)))
 rope = (ang.cos().repeat_interleave(2, 1).contiguous(), ang.sin().repeat_interleave(2, 1).contiguous())
+rope_vis = (rope[0][:nv], rope[1][:nv])
+rope_txt = (rope[0][nv:], rope[1][nv:]) if n_rope > nv else None
 mine = slice(rank * rows, min((rank + 1) * rows, s))
 
 fu = parallel.FusedUlysses(1, heads, geo, wp["top_k"], bench.P_REMAIN, nbr, head_dim=hd, dtype=dt)
 for dst, src in zip((fu.q_src, fu.k_src, fu.v_src), full):
     dst.copy_(src[:, mine])
-out = fu.run(wq, wk, 1e-6, rope, nv, dense=dense, **norm_kw).clone()
+out = fu.run(wq, wk, 1e-6, rope, n_rope, dense=dense, **norm_kw).clone()
 torch.cuda.synchronize()
 
 # NCCL form: all-to-all the projection rows to head shards, kernel 0 + pooled call locally, all-to-all the result back
@@ -101,12 +114,13 @@ def nccl_form():
     if wan:
         plan.qkv_prep(*srcs, dst_row=0, rope=rope, rope_rows=nv, pool=not dense, **f16)
     elif geo.gap:
-        plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
-                      pool=not dense, **f16)
-        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense, **f16)
+        plan.qkv_prep(*(x[:, :nv] for x in srcs), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope_vis,
+                      pool=not dense, **norm_kw, **f16)
+        plan.qkv_prep(*(x[:, nv:] for x in srcs), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope_txt,
+                      pool=not dense, **norm_kw, **f16)
     else:
-        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
-                      **norm_kw, **f16)
+        plan.qkv_prep(*srcs, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=n_rope,
+                      pool=not dense, **norm_kw, **f16)
     o = finish(plan)                                                                     # [1, S, hl, hd]
     return parallel.head_to_seq_shard(o).reshape(1, rows, heads * hd)
 
@@ -124,12 +138,13 @@ if check and (rank == 0 or not even):       # uneven shards: every rank checks i
     qa, ka, va = (torch.empty(1, heads, s, hd, dtype=dt, device=dev) for _ in range(3))
     pa = ops.Plan(qa, ka, va, geo, wp["top_k"], bench.P_REMAIN, nbr)
     if geo.gap:
-        pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope,
-                    pool=not dense, **f16)
-        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, pool=not dense, **f16)
+        pa.qkv_prep(*(x[:, :nv] for x in full), dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope_vis,
+                    pool=not dense, **norm_kw, **f16)
+        pa.qkv_prep(*(x[:, nv:] for x in full), dst_row=nv, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope_txt,
+                    pool=not dense, **norm_kw, **f16)
     else:
-        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=nv, pool=not dense,
-                    **norm_kw, **f16)
+        pa.qkv_prep(*full, dst_row=0, q_weight=wq, k_weight=wk, eps=1e-6, rope=rope, rope_rows=n_rope,
+                    pool=not dense, **norm_kw, **f16)
     single = finish(pa).reshape(1, s, heads * hd)[:, mine]
     torch.cuda.synchronize()
     same_as_single = bool(torch.equal(out.view(torch.int16), single.view(torch.int16)))
@@ -153,7 +168,7 @@ def timed(fn, n=10):
     return float(tt.item())
 
 
-ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, nv, dense=dense, **norm_kw))
+ms_fused = timed(lambda: fu.run(wq, wk, 1e-6, rope, n_rope, dense=dense, **norm_kw))
 ms_nccl = timed(nccl_form) if even else None
 oks = [None] * world
 dist.all_gather_object(oks, same_as_nccl)
